@@ -334,6 +334,7 @@ int liorf_debug_voxelgrid_stamps(liorf_ctx* ctx, int enable, unsigned long long*
 int liorf_debug_force_fused_voxelgrid(liorf_ctx* ctx, int on);   /* tests: one-kernel cooperative VoxelGrid path on small clouds too */
 int liorf_debug_s2m_global_state(liorf_ctx* ctx, int on);          /* tests: solver keeps per-query state in global memory (the multi-round layout) */
 int liorf_debug_s2m_disable_cache(liorf_ctx* ctx, int on);        /* tests: full 27-cell search + plane refit every iteration */
+int liorf_debug_s2m_grid(liorf_ctx* ctx, int ctas);               /* tests: solver CTAs of every launch, 2..SMs (0 = defaults) */
 int liorf_debug_s2m_clocks(liorf_ctx* ctx, int enable, long long* out /* 64*8, nullable */);
 int liorf_debug_s2m_arrivals(liorf_ctx* ctx, int enable, unsigned long long* out /* 64*160, nullable */);   /* %globaltimer stamps (debug) */   /* solver phase clocks (debug) */
 int liorf_get_keyframe(liorf_ctx* ctx, int id, liorf_point* out, int capacity, int* n, float pose6[6], double* time);

@@ -376,6 +376,10 @@ class Context:
     def disableSolverCache(self, on=True):
         _chk(self.lib.liorf_debug_s2m_disable_cache(self.h, C.c_int(int(on))), "liorf_debug_s2m_disable_cache")
 
+    def solverGrid(self, ctas=0):
+        """run the solver on `ctas` CTAs (ctas - 1 workers + the reducer) in every launch; 0 = the defaults"""
+        _chk(self.lib.liorf_debug_s2m_grid(self.h, C.c_int(int(ctas))), "liorf_debug_s2m_grid")
+
     def forceFusedVoxelGrid(self, on=True):
         _chk(self.lib.liorf_debug_force_fused_voxelgrid(self.h, C.c_int(int(on))), "liorf_debug_force_fused_voxelgrid")
 

@@ -88,6 +88,7 @@ struct liorf_ctx {
     float* d_tf6 = nullptr; LMDeviceState* d_lm = nullptr; S2MTrace* d_trace = nullptr; double* d_partial = nullptr; ulonglong2* d_wpart = nullptr; unsigned long long* d_res = nullptr; long long* d_dbg = nullptr; unsigned long long* d_dbg_gt = nullptr;
     IcpState* icp_state = nullptr; DevBuf<QueryCache> qcache; DevBuf<float4> cand; unsigned s2m_launch_seq = 0; S2MMail* d_mail = nullptr; bool mail_fresh = false; bool s2m_global_state = false;
     int s2m_grid = 0; bool s2m_no_cache = false; int map_vg_grid = 0;
+    int s2m_ctas = 0;                // tests: solver CTAs of every launch (0 = num_sms per function call, s2m_grid in liorf_process_frame)
     DevBuf<float4> h_coeff, h_sel_pts, h_ori_c, h_coeff_c; DevBuf<unsigned char> h_flag; DevBuf<int> h_idx; DevBuf<float> h_d2, h_plane;
     DevBuf<double> lm_partial; ScanWork combine_scan; int hook_n = 0;
     float* d_lm_out = nullptr;      // AtA[36] AtB[6] X[6]
@@ -292,6 +293,13 @@ int liorf_create(const liorf_params* p, liorf_ctx** out) {
     CUDA_TRY(cudaSetDevice(c->P.device));
     cudaDeviceProp prop; CUDA_TRY(cudaGetDeviceProperties(&prop, c->P.device));
     c->num_sms = prop.multiProcessorCount;
+    // The reducer CTA of the solver collects the partial sums of at most S2M_MAX_WORKERS workers (a register array sized at compile
+    // time); a grid of num_sms CTAs has num_sms - 1 workers.  A B200 (148 SMs) is within the limit, so this refusal never runs there.
+    if (c->num_sms - 1 > S2M_MAX_WORKERS) {
+        fprintf(stderr, "[liorf_b200] %d SMs: the solver supports at most %d (raise S2M_MAX_WORKERS in scan2map.cuh)\n", c->num_sms, S2M_MAX_WORKERS + 1);
+        delete c;
+        return LIORF_ERR_CUDA;
+    }
     // the main stream carries the latency-critical chain (deskew → downsample → solver); giving it the highest priority lets
     // its large-footprint CTAs (single-CTA VoxelGrid, one-CTA-per-SM solver) claim SMs from the concurrent local-map chain
     int prio_lo = 0, prio_hi = 0;
@@ -351,11 +359,14 @@ int liorf_create(const liorf_params* p, liorf_ctx** out) {
     CUDA_TRY(cudaFuncSetAttribute(k_scan2map_persistent, cudaFuncAttributeMaxDynamicSharedMemorySize, S2MP_SMEM));
     CUDA_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, k_scan2map_persistent, S2MP_BLOCK, S2MP_SMEM));
     if (occ < 1) { fprintf(stderr, "[liorf_b200] persistent kernel does not fit\n"); return LIORF_ERR_CUDA; }
-    // One persistent CTA per SM, on all but S2M_SPARE_SMS of them.  The solver's CTA owns its SM outright (512 threads x 128
-    // registers = the whole register file), so the SMs it leaves free are where the NEXT frame's cloudHandler + downsample
-    // (stream_pre) run while it iterates.  The solve is latency-bound (one round of <= 128 queries per CTA up to ~17k points), so
-    // the narrower grid costs nothing at the KITTI sizes; the grid is the same with and without look-ahead, which keeps the
-    // CTA-ordered fp64 partial sums — and therefore the results — bit-identical between the two.
+    // liorf_process_frame runs the solver on one persistent CTA per SM of all but S2M_SPARE_SMS SMs.  The solver's CTA owns its SM
+    // outright (512 threads x 128 registers = the whole register file), so the SMs it leaves free are where the NEXT frame's
+    // cloudHandler + downsample (stream_pre) run while it iterates.  The solve is latency-bound (one round of <= 128 queries per CTA up
+    // to ~17k points), so the narrower grid costs nothing at the KITTI sizes.  The grid is the same with and without look-ahead, so
+    // those two give bit-identical results.  The per-function calls (liorf_scan2map_optimization[_async]) launch num_sms CTAs instead:
+    // the grid width decides which worker serves each query, how the fp64 partial sums are grouped and from which scan size on the
+    // per-query state moves to global memory, so their results may differ from liorf_process_frame's in the last bits.
+    // liorf_debug_s2m_grid sets the width of both for tests.
     {
         int spare = S2M_SPARE_SMS;
         if (const char* e = std::getenv("LIORF_SOLVER_SPARE_SMS")) spare = std::atoi(e);
@@ -945,6 +956,9 @@ static int launch_s2m(liorf_ctx* c, int max_iters, int force_all, bool pipelined
     if ((rc = join_map(c))) return rc;
     S2MArgs a;
     a.qcache = c->qcache.p; a.cand = c->cand.p; a.res = c->d_res; a.wpart = c->d_wpart; a.err_flag = c->d_err; a.global_state = c->s2m_global_state ? 1 : 0;
+    // epochs of a launch: epoch_base + 1 .. epoch_base + max_iters; they must stay below the next launch's first one, or a worker could
+    // take a hand-off word the previous launch left behind for an answer
+    static_assert(S2M_MAX_ITERS <= 64, "the epoch stride of the solver launches is 64");
     a.epoch_base = (++c->s2m_launch_seq) * 64u;
     a.scan = c->scan_ds.p; a.n_scan = scan_ds_count(c);
     a.cell_start = c->grid.cell_start.p; a.gmap = c->grid.sorted.p; a.g = c->grid.dims; a.m_map = map_count(c);
@@ -954,7 +968,8 @@ static int launch_s2m(liorf_ctx* c, int max_iters, int force_all, bool pipelined
     for (int k = 0; k < 6; ++k) a.tf_init[k] = pose6_init ? pose6_init[k] : 0.f;
     void* args[] = {&a};
     ProfScope ps(c, SEC_SCAN2MAP); c->launches += 1;
-    CUDA_TRY(cudaLaunchCooperativeKernel((void*)k_scan2map_persistent, dim3(pipelined ? c->s2m_grid : c->num_sms), dim3(S2MP_BLOCK), args, S2MP_SMEM, c->stream));
+    const int ctas = c->s2m_ctas ? c->s2m_ctas : (pipelined ? c->s2m_grid : c->num_sms);
+    CUDA_TRY(cudaLaunchCooperativeKernel((void*)k_scan2map_persistent, dim3(ctas), dim3(S2MP_BLOCK), args, S2MP_SMEM, c->stream));
     c->mail_fresh = true;
     return LIORF_OK;
 }
@@ -2112,6 +2127,15 @@ int liorf_debug_s2m_global_state(liorf_ctx* c, int on) {
     LIORF_NVTX;
     if (!c) return LIORF_ERR_ARG;
     c->s2m_global_state = on != 0;
+    return LIORF_OK;
+}
+/* tests: the solver runs on `ctas` CTAs (ctas - 1 workers and the reducer) in every launch, per-function calls and liorf_process_frame
+ * alike, so that each layout of k_scan2map_persistent can be reached on any scan size; 0 = the defaults.  The cooperative launch needs
+ * every CTA resident at once, one per SM: 2 <= ctas <= num_sms.  The front end's share of the SMs in liorf_process_frame does not change. */
+int liorf_debug_s2m_grid(liorf_ctx* c, int ctas) {
+    LIORF_NVTX;
+    if (!c || (ctas != 0 && (ctas < 2 || ctas > c->num_sms))) return LIORF_ERR_ARG;
+    c->s2m_ctas = ctas;
     return LIORF_OK;
 }
 /* debug: %globaltimer stamps of the last solve, out[iter * 160 + k]: k < workers = that worker's arrival, 156 = reducer sums
