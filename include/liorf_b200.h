@@ -189,14 +189,19 @@ int liorf_sc_detect_loop_closure_id(liorf_ctx* ctx, int* loop_id, float* yaw_dif
  * rows [global_offset, global_offset + n_db) (single GPU: offset 0).  The steps of one batch on DEVICE buffers (d_* are device pointers):
  *   prepare: ring keys (a11) of Q query descriptors → d_qkeys [Q][20] f32 (d_qsk / d_qcn, nullable: sector keys / column norms [Q][60] f64)
  *   stage 1: exact top-3 per query → (dist[Q*3], idx[Q*3]); unfilled slots carry idx INT_MAX
- *   stage 2: distanceBtnScanContext for the candidates in [global_offset, global_offset + n_db) (others left untouched); the query's
- *            sector key and column norms are derived inside the kernel from its descriptor
- *   decide : strict-< argmin in kNN order + threshold (include/Scancontext.cpp:302-340) */
+ *   stage 2: distanceBtnScanContext for the candidates in [global_offset, global_offset + n_db); every other output slot is left
+ *            untouched, except that a candidate of INT_MAX (unfilled) or below 0 gives dist +inf and shift 0 in every context.  The
+ *            query's sector key and column norms are derived inside the kernel from its descriptor
+ *   decide : strict-< argmin in kNN order + threshold (include/Scancontext.cpp:302-340)
+ * Query descriptors (here and in liorf_sc_shard_query_dev / _phases_dev) need only 8-byte alignment in every stage, e.g. a float64
+ * tensor view at an odd element offset; 16-byte-aligned ones take the faster loads. */
 int liorf_sc_prepare_queries_dev(liorf_ctx* ctx, const void* d_qdescs, int Q, void* d_qkeys /*Q*20 f32*/, void* d_qsk /*Q*60 f64, nullable*/, void* d_qcn /*Q*60 f64, nullable*/);
 int liorf_sc_knn_batch_dev(liorf_ctx* ctx, const void* d_qkeys, int Q, int global_offset, void* d_dist, void* d_idx);
 int liorf_sc_distance_batch_dev(liorf_ctx* ctx, const void* d_qdescs, const void* d_cand_idx, int Q, int global_offset, void* d_pair_dist /*Q*3 f64*/, void* d_pair_shift /*Q*3 i32*/);
 int liorf_sc_decide_dev(liorf_ctx* ctx, const void* d_pair_dist, const void* d_pair_shift, const void* d_cand_idx, int Q,
                         void* d_loop_id, void* d_shift, void* d_dist);
+/* tests: out = {SMs, stage-2 CTAs per SM for 16-byte-aligned query descriptors, the same for 8-byte-aligned ones} */
+int liorf_debug_sc_distance_occupancy(liorf_ctx* ctx, int out[3]);
 /* Ring-key search implementation used by liorf_sc_knn_batch_dev / liorf_sc_query_batch / the sharded search:
  *   0 auto (tensor cores for batches of >= 64 queries against >= 4096 keys), 1 CUDA-core brute force,
  *   2 tcgen05 coarse filter + exact re-rank (csrc/sc_tensor.cuh).  All three return the same exact top-3

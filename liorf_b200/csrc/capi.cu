@@ -115,7 +115,7 @@ struct liorf_ctx {
                      cudaGraphExec_t graph = nullptr; const void* gsig[40] = {nullptr}; const void* last_sig[40] = {nullptr}; bool ipc_opened[SCSH_MAX] = {false};
                      DevBuf<int> list; int* d_nlist = nullptr; } shard;
     int sc_path = 0;                 // 0 auto, 1 CUDA-core brute force, 2 tensor-core filter + exact re-rank
-    bool sct_attr_set = false; int sct_last_Q = 0; bool scdb_attr_set = false; int scdb_blocks_per_sm = 1;
+    bool sct_attr_set = false; int sct_last_Q = 0; bool scdb_attr_set = false; int scdb_blocks_per_sm[2] = {1, 1};   // [kQ16]
     Profiler prof;
     double host_us[12] = {0}; long long host_frames = 0; bool host_timing = false;   // LIORF_HOST_TIMING=1 ([6..10]: pieces of the keyframe tail)
     cudaEvent_t tl_ev[8] = {nullptr}; double tl_ms[8] = {0}; // debug GPU timeline stamps of process_frame
@@ -1274,19 +1274,32 @@ static int sc_knn(liorf_ctx* c, liorf_ctx::KeySet& ks, int n_keys, const float* 
 }
 static liorf_ctx::KeySet& local_keys(liorf_ctx* c) { c->ks_local.keys = c->sc_keys.p; c->ks_local.n = c->sc_n; return c->ks_local; }
 
-// stage 2 for a batch of (query, candidate) pairs: TMA-staged kernel (sc_distance.cuh), persistent warps over the pairs
+// shared-memory limit and occupancy of both instantiations of the stage-2 kernel, once per context
+static int scdb_setup(liorf_ctx* c) {
+    if (c->scdb_attr_set) return LIORF_OK;
+    int occ = 0;
+    CUDA_TRY(cudaFuncSetAttribute(k_sc_distance_bulk<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, SCDB_SMEM));
+    CUDA_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, k_sc_distance_bulk<false>, SCDB_THREADS, SCDB_SMEM));
+    c->scdb_blocks_per_sm[0] = occ > 0 ? occ : 1;
+    CUDA_TRY(cudaFuncSetAttribute(k_sc_distance_bulk<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, SCDB_SMEM));
+    CUDA_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, k_sc_distance_bulk<true>, SCDB_THREADS, SCDB_SMEM));
+    c->scdb_blocks_per_sm[1] = occ > 0 ? occ : 1;
+    c->scdb_attr_set = true;
+    return LIORF_OK;
+}
+
+// stage 2 for a batch of (query, candidate) pairs: TMA-staged kernel (sc_distance.cuh), persistent warps over the pairs.
+// Query descriptors need only 8-byte alignment: a 16-byte-aligned array takes the kernel's 16-byte loads, any other the scalar-load
+// instantiation (same results).  Every launch of k_sc_distance_bulk goes through here.
 static int sc_distance_launch(liorf_ctx* c, const double* qd, const int* cand, int pairs, int global_offset, double* pd, int* ps,
                               const int* pair_list = nullptr, const int* n_list = nullptr, const ShardPush* push = nullptr) {
-    if (!c->scdb_attr_set) {
-        CUDA_TRY(cudaFuncSetAttribute(k_sc_distance_bulk, cudaFuncAttributeMaxDynamicSharedMemorySize, SCDB_SMEM));
-        int occ = 0;
-        CUDA_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, k_sc_distance_bulk, SCDB_THREADS, SCDB_SMEM));
-        c->scdb_blocks_per_sm = occ > 0 ? occ : 1; c->scdb_attr_set = true;
-    }
+    int rc;
+    if ((rc = scdb_setup(c))) return rc;
+    const bool q16 = ((uintptr_t)qd & 15) == 0;
     // persistent warps, one pair at a time each: the fewest CTAs that still finish in the same number of rounds (a sharded rank owns
     // about pairs / world of the pairs: 5.2 rounds of the full grid are 6 rounds either way, and the CTAs not launched leave their
     // shared memory to the other lanes' kernels)
-    const int cap = c->num_sms * c->scdb_blocks_per_sm;
+    const int cap = c->num_sms * c->scdb_blocks_per_sm[q16];
     const long long est = push ? ((long long)pairs + push->W.world - 1) / push->W.world : pairs;
     const long long rounds = std::max<long long>(1, (est + (long long)cap * SCDB_WARPS - 1) / ((long long)cap * SCDB_WARPS));
     int blocks = (int)((est + rounds * SCDB_WARPS - 1) / (rounds * SCDB_WARPS));
@@ -1294,8 +1307,10 @@ static int sc_distance_launch(liorf_ctx* c, const double* qd, const int* cand, i
     if (blocks < 1) blocks = 1;                                   // a rank that owns no pair still raises its phase-D flag
     ShardPush P; std::memset(&P, 0, sizeof(P));
     if (push) P = *push;
-    k_sc_distance_bulk<<<blocks, SCDB_THREADS, SCDB_SMEM, c->stream>>>(qd, cand, pairs, SC_NUM_CAND, c->sc_desc.p, c->sc_sk.p, c->sc_cn.p, global_offset, c->sc_n,
-                                                                          pd, ps, c->d_err, pair_list, n_list, P);
+    if (q16) k_sc_distance_bulk<true><<<blocks, SCDB_THREADS, SCDB_SMEM, c->stream>>>(qd, cand, pairs, SC_NUM_CAND, c->sc_desc.p, c->sc_sk.p, c->sc_cn.p, global_offset,
+                                                                                    c->sc_n, pd, ps, c->d_err, pair_list, n_list, P);
+    else k_sc_distance_bulk<false><<<blocks, SCDB_THREADS, SCDB_SMEM, c->stream>>>(qd, cand, pairs, SC_NUM_CAND, c->sc_desc.p, c->sc_sk.p, c->sc_cn.p, global_offset,
+                                                                                 c->sc_n, pd, ps, c->d_err, pair_list, n_list, P);
     CUDA_TRY(cudaGetLastError());
     c->launches += 1;
     return LIORF_OK;
@@ -1335,6 +1350,17 @@ int liorf_sc_decide_dev(liorf_ctx* c, const void* d_pair_dist, const void* d_pai
                                                          (int*)d_shift, (double*)d_dist);
     CUDA_TRY(cudaGetLastError());
     c->launches += 1;
+    return LIORF_OK;
+}
+
+/* tests: the stage-2 grid bound: SMs and CTAs per SM of the 16-byte-aligned and the 8-byte-aligned query instantiations */
+int liorf_debug_sc_distance_occupancy(liorf_ctx* c, int out[3]) {
+    LIORF_NVTX;
+    if (!c || !out) return LIORF_ERR_ARG;
+    CUDA_TRY(cudaSetDevice(c->P.device));
+    int rc;
+    if ((rc = scdb_setup(c))) return rc;
+    out[0] = c->num_sms; out[1] = c->scdb_blocks_per_sm[1]; out[2] = c->scdb_blocks_per_sm[0];
     return LIORF_OK;
 }
 

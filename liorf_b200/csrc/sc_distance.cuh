@@ -9,7 +9,7 @@
 // 15.6k 64-bit shared loads per pair, ~1 000 port cycles, and measured 1 570 cycles per pair per SM.  Here a lane owns two ADJACENT
 // columns (2l, 2l+1) and two adjacent shifts:
 //   fine search (:123-144)  the 7 shifts of 2 adjacent columns touch 8 consecutive candidate columns instead of 14 → 8 loads feed 14
-//                           multiply-adds per ring; the query's two columns come as one 16-byte global load;
+//                           multiply-adds per ring; the query's two columns come as one 16-byte global load (two 8-byte loads for an 8-byte-aligned query array);
 //   fastAlignUsingVkey (:93-113)  shift 2l+1 at column k reads what shift 2l read at column k-1 → carried in a register; the new value
 //                           and the next one arrive as one 16-byte load, so do v1[k], v1[k+1] (broadcast);
 // → ~7k shared loads (about 550 port cycles) per pair, same arithmetic in the same order: every fp64 sum keeps the reference's sequential
@@ -29,6 +29,16 @@ constexpr int SCDB_WARP_BYTES = SC_DESC * 8 + SCDB_VK1 * 8 + 7 * SC_SECTOR * 8; 
 constexpr int SCDB_SMEM = SCDB_WARPS * SCDB_WARP_BYTES + SCDB_WARPS * 8;
 static_assert(SCDB_WARP_BYTES % 16 == 0, "per-warp shared-memory block must keep 16-byte alignment");
 
+// Two adjacent columns of one ring of the caller's query descriptor.  kQ16: the descriptor array is 16-byte aligned → one 16-byte load;
+// otherwise (a float64 tensor view at an odd element offset is only 8-byte aligned) two 8-byte loads of the same values.
+template <bool kQ16>
+__device__ __forceinline__ double2 scdb_query_pair(const double* p) {
+    if constexpr (kQ16) return *reinterpret_cast<const double2*>(p);
+    else return make_double2(p[0], p[1]);
+}
+
+// kQ16: qdesc is 16-byte aligned (sc_distance_launch picks the instantiation); both read the same values and compute bit-identical results
+template <bool kQ16>
 __global__ void __launch_bounds__(SCDB_THREADS, 4) k_sc_distance_bulk(const double* __restrict__ qdesc, const int* __restrict__ cand, int n_pairs, int cand_per_query,
                                                                   const double* __restrict__ db_desc, const double* __restrict__ db_sk, const double* __restrict__ db_cn,
                                                                   int own_begin, int own_count, double* __restrict__ out_dist, int* __restrict__ out_shift, int* err_flag,
@@ -69,7 +79,7 @@ __global__ void __launch_bounds__(SCDB_THREADS, 4) k_sc_distance_bulk(const doub
             double suma = 0, sqa = 0, sumb = 0, sqb = 0;
 #pragma unroll
             for (int r = 0; r < SC_RING; ++r) {
-                const double2 v = *reinterpret_cast<const double2*>(sc1 + r * SC_SECTOR + c0);
+                const double2 v = scdb_query_pair<kQ16>(sc1 + r * SC_SECTOR + c0);
                 if (r < SCDB_CHUNK) qa[r] = v;
                 suma += v.x; sqa += v.x * v.x; sumb += v.y; sqb += v.y * v.y;
             }
@@ -142,7 +152,7 @@ __global__ void __launch_bounds__(SCDB_THREADS, 4) k_sc_distance_bulk(const doub
                 double2 qb[SCDB_CHUNK];
                 if (ch + 1 < SC_RING / SCDB_CHUNK) {
 #pragma unroll
-                    for (int u = 0; u < SCDB_CHUNK; ++u) qb[u] = *reinterpret_cast<const double2*>(sc1 + ((ch + 1) * SCDB_CHUNK + u) * SC_SECTOR + c0);
+                    for (int u = 0; u < SCDB_CHUNK; ++u) qb[u] = scdb_query_pair<kQ16>(sc1 + ((ch + 1) * SCDB_CHUNK + u) * SC_SECTOR + c0);
                 }
 #pragma unroll
                 for (int u = 0; u < SCDB_CHUNK; ++u) {

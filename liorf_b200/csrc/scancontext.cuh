@@ -272,7 +272,7 @@ __global__ void __launch_bounds__(64) k_sc_keys_batch(const double* __restrict__
         double s = 0, q = 0;
         for (int r = 0; r < SC_RING; ++r) { double v = s_d[r * SC_SECTOR + t]; s += v; q += v * v; }
         sectorkey[(size_t)e * SC_SECTOR + t] = s / SC_RING;
-        colnorm[(size_t)e * SC_SECTOR + t] = sqrt(q);
+        if (colnorm) colnorm[(size_t)e * SC_SECTOR + t] = sqrt(q);
     }
 }
 
