@@ -276,6 +276,22 @@ typedef struct {
 int liorf_loop_closure_icp(liorf_ctx* ctx, int loop_key_cur, int loop_key_pre, int history_search_num, int loop_index, float icp_leaf, float max_corr_dist,
                            int max_iters, liorf_icp_result* out);
 int liorf_icp_get_clouds(liorf_ctx* ctx, liorf_point* source, int cap_source, liorf_point* target, int cap_target);   /* test hook */
+/* performSCLoopClosure's registration for n_pairs keyframe pairs at once (batched verification of loop-closure candidates): pair p is
+ * exactly liorf_loop_closure_icp(ctx, loop_key_cur[p], loop_key_pre[p], history_search_num, loop_index[p], icp_leaf, max_corr_dist,
+ * max_iters, &out[p]) — every field of out[p] bit-identical to that call, whatever the batch size, order or grouping.  Duplicate pairs
+ * and cur == pre are allowed; a pair that fails the size guards gets ran = 0 with n_source / n_target filled in while the others run.
+ * Every argument is checked before any work is enqueued: a NULL array (n_pairs > 0), a key outside [0, n_keyframes), a loop_index
+ * outside [-1, n_keyframes) or a scalar the single-pair call refuses returns LIORF_ERR_ARG with out untouched; n_pairs = 0 is LIORF_OK.
+ * The pairs run in waves of consecutive pairs whose work buffers fit LIORF_ICP_BATCH_WAVE_BYTES of device memory (96 B per raw point
+ * of the two selections plus 16 MiB of grid cells per pair, at most 256 pairs; a larger pair runs alone).  The buffers are the call's
+ * own and stay allocated with the context, sized by the largest wave so far.  A wave synchronises with the host once after its clouds
+ * are built, once per 8 ICP iterations and once for the fitness scores, independently of its pair count; the batch checks the device
+ * error flag once.  liorf_icp_get_clouds keeps returning the clouds of the last single-pair call; keyframes, local map and front
+ * end are not touched. */
+#define LIORF_ICP_BATCH_WAVE_BYTES (4ull << 30)
+int liorf_loop_closure_icp_batch(liorf_ctx* ctx, const int* loop_key_cur, const int* loop_key_pre, const int* loop_index, int n_pairs,
+                                 int history_search_num, float icp_leaf, float max_corr_dist, int max_iters, liorf_icp_result* out);
+int liorf_debug_icp_batch_wave(liorf_ctx* ctx, int max_pairs);   /* tests: at most max_pairs pairs per internal wave (0 = the memory-bounded default) */
 
 /* ---- global map (SURVEY §8f-4) ---------------------------------------------------------------------------------- */
 /* mapOptimization::publishGlobalMap (src/mapOptmization.cpp:453-502): key poses within search_radius

@@ -454,6 +454,33 @@ class Context:
                                              C.c_float(icp_leaf), C.c_float(max_corr_dist), C.c_int(max_iters), C.byref(r)), "liorf_loop_closure_icp")
         return r
 
+    def loopClosureICPBatch(self, cur, pre, loop_index, history_search_num=25, icp_leaf=0.5, max_corr_dist=20.0, max_iters=100, as_arrays=False):
+        """loopClosureICP for many pairs in one call (liorf_loop_closure_icp_batch): pair p is loopClosureICP(cur[p], pre[p], history_search_num,
+        loop_index[p], ...) bit for bit.  loop_index: one value per pair, or a scalar for all.  Returns a ctypes array of IcpResult, or with
+        as_arrays=True a dict of numpy arrays with the same field names (transform as (n, 4, 4), pose6 as (n, 6))."""
+        cur = np.ascontiguousarray(cur, np.int32).reshape(-1)
+        pre = np.ascontiguousarray(pre, np.int32).reshape(-1)
+        li = np.ascontiguousarray(np.broadcast_to(np.asarray(loop_index, np.int32), cur.shape), np.int32)
+        if pre.shape != cur.shape:
+            raise ValueError("cur and pre must have the same length")
+        n = len(cur)
+        out = (IcpResult * max(n, 1))()
+        _chk(self.lib.liorf_loop_closure_icp_batch(self.h, _vp(cur), _vp(pre), _vp(li), C.c_int(n), C.c_int(history_search_num), C.c_float(icp_leaf),
+                                                   C.c_float(max_corr_dist), C.c_int(max_iters), out), "liorf_loop_closure_icp_batch")
+        res = (IcpResult * n).from_buffer(out) if n else (IcpResult * 0)()
+        if not as_arrays:
+            return res
+        d = {}
+        for f, t in IcpResult._fields_:
+            dt = np.int32 if t is C.c_int else np.float32
+            v = np.array([np.array(getattr(r, f), dt) for r in res], dt)
+            d[f] = v.reshape(n, 4, 4) if f == "transform" else v.reshape(n, 6) if f == "pose6" else v.reshape(n)
+        return d
+
+    def debugIcpBatchWave(self, max_pairs):
+        """tests: at most max_pairs pairs per internal wave of loopClosureICPBatch (0 = the memory-bounded default)"""
+        _chk(self.lib.liorf_debug_icp_batch_wave(self.h, C.c_int(max_pairs)), "liorf_debug_icp_batch_wave")
+
     def icpClouds(self, n_source, n_target):
         s = np.empty((max(n_source, 1), 4), np.float32); t = np.empty((max(n_target, 1), 4), np.float32)
         _chk(self.lib.liorf_icp_get_clouds(self.h, _vp(s), C.c_int(n_source), _vp(t), C.c_int(n_target)), "liorf_icp_get_clouds")

@@ -15,6 +15,7 @@
 #include "sc_shard.cuh"
 #include "sc_distance.cuh"
 #include "icp.cuh"
+#include "icp_batch.cuh"
 #include "../host/host_logic.hpp"
 #include <vector>
 #include <cstring>
@@ -108,6 +109,16 @@ struct liorf_ctx {
     // loop-closure ICP (icp.cuh)
     DevBuf<float4> icp_raw, icp_src, icp_src0, icp_tgt; MapGrid icp_grid; DevBuf<double> icp_partial; double* icp_out = nullptr; int* icp_counter = nullptr;
     DevBuf<KfSel> icp_sel; DevBuf<int> icp_nn_idx; DevBuf<float> icp_nn_d2;
+    // batched loop-closure ICP (icp_batch.cuh): work buffers of its own, sized by the largest wave so far
+    struct IcpBatch {
+        DevBuf<KfSel> sel; DevBuf<VgSegTile> tiles; DevBuf<int> seg_n, seg_vox, counters; DevBuf<unsigned> mm, keys, seg_start, counts, cell_start;
+        DevBuf<VoxMeta> metas; DevBuf<unsigned long long> seg_base; DevBuf<float4> raw, vox, src_cur, sorted;
+        DevBuf<IcpPairDesc> pd; DevBuf<int2> act; DevBuf<IcpState> st; DevBuf<double> partial, fit;
+        SortWork sort; ScanWork scan, grid_scan;
+        int* d_flags = nullptr;                 // [0] voxel total of the wave, [1] key range beyond 32 bits
+        unsigned char* h_stage = nullptr; size_t h_cap = 0;      // pinned: tables going up, counts / states / sums coming back
+        int max_pairs = 0;                      // tests: pairs per wave (0 = memory-bounded)
+    } icpb;
     liorf_guess_state guess_state = {}; float tf_mapped[6] = {0, 0, 0, 0, 0, 0};   // updateInitialGuess statics + transformTobeMapped
     // sharded search over peer windows (sc_shard.cuh)
     struct ScShard { bool ready = false; ShardWin W; int qmax = 0, kcap = 0; size_t win_bytes = 0, off_keys = 0; unsigned* d_batch = nullptr; unsigned* d_counter = nullptr;
@@ -335,6 +346,10 @@ int liorf_create(const liorf_params* p, liorf_ctx** out) {
     c->vg_map.sort.ticket = c->d_tick + 5; c->vg_map.sort.err_flag = c->d_err;
     c->vg_map.scan.ticket = c->d_tick + 6; c->vg_map.scan.err_flag = c->d_err;
     c->icp_grid.scan.ticket = c->d_tick + 7; c->icp_grid.scan.err_flag = c->d_err;
+    c->icpb.sort.ticket = c->d_tick + 11; c->icpb.sort.err_flag = c->d_err;
+    c->icpb.scan.ticket = c->d_tick + 12; c->icpb.scan.err_flag = c->d_err;
+    c->icpb.grid_scan.ticket = c->d_tick + 13; c->icpb.grid_scan.err_flag = c->d_err;
+    CUDA_TRY(cudaMalloc(&c->icpb.d_flags, 2 * sizeof(int)));
     CUDA_TRY(cudaMalloc(&c->dk.start_inv, 12 * sizeof(float)));
     c->dk.first_kept = c->d_counts + C_FIRST_KEPT;
     // the alternate front set: its own look-back tickets, VoxelGrid meta and deskew scalars
@@ -447,6 +462,16 @@ void liorf_destroy(liorf_ctx* c) {
     c->icp_raw.release(); c->icp_src.release(); c->icp_src0.release(); c->icp_tgt.release(); c->icp_partial.release(); c->icp_sel.release(); c->icp_nn_idx.release();
     c->icp_nn_d2.release(); c->icp_grid.counts.release(); c->icp_grid.cell_start.release(); c->icp_grid.sorted.release(); c->icp_grid.scan.status.release();
     if (c->icp_out) cudaFree(c->icp_out);
+    {
+        liorf_ctx::IcpBatch& B = c->icpb;
+        B.sel.release(); B.tiles.release(); B.seg_n.release(); B.seg_vox.release(); B.counters.release(); B.mm.release(); B.keys.release(); B.seg_start.release();
+        B.counts.release(); B.cell_start.release(); B.metas.release(); B.seg_base.release(); B.raw.release(); B.vox.release(); B.src_cur.release(); B.sorted.release();
+        B.pd.release(); B.act.release(); B.st.release(); B.partial.release(); B.fit.release();
+        B.sort.keys_alt.release(); B.sort.vals_a.release(); B.sort.vals_b.release(); B.sort.hist.release(); B.sort.status.release();
+        B.scan.status.release(); B.grid_scan.status.release();
+        if (B.d_flags) cudaFree(B.d_flags);
+        if (B.h_stage) cudaFreeHost(B.h_stage);
+    }
     if (c->sct_over_cnt) cudaFree(c->sct_over_cnt);
     for (VoxelGridWork* vw : {&c->vg, &c->vg_map, &c->alt.vg}) {
         vw->pts_sorted.release(); vw->cta_hist.release(); vw->cta_heads.release();
@@ -1786,19 +1811,28 @@ int liorf_sc_detect_loop_closure_id(liorf_ctx* c, int* loop_id, float* yaw_diff_
 // ------------------------------------------------------------------------------------------------ loop-closure ICP
 // clouds of loopFindNearKeyframes (:821-844) as performSCLoopClosure calls it (:652-653): every selected keyframe cloud is
 // transformed by the pose of keyframe `loop_index` (the reference passes base_key = 0), concatenated, VoxelGrid(icp leaf).
-static int icp_build_cloud(liorf_ctx* c, int key, int search_num, int loop_index, float leaf, DevBuf<float4>& out, int* n_out) {
-    int rc;
-    std::vector<KfSel> sel; long long total = 0;
+// loopFindNearKeyframes' selection (:826-835): keyframes key-search_num .. key+search_num that exist, in order; appends to sel with
+// destination offsets continuing from `total`.  sel == nullptr only counts the points.
+static void icp_select(const liorf_ctx* c, int key, int search_num, int loop_index, std::vector<KfSel>* sel, long long& total) {
     const int n_kf = (int)c->kfs.size();
     for (int i = -search_num; i <= search_num; ++i) {
         const int kn = key + i;
         if (kn < 0 || kn >= n_kf) continue;
         const Keyframe& k = c->kfs[kn];
-        const Keyframe& pk = c->kfs[loop_index != -1 ? loop_index : kn];
-        KfSel s; s.src_off = (int)k.off; s.count = k.count; s.dst_off = (int)total; s.pad = 0;
-        host_get_transformation(pk.pose[3], pk.pose[4], pk.pose[5], pk.pose[0], pk.pose[1], pk.pose[2], s.t);
-        total += k.count; sel.push_back(s);
+        if (sel) {
+            const Keyframe& pk = c->kfs[loop_index != -1 ? loop_index : kn];
+            KfSel s; s.src_off = (int)k.off; s.count = k.count; s.dst_off = (int)total; s.pad = 0;
+            host_get_transformation(pk.pose[3], pk.pose[4], pk.pose[5], pk.pose[0], pk.pose[1], pk.pose[2], s.t);
+            sel->push_back(s);
+        }
+        total += k.count;
     }
+}
+
+static int icp_build_cloud(liorf_ctx* c, int key, int search_num, int loop_index, float leaf, DevBuf<float4>& out, int* n_out) {
+    int rc;
+    std::vector<KfSel> sel; long long total = 0;
+    icp_select(c, key, search_num, loop_index, &sel, total);
     *n_out = 0;
     if (sel.empty() || total == 0) return LIORF_OK;
     if (total > 0x7fffffffLL) return LIORF_ERR_ARG;
@@ -1813,6 +1847,24 @@ static int icp_build_cloud(liorf_ctx* c, int key, int search_num, int loop_index
     *n_out = c->h_mail[900];
     c->launches += 10;
     return LIORF_OK;
+}
+
+// the result fields of a pair that ran, from the loop state and getFitnessScore's two sums (shared by the single and the batched call)
+static void icp_fill_result(const IcpState& hs, const double* fit_sums, liorf_icp_result* out) {
+    out->ran = 1;
+    out->iterations = hs.iterations;
+    out->converged = hs.converged ? 1 : 0; out->convergence_state = (int)hs.cc.state;
+    std::memcpy(out->transform, hs.final_T, sizeof(hs.final_T));
+    out->fitness = fit_sums[1] > 0 ? (float)(fit_sums[0] / fit_sums[1]) : 3.4028235e38f;
+    float t12[12]; for (int r = 0; r < 3; ++r) for (int k = 0; k < 4; ++k) t12[4 * r + k] = hs.final_T[4 * r + k];
+    liorf_host::get_translation_and_euler(t12, out->pose6[3], out->pose6[4], out->pose6[5], out->pose6[0], out->pose6[1], out->pose6[2]);   // :693
+}
+constexpr int ICP_CHUNK = 8;                         // iterations enqueued between two read-backs of the loop state
+static IcpState icp_initial_state(int max_iters) {
+    IcpState hs; std::memset(&hs, 0, sizeof(hs));
+    hs.cc = liorf_host::IcpConvergence(); hs.cc.max_iterations = max_iters;
+    for (int i = 0; i < 4; ++i) hs.inc[5 * i] = hs.final_T[5 * i] = 1.f;
+    return hs;
 }
 
 int liorf_loop_closure_icp(liorf_ctx* c, int loop_key_cur, int loop_key_pre, int history_search_num, int loop_index, float icp_leaf, float max_corr_dist,
@@ -1841,12 +1893,9 @@ int liorf_loop_closure_icp(liorf_ctx* c, int loop_key_cur, int loop_key_pre, int
     const float max_d2 = max_corr_dist * max_corr_dist;
     // the loop runs on the device (csrc/icp.cuh): iterations are enqueued in chunks and the state is read back once per chunk
     if (!c->icp_state) CUDA_TRY(cudaMalloc(&c->icp_state, sizeof(IcpState)));
-    IcpState hs; std::memset(&hs, 0, sizeof(hs));
-    hs.cc = liorf_host::IcpConvergence(); hs.cc.max_iterations = max_iters;
-    for (int i = 0; i < 4; ++i) hs.inc[5 * i] = hs.final_T[5 * i] = 1.f;
+    IcpState hs = icp_initial_state(max_iters);
     CUDA_TRY(cudaMemcpyAsync(c->icp_state, &hs, sizeof(hs), cudaMemcpyHostToDevice, c->stream));
     CUDA_TRY(cudaStreamSynchronize(c->stream));                       // hs is pageable: the copy must have left it before it is reused below
-    constexpr int ICP_CHUNK = 8;
     int enq = 0;
     while (!hs.done && enq < max_iters) {
         const int todo = std::min(ICP_CHUNK, max_iters - enq);
@@ -1857,26 +1906,18 @@ int liorf_loop_closure_icp(liorf_ctx* c, int loop_key_cur, int loop_key_pre, int
         CUDA_TRY(cudaMemcpyAsync(&hs, c->icp_state, sizeof(hs), cudaMemcpyDeviceToHost, c->stream));
         CUDA_TRY(cudaStreamSynchronize(c->stream));
     }
-    const bool converged = hs.converged != 0;
-    liorf_host::IcpConvergence cc = hs.cc;
-    float final_T[16]; std::memcpy(final_T, hs.final_T, sizeof(final_T));
-    out->iterations = hs.iterations;
     double* h_sums = reinterpret_cast<double*>(c->h_mail + 3000);   // 8-byte aligned slot of the pinned mailbox
-    out->converged = converged ? 1 : 0; out->convergence_state = (int)cc.state;
-    std::memcpy(out->transform, final_T, sizeof(final_T));
     // getFitnessScore(): the original source under the final transformation, no range limit
     {
-        IcpT Tf; std::memcpy(Tf.t, final_T, 12 * sizeof(float));
+        IcpT Tf; std::memcpy(Tf.t, hs.final_T, 12 * sizeof(float));
         const int rfit = 64;
         k_icp_fitness<<<blocks, ICP_BLOCK, 0, c->stream>>>(c->icp_src0.p, n_src, Tf, c->icp_grid.cell_start.p, c->icp_grid.sorted.p, c->icp_grid.dims, rfit, c->icp_partial.p,
                                                          c->icp_counter, c->icp_out);
         CUDA_TRY(cudaMemcpyAsync(h_sums, c->icp_out, 2 * sizeof(double), cudaMemcpyDeviceToHost, c->stream));
         CUDA_TRY(cudaStreamSynchronize(c->stream));
         ++c->launches;
-        out->fitness = h_sums[1] > 0 ? (float)(h_sums[0] / h_sums[1]) : 3.4028235e38f;
     }
-    float t12[12]; for (int r = 0; r < 3; ++r) for (int k = 0; k < 4; ++k) t12[4 * r + k] = final_T[4 * r + k];
-    liorf_host::get_translation_and_euler(t12, out->pose6[3], out->pose6[4], out->pose6[5], out->pose6[0], out->pose6[1], out->pose6[2]);   // :693
+    icp_fill_result(hs, h_sums, out);
     return check_err(c);
 }
 /* test hook: the two clouds of the last liorf_loop_closure_icp (cureKeyframeCloud / prevKeyframeCloud after the ICP VoxelGrid) */
@@ -1887,6 +1928,214 @@ int liorf_icp_get_clouds(liorf_ctx* c, liorf_point* source, int cap_source, lior
     CUDA_TRY(cudaStreamSynchronize(c->stream));
     if (source && cap_source > 0) CUDA_TRY(cudaMemcpy(source, c->icp_src0.p, (size_t)cap_source * sizeof(float4), cudaMemcpyDeviceToHost));
     if (target && cap_target > 0) CUDA_TRY(cudaMemcpy(target, c->icp_tgt.p, (size_t)cap_target * sizeof(float4), cudaMemcpyDeviceToHost));
+    return LIORF_OK;
+}
+
+// ------------------------------------------------------------------------------------------------ batched loop-closure ICP
+// liorf_loop_closure_icp for many pairs (icp_batch.cuh).  Pairs run in waves bounded by ICPB_WAVE_BYTES of work buffers; a wave costs
+// one host synchronisation after its clouds are built (voxel counts per cloud), one per chunk of ICP_CHUNK iterations, one for the
+// fitness sums, and the batch one error check — however many pairs the wave holds.
+constexpr size_t ICPB_WAVE_BYTES = LIORF_ICP_BATCH_WAVE_BYTES;
+constexpr size_t ICPB_BYTES_PER_POINT = 96;          // raw + voxel + working copy + cell-sorted copy (16 B each), sort keys / values / heads
+constexpr size_t ICPB_GRID_BYTES = (size_t)256 * 256 * 32 * 2 * sizeof(unsigned);      // per pair: cell counts + cell starts
+constexpr int ICPB_MAX_PAIRS = 256;                  // 512 clouds per wave; 2^29 grid cells
+
+struct IcpbPair { int cur, pre, li; long long raw_src, raw_tgt; };
+
+static int icpb_stage(liorf_ctx* c, size_t bytes) {   // pinned staging (grows between waves, when the stream is idle)
+    liorf_ctx::IcpBatch& B = c->icpb;
+    if (bytes <= B.h_cap) return LIORF_OK;
+    if (B.h_stage) { CUDA_TRY(cudaStreamSynchronize(c->stream)); CUDA_TRY(cudaFreeHost(B.h_stage)); B.h_stage = nullptr; B.h_cap = 0; }
+    const size_t cap = std::max<size_t>(bytes, 1 << 20);
+    CUDA_TRY(cudaHostAlloc(&B.h_stage, cap, cudaHostAllocDefault));
+    B.h_cap = cap;
+    return LIORF_OK;
+}
+
+// one wave: pairs P[0 .. W).  *split = 1 (nothing written to out) when the wave's VoxelGrid keys need more than 32 bits: the caller halves it.
+static int icpb_wave(liorf_ctx* c, const IcpbPair* P, int W, liorf_icp_result* const* out, int history_search_num, float leaf, float max_corr_dist,
+                     int max_iters, int* split) {
+    liorf_ctx::IcpBatch& B = c->icpb;
+    cudaStream_t s = c->stream;
+    int rc;
+    *split = 0;
+    // ---- selections of all 2 W clouds (cloud 2 j = pair j's source, 2 j + 1 its target), one tile table over them ----
+    const int S = 2 * W;
+    std::vector<KfSel> sel; std::vector<int> seg_n(S), seg_first(S); std::vector<VgSegTile> tiles;
+    long long total = 0;
+    for (int j = 0; j < W; ++j)
+        for (int side = 0; side < 2; ++side) {
+            const int sg = 2 * j + side;
+            const long long t0 = total;
+            if (side == 0) icp_select(c, P[j].cur, 0, P[j].li, &sel, total);                    // cureKeyframeCloud  (:652)
+            else icp_select(c, P[j].pre, history_search_num, P[j].li, &sel, total);            // prevKeyframeCloud  (:653)
+            seg_first[sg] = (int)t0; seg_n[sg] = (int)(total - t0);
+            for (long long b = t0; b < total; b += VGSEG_TILE) tiles.push_back(VgSegTile{sg, (int)b, (int)std::min<long long>(b + VGSEG_TILE, total), 0});
+        }
+    const int tot = (int)total, ns = (int)sel.size(), nt = (int)tiles.size();
+    // pinned staging: [up: sel | tiles | seg_n | seg_first | pair table | act (2 W) | states]  [down: seg_vox | flags | states | fitness sums]
+    size_t off = 0;
+    auto take = [&](size_t bytes) { const size_t o = off; off += (bytes + 255) & ~(size_t)255; return o; };
+    const size_t o_sel = take((size_t)ns * sizeof(KfSel)), o_tiles = take((size_t)nt * sizeof(VgSegTile)), o_segn = take((size_t)2 * S * sizeof(int));
+    const size_t o_pd = take((size_t)W * sizeof(IcpPairDesc)), o_act = take((size_t)2 * W * sizeof(int2)), o_st = take((size_t)W * sizeof(IcpState));
+    const size_t o_vox = take((size_t)2 * S * sizeof(int) + 2 * sizeof(int)), o_stb = take((size_t)W * sizeof(IcpState)), o_fit = take((size_t)2 * W * sizeof(double));
+    if ((rc = icpb_stage(c, off))) return rc;
+    unsigned char* H = B.h_stage;
+    int* h_vox = reinterpret_cast<int*>(H + o_vox);           // [2 S] (first voxel, count) per cloud, then the two flags
+    if (tot > 0) {
+        std::memcpy(H + o_sel, sel.data(), (size_t)ns * sizeof(KfSel));
+        std::memcpy(H + o_tiles, tiles.data(), (size_t)nt * sizeof(VgSegTile));
+        std::memcpy(H + o_segn, seg_n.data(), (size_t)S * sizeof(int)); std::memcpy(H + o_segn + (size_t)S * sizeof(int), seg_first.data(), (size_t)S * sizeof(int));
+        if ((rc = B.sel.reserve(ns)) || (rc = B.tiles.reserve(nt)) || (rc = B.seg_n.reserve((size_t)2 * S)) || (rc = B.seg_vox.reserve((size_t)2 * S)) ||
+            (rc = B.mm.reserve((size_t)6 * S)) || (rc = B.metas.reserve(S)) || (rc = B.seg_base.reserve((size_t)S + 1)) || (rc = B.raw.reserve(tot)) ||
+            (rc = B.keys.reserve(tot)) || (rc = B.seg_start.reserve((size_t)tot + 1)) || (rc = B.vox.reserve(tot))) return rc;
+        CUDA_TRY(cudaMemcpyAsync(B.sel.p, H + o_sel, (size_t)ns * sizeof(KfSel), cudaMemcpyHostToDevice, s));
+        CUDA_TRY(cudaMemcpyAsync(B.tiles.p, H + o_tiles, (size_t)nt * sizeof(VgSegTile), cudaMemcpyHostToDevice, s));
+        CUDA_TRY(cudaMemcpyAsync(B.seg_n.p, H + o_segn, (size_t)2 * S * sizeof(int), cudaMemcpyHostToDevice, s));
+        CUDA_TRY(cudaMemsetAsync(B.mm.p, 0xff, (size_t)3 * S * sizeof(unsigned), s));
+        CUDA_TRY(cudaMemsetAsync(B.mm.p + 3 * S, 0, (size_t)3 * S * sizeof(unsigned), s));
+        // ---- the clouds: one transform + concat, then the segmented VoxelGrid (voxelgrid.cuh) ----
+        k_transform_concat<<<(tot + 255) / 256, 256, 0, s>>>(c->kf_points.p, B.sel.p, ns, tot, B.raw.p);
+        k_vgseg_bounds<<<nt, 256, 0, s>>>(B.raw.p, B.tiles.p, B.mm.p, B.mm.p + 3 * S);
+        k_vgseg_meta<<<1, 1024, 0, s>>>(B.seg_n.p, S, B.mm.p, B.mm.p + 3 * S, leaf, B.metas.p, B.seg_base.p, B.d_flags + 1);
+        k_vgseg_keys<<<nt, 256, 0, s>>>(B.raw.p, B.tiles.p, B.seg_n.p + S, B.metas.p, B.seg_base.p, B.keys.p);
+        unsigned* sorted_idx = nullptr;
+        const Count cnt = Count::of_host(tot);
+        if ((rc = radix_sort_pairs_iota(B.keys.p, cnt, B.sort, &sorted_idx, s))) return rc;
+        if ((rc = launch_scan(cnt, VgHeadLoad{B.keys.p}, VgHeadStore{B.seg_start.p, cnt}, B.scan, (unsigned*)B.d_flags, s))) return rc;
+        k_vg_centroid<<<(tot + 127) / 128, 128, 0, s>>>(B.raw.p, sorted_idx, B.seg_start.p, (const unsigned*)B.d_flags, B.vox.p, nullptr, B.keys.p, nullptr);
+        k_vgseg_out<<<(S + 255) / 256, 256, 0, s>>>(B.keys.p, B.seg_start.p, (const unsigned*)B.d_flags, B.seg_base.p, S, B.seg_vox.p);
+        CUDA_TRY(cudaGetLastError());
+        c->launches += 16;
+        CUDA_TRY(cudaMemcpyAsync(h_vox, B.seg_vox.p, (size_t)2 * S * sizeof(int), cudaMemcpyDeviceToHost, s));
+        CUDA_TRY(cudaMemcpyAsync(h_vox + 2 * S, B.d_flags, 2 * sizeof(int), cudaMemcpyDeviceToHost, s));
+        CUDA_TRY(cudaStreamSynchronize(s));                                    // sync 1: voxel counts of every cloud
+        if (h_vox[2 * S + 1] && W > 1) { *split = 1; return LIORF_OK; }
+    } else {
+        std::memset(h_vox, 0, (size_t)(2 * S + 2) * sizeof(int));
+    }
+    const int n_vox = h_vox[2 * S];
+    // ---- guards (:655-656); the pairs that run get the single-pair call's block partition ----
+    std::vector<IcpPairDesc> pd; std::vector<int> slot_of;       // slot_of[q] = the wave's pair j
+    int blocks_total = 0, tgt_total = 0;
+    for (int j = 0; j < W; ++j) {
+        liorf_icp_result* o = out[j];
+        std::memset(o, 0, sizeof(*o));
+        for (int i = 0; i < 4; ++i) o->transform[5 * i] = 1.f;
+        const int so = h_vox[4 * j], sn = h_vox[4 * j + 1], to = h_vox[4 * j + 2], tn = h_vox[4 * j + 3];
+        o->n_source = sn; o->n_target = tn;
+        if (sn < 300 || tn < 1000) continue;
+        IcpPairDesc d;
+        d.src_off = so; d.n_src = sn; d.tgt_off = to; d.n_tgt = tn; d.tgt_first = tgt_total; d.part_off = blocks_total; d.pad = 0;
+        d.blocks = (sn + ICP_BLOCK - 1) / ICP_BLOCK; if (d.blocks > 4 * c->num_sms) d.blocks = 4 * c->num_sms;
+        blocks_total += d.blocks; tgt_total += tn;
+        pd.push_back(d); slot_of.push_back(j);
+    }
+    const int R = (int)pd.size();
+    if (R == 0) return LIORF_OK;
+    // ---- per-pair target grids in one pass ----
+    const GridDims g = c->icp_grid.dims;                           // the single-pair call's torus (icp_batch.cuh: why not smaller)
+    const int NC = grid_cells(g);
+    IcpPairDesc* h_pd = reinterpret_cast<IcpPairDesc*>(H + o_pd);
+    int2* h_act = reinterpret_cast<int2*>(H + o_act);               // [0, R) every pair (fitness), [R, 2 R) the pairs still running
+    IcpState* h_st = reinterpret_cast<IcpState*>(H + o_st);
+    IcpState* h_stb = reinterpret_cast<IcpState*>(H + o_stb);
+    double* h_fit = reinterpret_cast<double*>(H + o_fit);
+    std::memcpy(h_pd, pd.data(), (size_t)R * sizeof(IcpPairDesc));
+    for (int q = 0; q < R; ++q) { h_act[q] = make_int2(q, pd[q].part_off); h_act[R + q] = h_act[q]; h_st[q] = icp_initial_state(max_iters); }
+    if ((rc = B.pd.reserve(R)) || (rc = B.act.reserve((size_t)2 * R)) || (rc = B.st.reserve(R)) || (rc = B.fit.reserve((size_t)2 * R)) ||
+        (rc = B.partial.reserve((size_t)blocks_total * ICP_NSUM)) || (rc = reserve_zeroed(B.counters, R, s)) || (rc = reserve_zeroed(B.counts, (size_t)R * NC, s)) ||
+        (rc = B.cell_start.reserve((size_t)R * NC + 1)) || (rc = B.sorted.reserve(tgt_total)) || (rc = B.src_cur.reserve(n_vox))) return rc;
+    const int gtiles = (int)(((size_t)R * NC + GSCAN_TILE - 1) / GSCAN_TILE);
+    if ((rc = reserve_zeroed(B.grid_scan.status, gtiles, s))) return rc;
+    CUDA_TRY(cudaMemcpyAsync(B.pd.p, h_pd, (size_t)R * sizeof(IcpPairDesc), cudaMemcpyHostToDevice, s));
+    CUDA_TRY(cudaMemcpyAsync(B.act.p, h_act, (size_t)2 * R * sizeof(int2), cudaMemcpyHostToDevice, s));
+    CUDA_TRY(cudaMemcpyAsync(B.st.p, h_st, (size_t)R * sizeof(IcpState), cudaMemcpyHostToDevice, s));
+    k_icpb_grid_count<<<(tgt_total + 255) / 256, 256, 0, s>>>(B.vox.p, B.pd.p, R, tgt_total, g, B.counts.p);
+    k_grid_scan<<<gtiles, GSCAN_BLOCK, 0, s>>>(B.counts.p, B.cell_start.p, R * NC, B.grid_scan.ticket, B.grid_scan.status.p, B.grid_scan.err_flag);
+    k_icpb_grid_scatter<<<(tgt_total + 255) / 256, 256, 0, s>>>(B.vox.p, B.pd.p, R, tgt_total, g, B.counts.p, B.cell_start.p, B.sorted.p);
+    CUDA_TRY(cudaMemcpyAsync(B.src_cur.p, B.vox.p, (size_t)n_vox * sizeof(float4), cudaMemcpyDeviceToDevice, s));
+    c->launches += 3;
+    // ---- the ICP loops: one launch per iteration over every pair still running, read back once per chunk ----
+    const int r_max = (int)std::ceil(max_corr_dist) + 1;
+    const float max_d2 = max_corr_dist * max_corr_dist;
+    int n_act = R, act_blocks = blocks_total, enq = 0;
+    while (n_act > 0 && enq < max_iters) {
+        const int todo = std::min(ICP_CHUNK, max_iters - enq);
+        for (int k = 0; k < todo; ++k)
+            k_icpb_iteration<<<act_blocks, ICP_BLOCK, 0, s>>>(B.pd.p, B.act.p + R, n_act, B.src_cur.p, B.st.p, B.cell_start.p, B.sorted.p, g, r_max, max_d2,
+                                                              B.partial.p, B.counters.p);
+        CUDA_TRY(cudaGetLastError());
+        enq += todo; c->launches += todo;
+        CUDA_TRY(cudaMemcpyAsync(h_stb, B.st.p, (size_t)R * sizeof(IcpState), cudaMemcpyDeviceToHost, s));
+        CUDA_TRY(cudaStreamSynchronize(s));                                    // one per chunk
+        n_act = 0; act_blocks = 0;
+        for (int q = 0; q < R; ++q)
+            if (!h_stb[q].done) { h_act[R + n_act++] = make_int2(q, act_blocks); act_blocks += pd[q].blocks; }
+        if (n_act > 0 && enq < max_iters) CUDA_TRY(cudaMemcpyAsync(B.act.p + R, h_act + R, (size_t)n_act * sizeof(int2), cudaMemcpyHostToDevice, s));
+    }
+    // ---- getFitnessScore of every pair that ran ----
+    k_icpb_fitness<<<blocks_total, ICP_BLOCK, 0, s>>>(B.pd.p, B.act.p, R, B.vox.p, B.st.p, B.cell_start.p, B.sorted.p, g, 64, B.partial.p, B.counters.p, B.fit.p);
+    CUDA_TRY(cudaGetLastError());
+    ++c->launches;
+    CUDA_TRY(cudaMemcpyAsync(h_fit, B.fit.p, (size_t)2 * R * sizeof(double), cudaMemcpyDeviceToHost, s));
+    CUDA_TRY(cudaStreamSynchronize(s));                                        // the fitness sums
+    for (int q = 0; q < R; ++q) icp_fill_result(h_stb[q], h_fit + 2 * q, out[slot_of[q]]);
+    return LIORF_OK;
+}
+
+int liorf_loop_closure_icp_batch(liorf_ctx* c, const int* loop_key_cur, const int* loop_key_pre, const int* loop_index, int n_pairs, int history_search_num,
+                                 float icp_leaf, float max_corr_dist, int max_iters, liorf_icp_result* out) {
+    LIORF_NVTX;
+    if (!c || n_pairs < 0 || (n_pairs > 0 && (!loop_key_cur || !loop_key_pre || !loop_index || !out))) return LIORF_ERR_ARG;
+    if (history_search_num < 0 || max_iters < 1 || !(icp_leaf > 0.f) || !(max_corr_dist > 0.f)) return LIORF_ERR_ARG;
+    const int n_kf = (int)c->kfs.size();
+    std::vector<IcpbPair> P(n_pairs);
+    for (int p = 0; p < n_pairs; ++p) {
+        const int cur = loop_key_cur[p], pre = loop_key_pre[p], li = loop_index[p];
+        if (cur < 0 || cur >= n_kf || pre < 0 || pre >= n_kf || li < -1 || li >= n_kf) return LIORF_ERR_ARG;
+        IcpbPair& q = P[p]; q.cur = cur; q.pre = pre; q.li = li; q.raw_src = 0; q.raw_tgt = 0;
+        icp_select(c, cur, 0, li, nullptr, q.raw_src);
+        icp_select(c, pre, history_search_num, li, nullptr, q.raw_tgt);
+        if (q.raw_src > 0x7fffffffLL || q.raw_tgt > 0x7fffffffLL || q.raw_src + q.raw_tgt > 0x7fffffffLL) return LIORF_ERR_ARG;     // as the single-pair call
+    }
+    if (n_pairs == 0) return LIORF_OK;
+    CUDA_TRY(cudaSetDevice(c->P.device));
+    int rc;
+    if ((rc = join_map(c))) return rc;
+    // waves: consecutive pairs while their work buffers fit the budget (a pair larger than the budget runs alone)
+    std::vector<std::pair<int, int>> waves;
+    {
+        const int cap = c->icpb.max_pairs > 0 ? std::min(c->icpb.max_pairs, ICPB_MAX_PAIRS) : ICPB_MAX_PAIRS;
+        int b = 0; size_t bytes = 0; long long pts = 0;
+        for (int p = 0; p < n_pairs; ++p) {
+            const long long pp = P[p].raw_src + P[p].raw_tgt;
+            const size_t pb = (size_t)pp * ICPB_BYTES_PER_POINT + ICPB_GRID_BYTES;
+            if (p > b && (p - b >= cap || bytes + pb > ICPB_WAVE_BYTES || pts + pp > 0x7fffffffLL)) { waves.push_back({b, p}); b = p; bytes = 0; pts = 0; }
+            bytes += pb; pts += pp;
+        }
+        waves.push_back({b, n_pairs});
+    }
+    std::vector<liorf_icp_result> res(n_pairs);
+    std::vector<liorf_icp_result*> res_ptr(n_pairs);
+    for (int p = 0; p < n_pairs; ++p) res_ptr[p] = &res[p];
+    for (size_t w = 0; w < waves.size(); ++w) {
+        const int b = waves[w].first, e = waves[w].second;
+        int split = 0;
+        if ((rc = icpb_wave(c, P.data() + b, e - b, res_ptr.data() + b, history_search_num, icp_leaf, max_corr_dist, max_iters, &split))) return rc;
+        if (split) {                                   // the wave's voxel keys need more than 32 bits: run it as two
+            const int m = b + (e - b) / 2;
+            waves.insert(waves.begin() + w + 1, {{b, m}, {m, e}});
+        }
+    }
+    if ((rc = check_err(c))) return rc;
+    std::memcpy(out, res.data(), (size_t)n_pairs * sizeof(liorf_icp_result));
+    return LIORF_OK;
+}
+/* tests: at most max_pairs pairs per wave (0 = the memory-bounded default) */
+int liorf_debug_icp_batch_wave(liorf_ctx* c, int max_pairs) {
+    if (!c || max_pairs < 0) return LIORF_ERR_ARG;
+    c->icpb.max_pairs = max_pairs;
     return LIORF_OK;
 }
 

@@ -57,12 +57,16 @@ __device__ __forceinline__ bool icp_nearest(const float4 q, const unsigned* __re
     return bi != 0x7fffffff;
 }
 
-// One ICP iteration's device half.  src_cur ← T_inc * src_cur (pcl::transformPointCloud with the previous iteration's
-// estimate; identity on the first), correspondences with squared distance <= max_d2, partial sums → out[ICP_NSUM].
-// want_nn: also store the neighbour index / squared distance per source point (tests, fitness).
-__global__ void __launch_bounds__(ICP_BLOCK) k_icp_iteration(float4* __restrict__ src_cur, int n_src, IcpState* __restrict__ st, const unsigned* __restrict__ cell_start,
-                                                            const float4* __restrict__ gmap, GridDims g, int r_max, float max_d2, double* __restrict__ partial,
-                                                            int* __restrict__ counter, double* __restrict__ out, int* __restrict__ nn_idx, float* __restrict__ nn_d2) {
+// One ICP iteration's device half for ONE cloud pair, run by block `blk` of the `nblk` blocks that pair owns.  src_cur ← T_inc * src_cur
+// (pcl::transformPointCloud with the previous iteration's estimate; identity on the first), correspondences with squared distance
+// <= max_d2, per-block partial sums folded in block order by the pair's last block, which then runs the estimate / convergence step.
+// The block partition (blk, nblk, grid-stride nblk * ICP_BLOCK) is the whole of what fixes the fp64 summation order, so the single-pair
+// kernel and the batched one (icp_batch.cuh) give bit-identical results for the same pair.
+// out (nullable): the folded sums.  nn_idx / nn_d2 (nullable): the neighbour index / squared distance per source point (tests).
+__device__ __forceinline__ void icp_iteration_body(float4* __restrict__ src_cur, int n_src, IcpState* __restrict__ st, const unsigned* __restrict__ cell_start,
+                                                   const float4* __restrict__ gmap, GridDims g, int r_max, float max_d2, double* __restrict__ partial,
+                                                   int* __restrict__ counter, double* __restrict__ out, int* __restrict__ nn_idx, float* __restrict__ nn_d2,
+                                                   int blk, int nblk) {
     __shared__ double s_red[ICP_BLOCK / 32][ICP_NSUM];
     __shared__ bool s_last;
     __shared__ float s_T[12];
@@ -73,7 +77,7 @@ __global__ void __launch_bounds__(ICP_BLOCK) k_icp_iteration(float4* __restrict_
     double acc[ICP_NSUM];
 #pragma unroll
     for (int k = 0; k < ICP_NSUM; ++k) acc[k] = 0.0;
-    for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < n_src; i += gridDim.x * blockDim.x) {
+    for (int i = blk * ICP_BLOCK + threadIdx.x; i < n_src; i += nblk * ICP_BLOCK) {
         const float4 p = apply_affine_dev(s_T, src_cur[i]);
         src_cur[i] = p;
         float bd; int bi; float4 bp;
@@ -95,17 +99,18 @@ __global__ void __launch_bounds__(ICP_BLOCK) k_icp_iteration(float4* __restrict_
     __syncthreads();
     if (threadIdx.x < ICP_NSUM) {
         double s = 0; for (int w = 0; w < ICP_BLOCK / 32; ++w) s += s_red[w][threadIdx.x];
-        partial[blockIdx.x * ICP_NSUM + threadIdx.x] = s;
+        partial[blk * ICP_NSUM + threadIdx.x] = s;
         __threadfence();
     }
     __syncthreads();
-    if (threadIdx.x == 0) { const int t = atomicAdd(counter, 1); s_last = (t == (int)gridDim.x - 1); }
+    if (threadIdx.x == 0) { const int t = atomicAdd(counter, 1); s_last = (t == nblk - 1); }
     __syncthreads();
     if (!s_last) return;
     if (threadIdx.x < ICP_NSUM) {                              // fold the per-block partials in block order (deterministic whoever is last)
         const volatile double* vp = partial;
-        double s = 0; for (int b = 0; b < (int)gridDim.x; ++b) s += vp[b * ICP_NSUM + threadIdx.x];
-        out[threadIdx.x] = s; s_out[threadIdx.x] = s;
+        double s = 0; for (int b = 0; b < nblk; ++b) s += vp[b * ICP_NSUM + threadIdx.x];
+        if (out) out[threadIdx.x] = s;
+        s_out[threadIdx.x] = s;
     }
     __syncthreads();
     if (threadIdx.x == 0) {
@@ -126,16 +131,22 @@ __global__ void __launch_bounds__(ICP_BLOCK) k_icp_iteration(float4* __restrict_
     }
 }
 
-// getFitnessScore (pcl::Registration::getFitnessScore, max_range = DBL_MAX): mean squared nearest-neighbour distance of the
-// ORIGINAL source transformed by the final transformation.  out[0] = sum d2, out[1] = count.
-__global__ void __launch_bounds__(ICP_BLOCK) k_icp_fitness(const float4* __restrict__ src, int n_src, IcpT T_final, const unsigned* __restrict__ cell_start,
-                                                          const float4* __restrict__ gmap, GridDims g, int r_max, double* __restrict__ partial,
-                                                          int* __restrict__ counter, double* __restrict__ out) {
+__global__ void __launch_bounds__(ICP_BLOCK) k_icp_iteration(float4* __restrict__ src_cur, int n_src, IcpState* __restrict__ st, const unsigned* __restrict__ cell_start,
+                                                            const float4* __restrict__ gmap, GridDims g, int r_max, float max_d2, double* __restrict__ partial,
+                                                            int* __restrict__ counter, double* __restrict__ out, int* __restrict__ nn_idx, float* __restrict__ nn_d2) {
+    icp_iteration_body(src_cur, n_src, st, cell_start, gmap, g, r_max, max_d2, partial, counter, out, nn_idx, nn_d2, (int)blockIdx.x, (int)gridDim.x);
+}
+
+// getFitnessScore (pcl::Registration::getFitnessScore, max_range = DBL_MAX) for ONE pair, block `blk` of its `nblk`: mean squared
+// nearest-neighbour distance of the ORIGINAL source transformed by the final transformation T (row-major 3x4).  out[0] = sum d2, out[1] = count.
+__device__ __forceinline__ void icp_fitness_body(const float4* __restrict__ src, int n_src, const float* T, const unsigned* __restrict__ cell_start,
+                                                 const float4* __restrict__ gmap, GridDims g, int r_max, double* __restrict__ partial,
+                                                 int* __restrict__ counter, double* __restrict__ out, int blk, int nblk) {
     __shared__ double s_red[ICP_BLOCK / 32][2];
     __shared__ bool s_last;
     double sum = 0.0, cnt = 0.0;
-    for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < n_src; i += gridDim.x * blockDim.x) {
-        const float4 p = apply_affine_dev(T_final.t, src[i]);
+    for (int i = blk * ICP_BLOCK + threadIdx.x; i < n_src; i += nblk * ICP_BLOCK) {
+        const float4 p = apply_affine_dev(T, src[i]);
         float bd; int bi; float4 bp;
         if (icp_nearest(p, cell_start, gmap, g, r_max, bd, bi, bp)) { sum += (double)bd; cnt += 1.0; }
     }
@@ -145,19 +156,25 @@ __global__ void __launch_bounds__(ICP_BLOCK) k_icp_fitness(const float4* __restr
     __syncthreads();
     if (threadIdx.x < 2) {
         double s = 0; for (int w = 0; w < ICP_BLOCK / 32; ++w) s += s_red[w][threadIdx.x];
-        partial[blockIdx.x * 2 + threadIdx.x] = s;
+        partial[blk * 2 + threadIdx.x] = s;
         __threadfence();
     }
     __syncthreads();
-    if (threadIdx.x == 0) { const int t = atomicAdd(counter, 1); s_last = (t == (int)gridDim.x - 1); }
+    if (threadIdx.x == 0) { const int t = atomicAdd(counter, 1); s_last = (t == nblk - 1); }
     __syncthreads();
     if (!s_last) return;
     if (threadIdx.x < 2) {
         const volatile double* vp = partial;
-        double s = 0; for (int b = 0; b < (int)gridDim.x; ++b) s += vp[b * 2 + threadIdx.x];
+        double s = 0; for (int b = 0; b < nblk; ++b) s += vp[b * 2 + threadIdx.x];
         out[threadIdx.x] = s;
     }
     if (threadIdx.x == 0) *counter = 0;
+}
+
+__global__ void __launch_bounds__(ICP_BLOCK) k_icp_fitness(const float4* __restrict__ src, int n_src, IcpT T_final, const unsigned* __restrict__ cell_start,
+                                                          const float4* __restrict__ gmap, GridDims g, int r_max, double* __restrict__ partial,
+                                                          int* __restrict__ counter, double* __restrict__ out) {
+    icp_fitness_body(src, n_src, T_final.t, cell_start, gmap, g, r_max, partial, counter, out, (int)blockIdx.x, (int)gridDim.x);
 }
 
 }  // namespace liorf

@@ -744,4 +744,109 @@ inline int voxel_grid_device(const float4* in, Count cnt, float leaf, float4* ou
     return LIORF_OK;
 }
 
+// ---------------------------------------------------------------------------------------------------------------
+// Segmented VoxelGrid: S independent clouds ("segments", contiguous in one array) filtered in one pass, each exactly as
+// voxel_grid_device filters it alone — PCL's per-cloud min_b / div_b, the int32 overflow guard per segment (a segment that trips it
+// passes through unchanged), centroids summed sequentially in input order within each (segment, voxel).
+//   k_vgseg_bounds : per-segment min/max over host-planned tiles that never straddle two segments (order-independent atomics)
+//   k_vgseg_meta   : one thread per segment derives its VoxMeta and key range (div_b product, or the point count under the guard);
+//                    seg_base = exclusive prefix of the ranges, flags a total beyond 2^32
+//   k_vgseg_keys   : key = seg_base[segment] + PCL voxel index, so one 32-bit stable sort orders by (segment, voxel)
+//   then the multi-kernel path's radix sort, head scan and k_vg_centroid unchanged, and
+//   k_vgseg_out    : each segment's first voxel and voxel count (binary search of seg_base in the sorted voxel keys)
+// ---------------------------------------------------------------------------------------------------------------
+constexpr int VGSEG_TILE = 4096;
+struct VgSegTile { int seg, begin, end, pad; };
+
+__device__ __forceinline__ unsigned vgseg_ord(float f) {           // order-preserving float → unsigned (min/max by integer atomics)
+    const unsigned u = __float_as_uint(f);
+    return (u & 0x80000000u) ? ~u : (u | 0x80000000u);
+}
+__device__ __forceinline__ float vgseg_unord(unsigned u) { return __uint_as_float((u & 0x80000000u) ? (u & 0x7fffffffu) : ~u); }
+
+// mn[3 s + a] = encoded min (initialised to 0xffffffff), mx[3 s + a] = encoded max (initialised to 0)
+__global__ void __launch_bounds__(256) k_vgseg_bounds(const float4* __restrict__ pts, const VgSegTile* __restrict__ tiles, unsigned* __restrict__ mn_enc,
+                                                      unsigned* __restrict__ mx_enc) {
+    const VgSegTile t = tiles[blockIdx.x];
+    float mn[3] = {INFINITY, INFINITY, INFINITY}, mx[3] = {-INFINITY, -INFINITY, -INFINITY};
+    for (int i = t.begin + (int)threadIdx.x; i < t.end; i += blockDim.x) {
+        const float4 p = pts[i];
+        mn[0] = fminf(mn[0], p.x); mx[0] = fmaxf(mx[0], p.x);
+        mn[1] = fminf(mn[1], p.y); mx[1] = fmaxf(mx[1], p.y);
+        mn[2] = fminf(mn[2], p.z); mx[2] = fmaxf(mx[2], p.z);
+    }
+    __shared__ float s_red[8][6];
+#pragma unroll
+    for (int a = 0; a < 3; ++a)
+#pragma unroll
+        for (int o = 16; o > 0; o >>= 1) { mn[a] = fminf(mn[a], __shfl_xor_sync(FULL, mn[a], o)); mx[a] = fmaxf(mx[a], __shfl_xor_sync(FULL, mx[a], o)); }
+    if (lane_id() == 0) { for (int a = 0; a < 3; ++a) { s_red[warp_id()][a] = mn[a]; s_red[warp_id()][3 + a] = mx[a]; } }
+    __syncthreads();
+    if (threadIdx.x < 6) {
+        float v = s_red[0][threadIdx.x];
+        for (int w = 1; w < (int)blockDim.x / 32; ++w) v = threadIdx.x < 3 ? fminf(v, s_red[w][threadIdx.x]) : fmaxf(v, s_red[w][threadIdx.x]);
+        if (threadIdx.x < 3) atomicMin(mn_enc + t.seg * 3 + threadIdx.x, vgseg_ord(v)); else atomicMax(mx_enc + t.seg * 3 + threadIdx.x - 3, vgseg_ord(v));
+    }
+}
+
+// one block; S <= any size (threads stride), then thread 0 forms the prefix of the ranges
+__global__ void __launch_bounds__(1024) k_vgseg_meta(const int* __restrict__ seg_n, int S, const unsigned* __restrict__ mn_enc, const unsigned* __restrict__ mx_enc, float leaf, VoxMeta* __restrict__ metas,
+                                                     unsigned long long* __restrict__ seg_base, int* __restrict__ range_overflow) {
+    for (int s = threadIdx.x; s < S; s += blockDim.x) {
+        const int n = seg_n[s];
+        float mn[3], mx[3];
+        for (int a = 0; a < 3; ++a) { mn[a] = n > 0 ? vgseg_unord(mn_enc[s * 3 + a]) : 0.f; mx[a] = n > 0 ? vgseg_unord(mx_enc[s * 3 + a]) : 0.f; }
+        VoxMeta m;                                                    // k_vg_minmax's arithmetic
+        m.n = n;
+        m.inv = 1.0f / leaf;
+        long long d[3];
+        for (int a = 0; a < 3; ++a) {
+            m.minp[a] = mn[a]; m.maxp[a] = mx[a];
+            d[a] = (long long)((mx[a] - mn[a]) * m.inv) + 1;
+            m.min_b[a] = (int)floorf(mn[a] * m.inv);
+            const int max_b = (int)floorf(mx[a] * m.inv);
+            m.div_b[a] = max_b - m.min_b[a] + 1;
+        }
+        m.overflow = (n > 0 && d[0] * d[1] * d[2] > 2147483647LL) ? 1 : 0;
+        m.mul1 = m.div_b[0]; m.mul2 = m.div_b[0] * m.div_b[1];
+        metas[s] = m;
+        seg_base[s] = n <= 0 ? 0ull : m.overflow ? (unsigned long long)n : (unsigned long long)((long long)m.div_b[0] * m.div_b[1] * m.div_b[2]);
+    }
+    __syncthreads();
+    if (threadIdx.x == 0) {
+        unsigned long long run = 0;
+        for (int s = 0; s < S; ++s) { const unsigned long long r = seg_base[s]; seg_base[s] = run; run += r; }
+        seg_base[S] = run;
+        *range_overflow = run > (1ull << 32) ? 1 : 0;
+    }
+}
+
+__global__ void __launch_bounds__(256) k_vgseg_keys(const float4* __restrict__ pts, const VgSegTile* __restrict__ tiles, const int* __restrict__ seg_first,
+                                                    const VoxMeta* __restrict__ metas, const unsigned long long* __restrict__ seg_base, unsigned* __restrict__ keys) {
+    const VgSegTile t = tiles[blockIdx.x];
+    const VoxMeta& m = metas[t.seg];
+    const unsigned base = (unsigned)seg_base[t.seg];
+    const int first = seg_first[t.seg];
+    const float inv = m.inv;
+    for (int i = t.begin + (int)threadIdx.x; i < t.end; i += blockDim.x) {
+        if (m.overflow) { keys[i] = base + (unsigned)(i - first); continue; }      // every point its own voxel ⇒ output == input
+        keys[i] = base + vgf_key(pts[i], inv, m.min_b[0], m.min_b[1], m.min_b[2], m.mul1, m.mul2);
+    }
+}
+
+// seg_vox[2 s] = first voxel of segment s in the output, seg_vox[2 s + 1] = its voxel count
+__global__ void __launch_bounds__(256) k_vgseg_out(const unsigned* __restrict__ sorted_keys, const unsigned* __restrict__ seg_start, const unsigned* __restrict__ n_out,
+                                                   const unsigned long long* __restrict__ seg_base, int S, int* __restrict__ seg_vox) {
+    const int s = blockIdx.x * blockDim.x + threadIdx.x;
+    if (s >= S) return;
+    const int nv = (int)*n_out;
+    auto lower = [&](unsigned long long key) {                    // first voxel whose key >= key
+        int lo = 0, hi = nv;
+        while (lo < hi) { const int mid = (lo + hi) >> 1; if ((unsigned long long)sorted_keys[seg_start[mid]] < key) lo = mid + 1; else hi = mid; }
+        return lo;
+    };
+    const int b = lower(seg_base[s]), e = lower(seg_base[s + 1]);
+    seg_vox[2 * s] = b; seg_vox[2 * s + 1] = e - b;
+}
+
 }  // namespace liorf
