@@ -185,6 +185,18 @@ int liorf_sc_get(liorf_ctx* ctx, int i, double desc[1200], float ringkey[20], do
 /* replaces SCManager::detectLoopClosureID() (include/Scancontext.h:73) with the reference's semantics incl. the stale
  * tree (rebuilt every 10th call over keys[0 : n-30]).  cand3 / min_dist nullable diagnostics. */
 int liorf_sc_detect_loop_closure_id(liorf_ctx* ctx, int* loop_id, float* yaw_diff_rad, double* min_dist, int* cand3);
+/* detectLoopClosureID for Q calls at once.  Answer q is exactly what liorf_sc_detect_loop_closure_id returns when the database
+ * held its first n_db[q] entries (query = row n_db[q] - 1) and the stale tree covered keys [0, n_tree[q]) — every output
+ * bit-identical, whatever Q, the order of the queries or the search path.  Read-only: the context's own detector state (call
+ * counter, tree snapshot), its database and every other search are untouched; works on a borrowed database.
+ *   n_db[q] < 31        : loop_id -1, yaw 0, min_dist / cand3 entries untouched (the single call's early-out); never reaches the device
+ *   n_tree[q] < 3       : unfilled kNN slots are candidate 0, as in the single call; cand3 holds the substituted ids
+ *   LIORF_ERR_ARG, outputs untouched, nothing enqueued: a NULL mandatory array with Q > 0, n_db[q] outside [1, liorf_sc_size],
+ *                   or n_db[q] >= 31 with n_tree[q] outside [1, n_db[q] - 30].  Q = 0 is LIORF_OK.
+ * One upload of the indices, one download of the answers and one synchronisation, whatever Q.  The ring-key search takes the path
+ * liorf_sc_set_search_path selects for a batch of this size.  Python's liorf_b200.sc_tree_schedule gives the n_tree a call history saw. */
+int liorf_sc_detect_loop_closure_id_batch(liorf_ctx* ctx, const int* n_db, const int* n_tree, int Q,
+                                          int* loop_id, float* yaw_diff_rad, double* min_dist /*nullable*/, int* cand3 /*nullable, [Q][3]*/);
 /* batched search (BASELINE config 5): Q queries against the context's database rows [0, n_db) which represent GLOBAL
  * rows [global_offset, global_offset + n_db) (single GPU: offset 0).  The steps of one batch on DEVICE buffers (d_* are device pointers):
  *   prepare: ring keys (a11) of Q query descriptors → d_qkeys [Q][20] f32 (d_qsk / d_qcn, nullable: sector keys / column norms [Q][60] f64)

@@ -11,4 +11,4 @@ import os as _os
 _os.environ.setdefault("CUDA_DEVICE_MAX_CONNECTIONS", "32")
 
 from ._lib import load_library, library_path, build_library  # noqa: F401,E402
-from .api import imuDeskewInfo, Context, Params, LMTrace, FrameIn, FrameOut, CloudInfoGuess, GuessState, P4, PRAW  # noqa: F401
+from .api import imuDeskewInfo, sc_tree_schedule, Context, Params, LMTrace, FrameIn, FrameOut, CloudInfoGuess, GuessState, P4, PRAW  # noqa: F401

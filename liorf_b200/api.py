@@ -89,6 +89,23 @@ def imuDeskewInfo(stamp, gyro_xyz, time_scan_cur, time_scan_end, check_gate=True
                 rpy_index=rpy.value)
 
 
+def sc_tree_schedule(n_db_calls):
+    """The stale-tree size each detectLoopClosureID call of a call history saw, starting from a fresh SCManager: n_db_calls[i] is the
+    database size at call i.  A call with fewer than 31 entries returns early and does not advance the call counter (0 here); a call whose
+    counter is a multiple of 10 rebuilds the tree over keys [0, n - 30) (include/Scancontext.cpp:263-281).  Feeds detectLoopClosureIDBatch."""
+    n_db_calls = np.asarray(n_db_calls, np.int64).reshape(-1)
+    out = np.zeros(len(n_db_calls), np.int32)
+    counter, tree = 0, 0
+    for i, n in enumerate(n_db_calls):
+        if n < 31:
+            continue
+        if counter % 10 == 0:
+            tree = int(n) - 30
+        counter += 1
+        out[i] = tree
+    return out
+
+
 class LiorfError(RuntimeError):
     pass
 
@@ -446,6 +463,21 @@ class Context:
         lid = C.c_int(-1); yaw = C.c_float(0); md = C.c_double(0); cand = np.zeros(3, np.int32)
         _chk(self.lib.liorf_sc_detect_loop_closure_id(self.h, C.byref(lid), C.byref(yaw), C.byref(md), _vp(cand)), "liorf_sc_detect_loop_closure_id")
         return lid.value, yaw.value, md.value, cand
+
+    def detectLoopClosureIDBatch(self, n_db, n_tree):
+        """detectLoopClosureID for many calls at once (liorf_sc_detect_loop_closure_id_batch): entry q is the tuple detectLoopClosureID()
+        returns when the database held its first n_db[q] entries and the stale tree covered keys [0, n_tree[q]) (sc_tree_schedule gives the
+        n_tree of a call history).  Read-only: the detector state of this context is left as it was.
+        Returns (loop_id int32[Q], yaw float32[Q], min_dist float64[Q], cand3 int32[Q, 3]); min_dist / cand3 are 0 for early-out queries."""
+        n_db = np.ascontiguousarray(n_db, np.int32).reshape(-1)
+        n_tree = np.ascontiguousarray(n_tree, np.int32).reshape(-1)
+        if n_db.shape != n_tree.shape:
+            raise ValueError("n_db and n_tree must have the same length")
+        Q = len(n_db)
+        lid = np.full(Q, -1, np.int32); yaw = np.zeros(Q, np.float32); md = np.zeros(Q, np.float64); cand = np.zeros((Q, 3), np.int32)
+        _chk(self.lib.liorf_sc_detect_loop_closure_id_batch(self.h, _vp(n_db), _vp(n_tree), C.c_int(Q), _vp(lid), _vp(yaw), _vp(md), _vp(cand)),
+             "liorf_sc_detect_loop_closure_id_batch")
+        return lid, yaw, md, cand
 
     def loopClosureICP(self, loop_key_cur, loop_key_pre, history_search_num=25, loop_index=0, icp_leaf=0.5, max_corr_dist=20.0, max_iters=100):
         """the ICP of performSCLoopClosure (src/mapOptmization.cpp:624-730) between two stored keyframes"""

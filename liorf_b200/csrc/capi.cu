@@ -100,6 +100,8 @@ struct liorf_ctx {
     DevBuf<float> sc_part_d; DevBuf<int> sc_part_i;
     DevBuf<float> sc_q_d; DevBuf<int> sc_q_i; DevBuf<double> sc_pair_d; DevBuf<int> sc_pair_s;
     DevBuf<double> sc_qdesc; DevBuf<float> sc_qkeys; DevBuf<int> sc_res_i; DevBuf<double> sc_res_d;
+    // batched detectLoopClosureID: answers + query indices in one device block (one download, one upload) and its pinned host mirror
+    DevBuf<int> scdb_io; int* h_scdb = nullptr; size_t h_scdb_cap = 0;
     // tensor-core ring-key search (sc_tensor.cuh): operand images + work buffers.  A KeySet = a ring-key array the filter searches + the B
     // operand image built from it: ks_local = this context's own rows (sc_keys), ks_all = the replicated index of a sharded database
     struct KeySet { const float* keys = nullptr; int n = 0; unsigned gen = 0; DevBuf<uint8_t> bimg; float* center = nullptr; unsigned* nmax = nullptr;
@@ -457,6 +459,7 @@ void liorf_destroy(liorf_ctx* c) {
     c->sc_part_d.release(); c->sc_part_i.release();
     c->sc_q_d.release(); c->sc_q_i.release(); c->sc_pair_d.release(); c->sc_pair_s.release();
     c->sc_qdesc.release(); c->sc_qkeys.release(); c->sc_res_i.release(); c->sc_res_d.release();
+    c->scdb_io.release(); if (c->h_scdb) cudaFreeHost(c->h_scdb);
     c->sct_aimg.release(); c->sct_cmin.release(); c->sct_cmin32.release(); c->sct_qnorm.release(); c->sct_part.release(); c->sct_cand.release(); c->sct_cnt.release();
     for (liorf_ctx::KeySet* k : {&c->ks_local, &c->ks_all}) { k->bimg.release(); if (k->center) cudaFree(k->center); if (k->nmax) cudaFree(k->nmax); }
     c->icp_raw.release(); c->icp_src.release(); c->icp_src0.release(); c->icp_tgt.release(); c->icp_partial.release(); c->icp_sel.release(); c->icp_nn_idx.release();
@@ -1216,7 +1219,9 @@ int liorf_sc_get(liorf_ctx* c, int i, double desc[1200], float ringkey[20], doub
 }
 
 // local exact top-3 of Q queries over keys[0:n_keys) → d_dist/d_idx [Q][3]; unfilled slots: dist +inf, idx INT_MAX
-static int sc_knn_brute(liorf_ctx* c, const float* d_keys, int n_keys, const float* d_qkeys, int Q, int global_offset, float* d_dist, int* d_idx) {
+// lim (nullable, device [Q]): query q sees only keys [0, lim[q]) (every lim[q] <= n_keys)
+static int sc_knn_brute(liorf_ctx* c, const float* d_keys, int n_keys, const float* d_qkeys, int Q, int global_offset, float* d_dist, int* d_idx,
+                        const int* lim = nullptr) {
     int rc;
     if (Q <= 0) return LIORF_OK;
     const int bx = (Q + SCK_BLOCK - 1) / SCK_BLOCK;
@@ -1226,7 +1231,8 @@ static int sc_knn_brute(liorf_ctx* c, const float* d_keys, int n_keys, const flo
     chunks = (n_keys + kpc - 1) / kpc; if (chunks < 1) chunks = 1;
     if ((rc = c->sc_part_d.reserve((size_t)chunks * Q * 3)) || (rc = c->sc_part_i.reserve((size_t)chunks * Q * 3))) return rc;
     ProfScope ps(c, SEC_SC_SEARCH); c->launches += 2;
-    k_sc_knn_tile<<<dim3(bx, chunks), SCK_BLOCK, 0, c->stream>>>(d_keys, n_keys, global_offset, d_qkeys, Q, kpc, c->sc_part_d.p, c->sc_part_i.p);
+    if (lim) k_sc_knn_tile<true><<<dim3(bx, chunks), SCK_BLOCK, 0, c->stream>>>(d_keys, n_keys, global_offset, d_qkeys, Q, kpc, c->sc_part_d.p, c->sc_part_i.p, lim);
+    else k_sc_knn_tile<false><<<dim3(bx, chunks), SCK_BLOCK, 0, c->stream>>>(d_keys, n_keys, global_offset, d_qkeys, Q, kpc, c->sc_part_d.p, c->sc_part_i.p, nullptr);
     k_sc_merge_top3<<<(Q + 127) / 128, 128, 0, c->stream>>>(c->sc_part_d.p, c->sc_part_i.p, chunks, (size_t)Q * 3, Q, d_dist, d_idx);
     CUDA_TRY(cudaGetLastError());
     return LIORF_OK;
@@ -1245,6 +1251,7 @@ static int sct_prepare(liorf_ctx* c, liorf_ctx::KeySet& ks, int n_keys, const fl
     if (!c->sct_attr_set) {
         CUDA_TRY(cudaFuncSetAttribute(k_sc_tensor<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, SCT_SMEM));
         CUDA_TRY(cudaFuncSetAttribute(k_sc_tensor<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, SCT_SMEM));
+        CUDA_TRY(cudaFuncSetAttribute(k_sc_tensor<false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, SCT_SMEM));
         c->sct_attr_set = true;
     }
     if (ks.img_n != n_keys || ks.img_gen != ks.gen || ks.img_keys != ks.keys) {
@@ -1262,26 +1269,34 @@ static int sct_prepare(liorf_ctx* c, liorf_ctx::KeySet& ks, int n_keys, const fl
         (rc = c->sct_cand.reserve((size_t)Q * SCT_CAP)) || (rc = c->sct_cnt.reserve(Q))) return rc;
     k_sct_image<false><<<(int)((rows + 127) / 128), 128, 0, c->stream>>>(d_qkeys, Q, (int)rows, nkt, ks.center, c->sct_aimg.p, c->sct_qnorm.p, nullptr);
     a.a_img = c->sct_aimg.p; a.b_img = ks.bimg.p; a.Q = Q; a.n_keys = n_keys; a.nkt = nkt; a.n_sqt = n_sqt;
-    a.cmin = c->sct_cmin.p; a.cmin32 = c->sct_cmin32.p; a.dump = nullptr; a.err_flag = c->d_err;
+    a.cmin = c->sct_cmin.p; a.cmin32 = c->sct_cmin32.p; a.dump = nullptr; a.err_flag = c->d_err; a.lim = nullptr;
     c->launches += 1;
     return LIORF_OK;
 }
 
 // exact top-3 of Q queries over the first n_keys keys of a key set on the tensor cores.  push != nullptr: sharded search, the result goes
-// into every rank's window (phase C) from the re-rank kernel itself
-static int sc_knn_tensor(liorf_ctx* c, liorf_ctx::KeySet& ks, int n_keys, const float* d_qkeys, int Q, int idx_offset, float* d_dist, int* d_idx, const ShardPush* push = nullptr) {
+// into every rank's window (phase C) from the re-rank kernel itself.  lim (nullable, device [Q]): query q sees only keys [0, lim[q]); the
+// filter still runs over the operand image of all n_keys keys, so the cached image is reused whatever the limits
+static int sc_knn_tensor(liorf_ctx* c, liorf_ctx::KeySet& ks, int n_keys, const float* d_qkeys, int Q, int idx_offset, float* d_dist, int* d_idx, const ShardPush* push = nullptr,
+                         const int* lim = nullptr) {
     int rc, grid;
     SctArgs a;
     ProfScope ps(c, SEC_SC_SEARCH);
     const int nkt = (n_keys + SCT_KT - 1) / SCT_KT, rows = ((Q + SCT_QT - 1) / SCT_QT) * SCT_QT;
     if ((rc = sct_prepare(c, ks, n_keys, d_qkeys, Q, a, grid))) return rc;
-    { ProfScope pg(c, SEC_SC_GEMM); k_sc_tensor<false><<<grid, SCT_THREADS, SCT_SMEM, c->stream>>>(a); }
+    a.lim = lim;
+    {
+        ProfScope pg(c, SEC_SC_GEMM);
+        if (lim) k_sc_tensor<false, true><<<grid, SCT_THREADS, SCT_SMEM, c->stream>>>(a);
+        else k_sc_tensor<false><<<grid, SCT_THREADS, SCT_SMEM, c->stream>>>(a);
+    }
     k_sct_top3<<<dim3(rows / 32, SCS_SPLITS), 32 * SCS_SLICES, 0, c->stream>>>(c->sct_cmin.p, nkt, rows, c->sct_part.p, Q, c->sct_cnt.p, c->sct_over_cnt);
     k_sct_select<<<dim3(rows / 32, SCS_SPLITS), 32 * SCS_SLICES, 0, c->stream>>>(c->sct_cmin.p, c->sct_cmin32.p, nkt, rows, c->sct_part.p, c->sct_qnorm.p, Q, ks.nmax,
                                                                                  c->sct_cand.p, c->sct_cnt.p);
     ShardPush P; std::memset(&P, 0, sizeof(P));
     if (push) P = *push;
-    k_sct_rerank<<<(Q + 7) / 8, 256, 0, c->stream>>>(ks.keys, n_keys, nkt, idx_offset, d_qkeys, Q, c->sct_cand.p, c->sct_cnt.p, d_dist, d_idx, c->sct_over_cnt, P);
+    if (lim) k_sct_rerank<true><<<(Q + 7) / 8, 256, 0, c->stream>>>(ks.keys, n_keys, nkt, idx_offset, d_qkeys, Q, c->sct_cand.p, c->sct_cnt.p, d_dist, d_idx, c->sct_over_cnt, P, lim);
+    else k_sct_rerank<false><<<(Q + 7) / 8, 256, 0, c->stream>>>(ks.keys, n_keys, nkt, idx_offset, d_qkeys, Q, c->sct_cand.p, c->sct_cnt.p, d_dist, d_idx, c->sct_over_cnt, P, nullptr);
     CUDA_TRY(cudaGetLastError());
     c->launches += 4; c->sct_last_Q = Q;
     return LIORF_OK;
@@ -1774,6 +1789,9 @@ int liorf_sc_shard_query_async(liorf_ctx* c, const double* qdescs, int Q, int gl
     return LIORF_OK;
 }
 
+// yawDiffRad of detectLoopClosureID from the decided column shift: deg2rad(float) of the shift in degrees (:17-20, :339)
+static float sc_yaw_rad(int nn_align) { return (float)((float)(nn_align * (360.0 / 60.0)) * M_PI / 180.0); }
+
 int liorf_sc_detect_loop_closure_id(liorf_ctx* c, int* loop_id, float* yaw_diff_rad, double* min_dist, int* cand3) {
     LIORF_NVTX;
     if (!c || !loop_id || !yaw_diff_rad) return LIORF_ERR_ARG;
@@ -1803,7 +1821,72 @@ int liorf_sc_detect_loop_closure_id(liorf_ctx* c, int* loop_id, float* yaw_diff_
     double md; std::memcpy(&md, c->h_mail + 720, sizeof(double));
     if (min_dist) *min_dist = md;
     if (cand3) { cand3[0] = cand[0]; cand3[1] = cand[1]; cand3[2] = cand[2]; }
-    *yaw_diff_rad = (float)((float)(nn_align * (360.0 / 60.0)) * M_PI / 180.0);   // deg2rad(float) (:17-20, :339)
+    *yaw_diff_rad = sc_yaw_rad(nn_align);
+    return LIORF_OK;
+}
+
+/* detectLoopClosureID for Q calls at once (header): query q is row n_db[q] - 1, searched over keys [0, n_tree[q]).  Queries past the
+ * early-out are gathered into contiguous query buffers; stage 1 runs with per-query key limits, stage 2 and the decision are the batch
+ * search's kernels.  Device layout of scdb_io (ints, Qd gathered queries): dist f64[Qd] | loop_id[Qd] | shift[Qd] | cand[3 Qd] | n_db[Qd] |
+ * n_tree[Qd] — the first 7 Qd ints come back in one copy, the last 2 Qd go up in one. */
+int liorf_sc_detect_loop_closure_id_batch(liorf_ctx* c, const int* n_db, const int* n_tree, int Q, int* loop_id, float* yaw_diff_rad, double* min_dist, int* cand3) {
+    LIORF_NVTX;
+    if (!c || Q < 0 || (Q > 0 && (!n_db || !n_tree || !loop_id || !yaw_diff_rad))) return LIORF_ERR_ARG;
+    int Qd = 0, max_tree = 0, min_tree = 0x7fffffff;
+    for (int q = 0; q < Q; ++q) {
+        if (n_db[q] < 1 || n_db[q] > c->sc_n) return LIORF_ERR_ARG;
+        if (n_db[q] < SC_EXCLUDE_RECENT + 1) continue;                          // :263-267
+        if (n_tree[q] < 1 || n_tree[q] > n_db[q] - SC_EXCLUDE_RECENT) return LIORF_ERR_ARG;
+        ++Qd; max_tree = std::max(max_tree, n_tree[q]); min_tree = std::min(min_tree, n_tree[q]);
+    }
+    if (Q == 0) return LIORF_OK;
+    CUDA_TRY(cudaSetDevice(c->P.device));
+    int rc;
+    if (Qd > 0) {
+        const size_t io_ints = (size_t)9 * Qd;
+        if (io_ints > c->h_scdb_cap) {
+            if (c->h_scdb) { CUDA_TRY(cudaStreamSynchronize(c->stream)); CUDA_TRY(cudaFreeHost(c->h_scdb)); c->h_scdb = nullptr; c->h_scdb_cap = 0; }
+            const size_t cap = std::max<size_t>(io_ints, 1 << 16);
+            CUDA_TRY(cudaHostAlloc(&c->h_scdb, cap * sizeof(int), cudaHostAllocDefault));
+            c->h_scdb_cap = cap;
+        }
+        if ((rc = c->scdb_io.reserve(io_ints)) || (rc = c->sc_qdesc.reserve((size_t)Qd * SC_DESC)) || (rc = c->sc_qkeys.reserve((size_t)Qd * SC_RING)) ||
+            (rc = sc_reserve_query(c, Qd))) return rc;
+        int* H = c->h_scdb;
+        for (int q = 0, k = 0; q < Q; ++q)
+            if (n_db[q] >= SC_EXCLUDE_RECENT + 1) { H[7 * Qd + k] = n_db[q]; H[8 * Qd + k] = n_tree[q]; ++k; }
+        int* D = c->scdb_io.p;
+        double* d_dist = reinterpret_cast<double*>(D);
+        int *d_loop = D + 2 * Qd, *d_shift = D + 3 * Qd, *d_cand = D + 4 * Qd, *d_rows = D + 7 * Qd, *d_lim = D + 8 * Qd;
+        CUDA_TRY(cudaMemcpyAsync(d_rows, H + 7 * Qd, (size_t)2 * Qd * sizeof(int), cudaMemcpyHostToDevice, c->stream));
+        k_sc_gather_queries<<<Qd, 128, 0, c->stream>>>(c->sc_desc.p, c->sc_keys.p, d_rows, Qd, c->sc_qdesc.p, c->sc_qkeys.p);
+        CUDA_TRY(cudaGetLastError());
+        c->launches += 1;
+        // stage 1 on the path the batch search would take for Qd queries against this database; the CUDA-core kernel needs to look no
+        // further than the largest limit, the tensor-core filter keeps the database's operand image
+        if (sc_want_tensor(c, Qd, c->sc_n)) rc = sc_knn_tensor(c, local_keys(c), c->sc_n, c->sc_qkeys.p, Qd, 0, c->sc_q_d.p, d_cand, nullptr, d_lim);
+        else rc = sc_knn_brute(c, c->sc_keys.p, max_tree, c->sc_qkeys.p, Qd, 0, c->sc_q_d.p, d_cand, d_lim);
+        if (rc) return rc;
+        if (min_tree < SC_NUM_CAND) {
+            k_sc_cand_unfilled_to_zero<<<(3 * Qd + 127) / 128, 128, 0, c->stream>>>(d_cand, 3 * Qd);
+            CUDA_TRY(cudaGetLastError());
+            c->launches += 1;
+        }
+        if ((rc = sc_distance_launch(c, c->sc_qdesc.p, d_cand, 3 * Qd, 0, c->sc_pair_d.p, c->sc_pair_s.p))) return rc;
+        if ((rc = liorf_sc_decide_dev(c, c->sc_pair_d.p, c->sc_pair_s.p, d_cand, Qd, d_loop, d_shift, d_dist))) return rc;
+        CUDA_TRY(cudaMemcpyAsync(H, D, (size_t)7 * Qd * sizeof(int), cudaMemcpyDeviceToHost, c->stream));
+        if ((rc = check_err(c))) return rc;
+    }
+    const int* H = c->h_scdb;
+    for (int q = 0, k = 0; q < Q; ++q) {
+        loop_id[q] = -1; yaw_diff_rad[q] = 0.f;
+        if (n_db[q] < SC_EXCLUDE_RECENT + 1) continue;
+        loop_id[q] = H[2 * Qd + k];
+        yaw_diff_rad[q] = sc_yaw_rad(H[3 * Qd + k]);
+        if (min_dist) std::memcpy(min_dist + q, H + 2 * (size_t)k, sizeof(double));
+        if (cand3) for (int j = 0; j < 3; ++j) cand3[3 * (size_t)q + j] = H[4 * Qd + 3 * k + j];
+        ++k;
+    }
     return LIORF_OK;
 }
 

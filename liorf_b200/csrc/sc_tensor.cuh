@@ -249,11 +249,16 @@ struct SctArgs {
     float* cmin32;             // out: [nkt * 4][n_sqt * SCT_QT]  minimum d~ of each 32-key chunk (read only for tiles that pass)
     float* dump;               // DUMP (tests): every d~, [n_sqt * SCT_QT][nkt * SCT_KT] indexed by database key
     int* err_flag;
+    const int* lim;            // LIM: [Q] query q sees only keys [0, lim[q])
 };
 
 __device__ __forceinline__ long long sct_first_step(int cta, long long total, int grid) { return (long long)cta * total / grid; }
 
-template <bool DUMP>
+// LIM (batched detectLoopClosureID, a.lim): query q sees only keys [0, lim[q]).  Key tiles interleave the keys (column i of tile kt is key
+// i * nkt + kt), so that prefix is a column prefix in every tile: q keeps the first ceil((lim[q] - kt) / nkt) columns of tile kt.  The epilogue
+// sets the other columns to +inf before its min trees — never to 3.0e38f, which the selection's `<= thr` could pass — so the masked minima
+// feed k_sct_top3 / k_sct_select unchanged: three chunks with finite masked minima still hold three distinct keys of the prefix.
+template <bool DUMP, bool LIM = false>
 __global__ void __launch_bounds__(SCT_THREADS, 1) k_sc_tensor(SctArgs a) {
     extern __shared__ uint8_t sct_smem_raw[];
     uint8_t* smem = reinterpret_cast<uint8_t*>(((uintptr_t)sct_smem_raw + 1023) & ~(uintptr_t)1023);
@@ -338,9 +343,11 @@ __global__ void __launch_bounds__(SCT_THREADS, 1) k_sc_tensor(SctArgs a) {
         const uint32_t t_lane = tmem_base + ((uint32_t)(32 * qd) << 16) + j * SCT_SUB;
         const size_t n_rows = (size_t)a.n_sqt * SCT_QT;
         int sqt = sqt0, kt = kt0;
+        int lim_a = 0, lim_b = 0;                                  // LIM: this row's limit = lim_a * nkt + lim_b → tile kt keeps lim_a + (kt < lim_b) columns
         for (int it = 0; it < n_steps; ++it) {
             const int q = sqt * SCT_QT + j * SCT_SUB + row;
             const int acc = it & 1;
+            if (LIM && (it == 0 || kt == 0)) { const int L = q < a.Q ? __ldg(a.lim + q) : 0; lim_a = L / a.nkt; lim_b = L % a.nkt; }
             if (!mbar_wait(BAR(T_FULL + acc), (it >> 1) & 1, s_abort, a.err_flag)) break;
             tc_fence_after();
             const uint32_t tcol = t_lane + acc * 256;
@@ -351,6 +358,19 @@ __global__ void __launch_bounds__(SCT_THREADS, 1) k_sc_tensor(SctArgs a) {
             tc_fence_before();
             __syncwarp();
             if (lane == 0) mbar_arrive(BAR(T_EMPTY + acc));        // the values are in registers: release the accumulator stage early
+            if constexpr (LIM) {
+                const int ncol = lim_a + (kt < lim_b ? 1 : 0);
+                if (ncol < SCT_KT) {
+                    const uint32_t INF = 0x7f800000u;
+#pragma unroll
+                    for (int i = 0; i < 32; ++i) {
+                        if (i >= ncol) v0[i] = INF;
+                        if (32 + i >= ncol) v1[i] = INF;
+                        if (64 + i >= ncol) v2[i] = INF;
+                        if (96 + i >= ncol) v3[i] = INF;
+                    }
+                }
+            }
             if (DUMP) {
                 float* o = a.dump + (size_t)q * ((size_t)a.nkt * SCT_KT);
 #pragma unroll
@@ -465,12 +485,15 @@ __global__ void __launch_bounds__(32 * SCS_SLICES) k_sct_select(const float* __r
 // Sharded search (sc_shard.cuh, P.enabled): the queries are this rank's slice [P.q0, P.q0 + Q) of the batch and the result — the
 // GLOBAL top-3, the keys being the replicated index — goes straight into the candidate array of every rank's window (phase C);
 // the last block raises the flags: compute and transfer in ONE kernel.
+// LIM (batched detectLoopClosureID): query q sees only keys [0, lim[q]): candidate keys past it are skipped, the overflow scan stops there.
+template <bool LIM>
 __global__ void __launch_bounds__(256) k_sct_rerank(const float* __restrict__ keys, int n_keys, int nkt, int idx_offset, const float* __restrict__ qkeys, int Q,
                                                    const int* __restrict__ cand, const int* __restrict__ cand_cnt, float* __restrict__ out_d, int* __restrict__ out_i,
-                                                   int* __restrict__ over_cnt, ShardPush P) {
+                                                   int* __restrict__ over_cnt, ShardPush P, const int* __restrict__ lim) {
     const int q = blockIdx.x * (blockDim.x / 32) + warp_id();
     const int l = lane_id();
     if (q < Q) {
+        if (LIM) n_keys = lim[q];
         const int n = cand_cnt[q];
         float aq[20];
 #pragma unroll

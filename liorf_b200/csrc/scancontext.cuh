@@ -99,8 +99,11 @@ __device__ __forceinline__ void top3_insert(Top3& t, float d, int i) {
 constexpr int SCK_BLOCK = 128;          // queries per block (one query per thread)
 constexpr int SCK_TILE = 256;           // keys staged in shared memory per step
 // grid = (ceil(Q / SCK_BLOCK), n_chunks).  Each (query, chunk) emits a local top-3 → part[(chunk * Q + q) * 3 + j].
+// LIM (batched detectLoopClosureID): query q counts key k only if k < lim[q] (k before idx_offset), the stale tree's key prefix.  The
+// shared-memory staging stays block-uniform up to the largest limit of the block, so a chunk past every limit of its block stops at once.
+template <bool LIM>
 __global__ void __launch_bounds__(SCK_BLOCK) k_sc_knn_tile(const float* __restrict__ keys, int n_keys, int idx_offset, const float* __restrict__ qkeys, int Q,
-                                                          int keys_per_chunk, float* __restrict__ part_d, int* __restrict__ part_i) {
+                                                          int keys_per_chunk, float* __restrict__ part_d, int* __restrict__ part_i, const int* __restrict__ lim) {
     __shared__ float4 s_keys[SCK_TILE * 5];
     const int q = blockIdx.x * SCK_BLOCK + threadIdx.x;
     float a[20];
@@ -108,7 +111,17 @@ __global__ void __launch_bounds__(SCK_BLOCK) k_sc_knn_tile(const float* __restri
     for (int k = 0; k < 20; ++k) a[k] = q < Q ? __ldg(qkeys + 20 * (size_t)q + k) : 0.f;
     Top3 t; top3_init(t);
     const int k_begin = blockIdx.y * keys_per_chunk;
-    const int k_end = min(n_keys, k_begin + keys_per_chunk);
+    int k_end = min(n_keys, k_begin + keys_per_chunk);
+    int my_lim = n_keys;
+    if constexpr (LIM) {
+        __shared__ int s_lmax;
+        my_lim = q < Q ? __ldg(lim + q) : 0;
+        if (threadIdx.x == 0) s_lmax = 0;
+        __syncthreads();
+        atomicMax(&s_lmax, my_lim);
+        __syncthreads();
+        k_end = min(k_end, s_lmax);
+    }
     for (int base = k_begin; base < k_end; base += SCK_TILE) {
         const int cnt = min(SCK_TILE, k_end - base);
         __syncthreads();
@@ -117,7 +130,7 @@ __global__ void __launch_bounds__(SCK_BLOCK) k_sc_knn_tile(const float* __restri
         __syncthreads();
         for (int k = 0; k < cnt; ++k) {
             float d = ringkey_dist_dev(a, s_keys + 5 * k);
-            top3_insert(t, d, idx_offset + base + k);
+            if (!LIM || base + k < my_lim) top3_insert(t, d, idx_offset + base + k);
         }
     }
     if (q < Q) {
@@ -255,6 +268,23 @@ __global__ void __launch_bounds__(128) k_sc_decide(const double* __restrict__ pa
 #pragma unroll
     for (int c = 0; c < SC_NUM_CAND; ++c) { double d = pair_dist[3 * (size_t)q + c]; if (d < mn) { mn = d; al = pair_shift[3 * (size_t)q + c]; nn = cand[3 * (size_t)q + c]; } }
     loop_id[q] = mn < SC_DIST_THRES ? nn : -1; shift[q] = al; dist[q] = mn;
+}
+
+// batched detectLoopClosureID: the stored descriptor and stored ring key of database row rows1[q] - 1 (the newest row when the database
+// held rows1[q] entries) → contiguous query q.  One block per query.
+__global__ void __launch_bounds__(128) k_sc_gather_queries(const double* __restrict__ db_desc, const float* __restrict__ db_keys, const int* __restrict__ rows1, int Q,
+                                                          double* __restrict__ qdesc, float* __restrict__ qkeys) {
+    const int q = blockIdx.x; if (q >= Q) return;
+    const size_t r = (size_t)(rows1[q] - 1);
+    const double2* src = reinterpret_cast<const double2*>(db_desc + r * SC_DESC);
+    double2* dst = reinterpret_cast<double2*>(qdesc + (size_t)q * SC_DESC);
+    for (int i = threadIdx.x; i < SC_DESC / 2; i += blockDim.x) dst[i] = __ldg(src + i);
+    if (threadIdx.x < SC_RING) qkeys[(size_t)q * SC_RING + threadIdx.x] = __ldg(db_keys + r * SC_RING + threadIdx.x);
+}
+// an unfilled kNN slot (a tree of fewer than 3 keys) is candidate 0: the reference's result vectors are zero-initialised (:289-290)
+__global__ void __launch_bounds__(128) k_sc_cand_unfilled_to_zero(int* __restrict__ cand, int n) {
+    const int i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i < n && cand[i] == 0x7fffffff) cand[i] = 0;
 }
 
 // keys (fp32 ring key, sector key, column norms) for externally supplied descriptors — batch version of k_sc_finalize
