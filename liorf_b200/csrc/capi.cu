@@ -47,22 +47,26 @@ constexpr int PROF_RING = 64;
 constexpr int S2M_SPARE_SMS = 16;      // SMs the persistent solver leaves to the concurrent front end of the next frame
 struct Profiler {
     bool enabled = false; unsigned mask = 0xffu;        // mask: sections that record events (bit = section id)
-    cudaEvent_t ev[PROF_RING][2]; int sec[PROF_RING]; int pending = 0; bool created = false;
+    Event ev[PROF_RING][2]; int sec[PROF_RING]; int pending = 0; bool created = false;
     double ms[SEC_COUNT] = {0}; long long calls[SEC_COUNT] = {0};
 };
 
+// The ScanContext database: one context owns it, others may borrow it (liorf_sc_borrow_database)
+struct ScDatabase { DevBuf<double> desc, sk, cn; DevBuf<float> keys; };
+
+// Every member that holds a CUDA resource owns it (common.cuh); raw pointers are views into memory another member owns.
 struct liorf_ctx {
     liorf_params P;
-    cudaStream_t stream = nullptr;
+    Stream stream;
     int num_sms = kNumSMs;
     // device scalars
-    int* d_counts = nullptr;        // C_COUNT ints of the CURRENT front set (N_SCAN, N_DS, FIRST_KEPT, hook counts)
-    int* d_counts_base = nullptr;   // [front set 0 | shared | front set 1], C_COUNT ints each: either set is contiguous with the shared block
-    int* d_shared = nullptr;        // counts that do not belong to a front set (C_M_DS)
-    int* d_misc = nullptr;          // counters / error flag (zero-initialised)
-    unsigned long long* d_tick = nullptr;   // look-back ticket words (prims.cuh: draw_ticket), one per scan / sort work area
-    int* d_err = nullptr;
-    int* h_mail = nullptr;          // pinned mailbox (128 KB: scalars/trace in the lower half, IMU table staging in the upper)
+    int* d_counts = nullptr;        // view: C_COUNT ints of the CURRENT front set (N_SCAN, N_DS, FIRST_KEPT, hook counts)
+    DevMem<int> d_counts_base;      // [front set 0 | shared | front set 1], C_COUNT ints each: either set is contiguous with the shared block
+    int* d_shared = nullptr;        // view: counts that do not belong to a front set (C_M_DS)
+    DevMem<int> d_misc;             // counters / error flag (zero-initialised)
+    DevMem<unsigned long long> d_tick;   // look-back ticket words (prims.cuh: draw_ticket), one per scan / sort work area
+    int* d_err = nullptr;           // view: d_misc[0]
+    HostBuf<int> h_mail;            // pinned mailbox (128 KB: scalars/trace in the lower half, IMU table staging in the upper)
     // clouds
     DevBuf<float4> scan, scan_ds, map_raw, map_ds, kf_points;
     DevBuf<int> membership, out_keys;
@@ -72,44 +76,45 @@ struct liorf_ctx {
     int m_bound = 0;
     VoxelGridWork vg;               // scan-side VoxelGrid work area (main stream)
     VoxelGridWork vg_map;           // map-side work area: the local-map chain runs concurrently on stream_map
-    cudaStream_t stream_map = nullptr;
-    cudaEvent_t ev_main = nullptr, ev_map = nullptr; bool map_pending = false;
+    Stream stream_map;
+    Event ev_main, ev_map; bool map_pending = false;
     MapGrid grid;
     DeskewWork dk;
     std::vector<Keyframe> kfs;
     size_t kf_used = 0;
     DevBuf<KfSel> d_sel;
-    KfSel* h_sel = nullptr; int h_sel_cap = 0;       // two halves, alternated per call (see stage_slot)
-    cudaEvent_t stage_ev[2][2] = {{nullptr, nullptr}, {nullptr, nullptr}}; int stage_turn[2] = {0, 0};   // [0] = selection table, [1] = IMU table
+    HostBuf<KfSel> h_sel;                            // two halves, alternated per call (see stage_slot)
+    Event stage_ev[2][2]; int stage_turn[2] = {0, 0};   // [0] = selection table, [1] = IMU table
     // the local-map chain as CUDA graphs (one pair per 64k-point size bucket): ~20 stream operations become 2 launches
-    struct MapGraphs { cudaGraphExec_t vg = nullptr, grid = nullptr; const void* sig[20] = {nullptr}; };
+    struct MapGraphs { GraphExec vg, grid; const void* sig[20] = {nullptr}; };
     std::map<int, MapGraphs> map_graphs; bool use_graphs = true;
     std::vector<int> last_sel; unsigned long long pose_version = 0, last_sel_version = ~0ull; bool map_valid = false;
     // LM
-    float* d_tf6 = nullptr; LMDeviceState* d_lm = nullptr; S2MTrace* d_trace = nullptr; double* d_partial = nullptr; ulonglong2* d_wpart = nullptr; unsigned long long* d_res = nullptr; long long* d_dbg = nullptr; unsigned long long* d_dbg_gt = nullptr;
-    IcpState* icp_state = nullptr; DevBuf<QueryCache> qcache; DevBuf<float4> cand; unsigned s2m_launch_seq = 0; S2MMail* d_mail = nullptr; bool mail_fresh = false; bool s2m_global_state = false;
+    DevMem<float> d_tf6; DevMem<LMDeviceState> d_lm; DevMem<S2MTrace> d_trace; DevMem<double> d_partial; DevMem<ulonglong2> d_wpart; DevMem<unsigned long long> d_res; DevMem<long long> d_dbg; DevMem<unsigned long long> d_dbg_gt;
+    DevMem<IcpState> icp_state; DevBuf<QueryCache> qcache; DevBuf<float4> cand; unsigned s2m_launch_seq = 0; DevMem<S2MMail> d_mail; bool mail_fresh = false; bool s2m_global_state = false;
     int s2m_grid = 0; bool s2m_no_cache = false; int map_vg_grid = 0;
     int s2m_ctas = 0;                // tests: solver CTAs of every launch (0 = num_sms per function call, s2m_grid in liorf_process_frame)
     DevBuf<float4> h_coeff, h_sel_pts, h_ori_c, h_coeff_c; DevBuf<unsigned char> h_flag; DevBuf<int> h_idx; DevBuf<float> h_d2, h_plane;
     DevBuf<double> lm_partial; ScanWork combine_scan; int hook_n = 0;
-    float* d_lm_out = nullptr;      // AtA[36] AtB[6] X[6]
+    DevMem<float> d_lm_out;         // AtA[36] AtB[6] X[6]
     // ScanContext
-    DevBuf<double> sc_desc, sc_sk, sc_cn; DevBuf<float> sc_keys; int sc_n = 0; bool sc_borrowed = false;   // borrowed: the database buffers belong to another context
-    unsigned* d_bins = nullptr;
+    ScDatabase sc_own; ScDatabase* sc_db = &sc_own; int sc_n = 0;   // sc_db: sc_own, or the owner's database when borrowed
+    bool sc_borrowed() const { return sc_db != &sc_own; }
+    DevMem<unsigned> d_bins;
     int sc_tree_n = 0, sc_counter = 0;
     DevBuf<float> sc_part_d; DevBuf<int> sc_part_i;
     DevBuf<float> sc_q_d; DevBuf<int> sc_q_i; DevBuf<double> sc_pair_d; DevBuf<int> sc_pair_s;
     DevBuf<double> sc_qdesc; DevBuf<float> sc_qkeys; DevBuf<int> sc_res_i; DevBuf<double> sc_res_d;
     // batched detectLoopClosureID: answers + query indices in one device block (one download, one upload) and its pinned host mirror
-    DevBuf<int> scdb_io; int* h_scdb = nullptr; size_t h_scdb_cap = 0;
+    DevBuf<int> scdb_io; HostBuf<int> h_scdb;
     // tensor-core ring-key search (sc_tensor.cuh): operand images + work buffers.  A KeySet = a ring-key array the filter searches + the B
-    // operand image built from it: ks_local = this context's own rows (sc_keys), ks_all = the replicated index of a sharded database
-    struct KeySet { const float* keys = nullptr; int n = 0; unsigned gen = 0; DevBuf<uint8_t> bimg; float* center = nullptr; unsigned* nmax = nullptr;
+    // operand image built from it: ks_local = this context's own rows (sc_db->keys), ks_all = the replicated index of a sharded database
+    struct KeySet { const float* keys = nullptr; int n = 0; unsigned gen = 0; DevBuf<uint8_t> bimg; DevMem<float> center; DevMem<unsigned> nmax;   // keys: view
                     int img_n = -1; unsigned img_gen = 0; const float* img_keys = nullptr; } ks_local, ks_all;
     DevBuf<uint8_t> sct_aimg; DevBuf<float> sct_cmin, sct_cmin32, sct_qnorm, sct_part; DevBuf<int> sct_cand, sct_cnt;
-    int* sct_over_cnt = nullptr;
+    DevMem<int> sct_over_cnt;
     // loop-closure ICP (icp.cuh)
-    DevBuf<float4> icp_raw, icp_src, icp_src0, icp_tgt; MapGrid icp_grid; DevBuf<double> icp_partial; double* icp_out = nullptr; int* icp_counter = nullptr;
+    DevBuf<float4> icp_raw, icp_src, icp_src0, icp_tgt; MapGrid icp_grid; DevBuf<double> icp_partial; DevMem<double> icp_out; int* icp_counter = nullptr;   // icp_counter: view
     DevBuf<KfSel> icp_sel; DevBuf<int> icp_nn_idx; DevBuf<float> icp_nn_d2;
     // batched loop-closure ICP (icp_batch.cuh): work buffers of its own, sized by the largest wave so far
     struct IcpBatch {
@@ -117,46 +122,54 @@ struct liorf_ctx {
         DevBuf<VoxMeta> metas; DevBuf<unsigned long long> seg_base; DevBuf<float4> raw, vox, src_cur, sorted;
         DevBuf<IcpPairDesc> pd; DevBuf<int2> act; DevBuf<IcpState> st; DevBuf<double> partial, fit;
         SortWork sort; ScanWork scan, grid_scan;
-        int* d_flags = nullptr;                 // [0] voxel total of the wave, [1] key range beyond 32 bits
-        unsigned char* h_stage = nullptr; size_t h_cap = 0;      // pinned: tables going up, counts / states / sums coming back
+        DevMem<int> d_flags;                    // [0] voxel total of the wave, [1] key range beyond 32 bits
+        HostBuf<unsigned char> h_stage;         // pinned: tables going up, counts / states / sums coming back
         int max_pairs = 0;                      // tests: pairs per wave (0 = memory-bounded)
     } icpb;
     liorf_guess_state guess_state = {}; float tf_mapped[6] = {0, 0, 0, 0, 0, 0};   // updateInitialGuess statics + transformTobeMapped
     // sharded search over peer windows (sc_shard.cuh)
-    struct ScShard { bool ready = false; ShardWin W; int qmax = 0, kcap = 0; size_t win_bytes = 0, off_keys = 0; unsigned* d_batch = nullptr; unsigned* d_counter = nullptr;
-                     unsigned keys_gen = 0; bool keys_pushed = false;
-                     cudaGraphExec_t graph = nullptr; const void* gsig[40] = {nullptr}; const void* last_sig[40] = {nullptr}; bool ipc_opened[SCSH_MAX] = {false};
-                     DevBuf<int> list; int* d_nlist = nullptr; } shard;
+    // W.base[] and W.keys_all[] are views: of win, of a peer's window mapped into ipc[], or of a window of another context in this process
+    struct ScShard { bool ready = false; ShardWin W; int qmax = 0, kcap = 0; size_t win_bytes = 0, off_keys = 0; unsigned* d_batch = nullptr; DevMem<unsigned> d_counter;
+                     DevMem<unsigned char> win; IpcMapping<unsigned char> ipc[SCSH_MAX]; unsigned keys_gen = 0; bool keys_pushed = false;
+                     GraphExec graph; const void* gsig[40] = {nullptr}; const void* last_sig[40] = {nullptr};
+                     DevBuf<int> list; int* d_nlist = nullptr; } shard;   // d_batch, d_nlist, W.wait_ns: views of d_counter
     int sc_path = 0;                 // 0 auto, 1 CUDA-core brute force, 2 tensor-core filter + exact re-rank
     bool sct_attr_set = false; int sct_last_Q = 0; bool scdb_attr_set = false; int scdb_blocks_per_sm[2] = {1, 1};   // [kQ16]
     Profiler prof;
     double host_us[12] = {0}; long long host_frames = 0; bool host_timing = false;   // LIORF_HOST_TIMING=1 ([6..10]: pieces of the keyframe tail)
-    cudaEvent_t tl_ev[8] = {nullptr}; double tl_ms[8] = {0}; // debug GPU timeline stamps of process_frame
+    Event tl_ev[8]; double tl_ms[8] = {0}; // debug GPU timeline stamps of process_frame
     long long launches = 0;         // kernels launched by this context (bench.py's gpu_launches)
     // ---- pipelined front end (cloudHandler of frame i+1 overlaps laserCloudInfoHandler of frame i) ----
     // Everything projectPointCloud + downsampleCurrentScan read or write for ONE frame lives in a "front set"; the context
     // holds two and swaps them, so the next frame's set is filled on stream_pre while the solver works on the current one.
     struct FrontSet {
         DevBuf<float4> scan, scan_ds; DeskewWork dk; VoxelGridWork vg;
-        int* d_counts = nullptr; int n_scan_bound = 0, h_n_scan = -1, h_n_ds = -1;
+        int* d_counts = nullptr; int n_scan_bound = 0, h_n_scan = -1, h_n_ds = -1;   // d_counts: view
     } alt;
-    cudaStream_t stream_pre = nullptr;
-    cudaEvent_t ev_pre_done = nullptr, ev_frame_start = nullptr;
+    Stream stream_pre;
+    Event ev_pre_done, ev_frame_start;
     bool pre_valid = false, frame_start_recorded = false; int pre_index = 0, pre_n = 0; const void* pre_pts = nullptr;
+    ~liorf_ctx() {          // no stream may still use what the members release as they are destroyed
+        if (!stream) return;                 // nothing was created on the device
+        cudaSetDevice(P.device);
+        cudaStreamSynchronize(stream);
+        if (stream_pre) cudaStreamSynchronize(stream_pre);
+        if (stream_map) cudaStreamSynchronize(stream_map);
+    }
 };
 
 // The two secondary streams are created on first use: a context that only searches the ScanContext database (one lane of a sharded search)
 // never needs them, and every stream a process creates competes for the device's hardware channels (CUDA_DEVICE_MAX_CONNECTIONS) — streams
 // that share a channel serialise, which turned cross-GPU flag waits of different lanes into a cycle (DESIGN.md §7).
-static int make_low_priority_stream(cudaStream_t* out) {
+static int make_low_priority_stream(Stream& out) {
     int prio_lo = 0, prio_hi = 0;
     CUDA_TRY(cudaDeviceGetStreamPriorityRange(&prio_lo, &prio_hi));
     if (std::getenv("LIORF_NO_PRIO")) prio_lo = 0;
-    CUDA_TRY(cudaStreamCreateWithPriority(out, cudaStreamNonBlocking, prio_lo));
+    CUDA_TRY(stream_create(out, prio_lo));
     return LIORF_OK;
 }
-static int need_stream_map(liorf_ctx* c) { return c->stream_map ? LIORF_OK : make_low_priority_stream(&c->stream_map); }
-static int need_stream_pre(liorf_ctx* c) { return c->stream_pre ? LIORF_OK : make_low_priority_stream(&c->stream_pre); }
+static int need_stream_map(liorf_ctx* c) { return c->stream_map ? LIORF_OK : make_low_priority_stream(c->stream_map); }
+static int need_stream_pre(liorf_ctx* c) { return c->stream_pre ? LIORF_OK : make_low_priority_stream(c->stream_pre); }
 
 // swaps the current front set with the alternate one (pointer swaps only)
 static void front_swap(liorf_ctx* c) {
@@ -167,11 +180,11 @@ static void front_swap(liorf_ctx* c) {
 // D2H of the current set's counts together with the shared block: ONE 2 x C_COUNT copy into h_mail[0 : 2 C_COUNT)
 static cudaError_t mail_counts(liorf_ctx* c) {
     const int* src = c->d_counts < c->d_shared ? c->d_counts : c->d_shared;
-    return cudaMemcpyAsync(c->h_mail, src, 2 * C_COUNT * sizeof(int), cudaMemcpyDeviceToHost, c->stream);
+    return cudaMemcpyAsync(c->h_mail.p, src, 2 * C_COUNT * sizeof(int), cudaMemcpyDeviceToHost, c->stream);
 }
 static void take_counts(liorf_ctx* c) {
     const int so = c->d_counts < c->d_shared ? 0 : C_COUNT, sh = C_COUNT - so;
-    c->h_n_scan = c->h_mail[so + C_N_SCAN]; c->h_n_ds = c->h_mail[so + C_N_DS]; c->h_m_ds = c->h_mail[sh + C_M_DS];
+    c->h_n_scan = c->h_mail.p[so + C_N_SCAN]; c->h_n_ds = c->h_mail.p[so + C_N_DS]; c->h_m_ds = c->h_mail.p[sh + C_M_DS];
 }
 
 static void prof_flush(liorf_ctx* c) {           // call only when the stream is idle (after a sync)
@@ -193,7 +206,7 @@ struct ProfScope {
     ProfScope(liorf_ctx* c_, int sec, cudaStream_t st_ = nullptr) : c(c_), st(st_ ? st_ : c_->stream) {
         Profiler& p = c->prof;
         if (!p.enabled || !((p.mask >> sec) & 1u)) return;
-        if (!p.created) { for (int i = 0; i < PROF_RING; ++i) { cudaEventCreate(&p.ev[i][0]); cudaEventCreate(&p.ev[i][1]); } p.created = true; }
+        if (!p.created) { for (auto& e : p.ev) { (void)event_create(e[0], cudaEventDefault); (void)event_create(e[1], cudaEventDefault); } p.created = true; }
         if (p.pending == PROF_RING) { cudaStreamSynchronize(c->stream); if (c->stream_map) cudaStreamSynchronize(c->stream_map); prof_flush(c); }
         slot = p.pending++; p.sec[slot] = sec;
         cudaEventRecord(p.ev[slot][0], st);
@@ -218,7 +231,7 @@ static void host_get_transformation(float x, float y, float z, float roll, float
 // consumed, so re-use never needs a stream synchronise (the event is normally long complete).
 static int stage_slot(liorf_ctx* c, int which) {
     const int turn = c->stage_turn[which] ^= 1;
-    if (!c->stage_ev[which][turn]) { if (cudaEventCreateWithFlags(&c->stage_ev[which][turn], cudaEventDisableTiming) != cudaSuccess) return -1; }
+    if (!c->stage_ev[which][turn]) { if (event_create(c->stage_ev[which][turn], cudaEventDisableTiming) != cudaSuccess) return -1; }
     else if (cudaEventSynchronize(c->stage_ev[which][turn]) != cudaSuccess) return -1;
     return turn;
 }
@@ -238,10 +251,10 @@ static int upload_pose(liorf_ctx* c, const float* pose6) {          // by kernel
 static int check_err(liorf_ctx* c) {      // after a stream sync: sticky device-side error flag (bounded look-back spins)
     int e = 0;
     { int rcj = join_map(c); if (rcj) return rcj; }
-    CUDA_TRY(cudaMemcpyAsync(c->h_mail + 4000, c->d_err, sizeof(int), cudaMemcpyDeviceToHost, c->stream));
+    CUDA_TRY(cudaMemcpyAsync(c->h_mail.p + 4000, c->d_err, sizeof(int), cudaMemcpyDeviceToHost, c->stream));
     CUDA_TRY(cudaStreamSynchronize(c->stream));
     prof_flush(c);
-    e = c->h_mail[4000];
+    e = c->h_mail.p[4000];
     if (e) {
         fprintf(stderr, "[liorf_b200] device error flag %d (%s)\n", e, e == 5 ? "an mbarrier wait gave up" : e >= 0x30 ? "a peer's exchange flag never arrived: 0x30 + phase, C=0 D=1 KEYS=2" :
                 e == 2 ? "solver: a worker / the reducer never arrived" : "look-back predecessor never arrived");
@@ -261,9 +274,10 @@ static int read_counts(liorf_ctx* c) {
 
 static int sc_reserve(liorf_ctx* c, int n) {
     int rc;
-    if (c->sc_borrowed) return (size_t)n * SC_RING <= c->sc_keys.cap ? LIORF_OK : LIORF_ERR_STATE;      // a borrowed database is read-only here
-    if ((rc = c->sc_desc.reserve((size_t)n * SC_DESC, c->stream, true)) || (rc = c->sc_sk.reserve((size_t)n * SC_SECTOR, c->stream, true)) ||
-        (rc = c->sc_cn.reserve((size_t)n * SC_SECTOR, c->stream, true)) || (rc = c->sc_keys.reserve((size_t)n * SC_RING, c->stream, true))) return rc;
+    ScDatabase& db = *c->sc_db;
+    if (c->sc_borrowed()) return (size_t)n * SC_RING <= db.keys.cap ? LIORF_OK : LIORF_ERR_STATE;      // a borrowed database is read-only here
+    if ((rc = db.desc.reserve((size_t)n * SC_DESC, c->stream, true)) || (rc = db.sk.reserve((size_t)n * SC_SECTOR, c->stream, true)) ||
+        (rc = db.cn.reserve((size_t)n * SC_SECTOR, c->stream, true)) || (rc = db.keys.reserve((size_t)n * SC_RING, c->stream, true))) return rc;
     return LIORF_OK;
 }
 
@@ -292,7 +306,7 @@ int liorf_create(const liorf_params* p, liorf_ctx** out) {
         fprintf(stderr, "[liorf_b200] no CUDA device: this library has no CPU path\n");
         return LIORF_ERR_CUDA;
     }
-    liorf_ctx* c = new (std::nothrow) liorf_ctx();
+    std::unique_ptr<liorf_ctx> c(new (std::nothrow) liorf_ctx());      // every early return below frees what was created so far
     if (!c) return LIORF_ERR_ARG;
     c->P = *p;
     c->host_timing = std::getenv("LIORF_HOST_TIMING") != nullptr;
@@ -300,8 +314,8 @@ int liorf_create(const liorf_params* p, liorf_ctx** out) {
     if (c->P.grid_dim_x == 0) c->P.grid_dim_x = 256;
     if (c->P.grid_dim_y == 0) c->P.grid_dim_y = 256;
     if (c->P.grid_dim_z == 0) c->P.grid_dim_z = 32;
-    if (!is_pow2(c->P.grid_dim_x) || !is_pow2(c->P.grid_dim_y) || !is_pow2(c->P.grid_dim_z) || c->P.grid_dim_x < 4) { delete c; return LIORF_ERR_ARG; }
-    if (c->P.downsampleRate < 1 || c->P.point_filter_num < 1) { delete c; return LIORF_ERR_ARG; }
+    if (!is_pow2(c->P.grid_dim_x) || !is_pow2(c->P.grid_dim_y) || !is_pow2(c->P.grid_dim_z) || c->P.grid_dim_x < 4) return LIORF_ERR_ARG;
+    if (c->P.downsampleRate < 1 || c->P.point_filter_num < 1) return LIORF_ERR_ARG;
     c->grid.dims = GridDims{c->P.grid_dim_x, c->P.grid_dim_y, c->P.grid_dim_z};
     CUDA_TRY(cudaSetDevice(c->P.device));
     cudaDeviceProp prop; CUDA_TRY(cudaGetDeviceProperties(&prop, c->P.device));
@@ -310,7 +324,6 @@ int liorf_create(const liorf_params* p, liorf_ctx** out) {
     // time); a grid of num_sms CTAs has num_sms - 1 workers.  A B200 (148 SMs) is within the limit, so this refusal never runs there.
     if (c->num_sms - 1 > S2M_MAX_WORKERS) {
         fprintf(stderr, "[liorf_b200] %d SMs: the solver supports at most %d (raise S2M_MAX_WORKERS in scan2map.cuh)\n", c->num_sms, S2M_MAX_WORKERS + 1);
-        delete c;
         return LIORF_ERR_CUDA;
     }
     // the main stream carries the latency-critical chain (deskew → downsample → solver); giving it the highest priority lets
@@ -318,16 +331,16 @@ int liorf_create(const liorf_params* p, liorf_ctx** out) {
     int prio_lo = 0, prio_hi = 0;
     CUDA_TRY(cudaDeviceGetStreamPriorityRange(&prio_lo, &prio_hi));
     if (std::getenv("LIORF_NO_PRIO")) prio_lo = prio_hi = 0;
-    CUDA_TRY(cudaStreamCreateWithPriority(&c->stream, cudaStreamNonBlocking, prio_hi));
-    CUDA_TRY(cudaMalloc(&c->d_counts_base, 3 * C_COUNT * sizeof(int)));
+    CUDA_TRY(stream_create(c->stream, prio_hi));
+    CUDA_TRY(dev_alloc(c->d_counts_base, 3 * C_COUNT));
     CUDA_TRY(cudaMemset(c->d_counts_base, 0, 3 * C_COUNT * sizeof(int)));
     c->d_counts = c->d_counts_base; c->d_shared = c->d_counts_base + C_COUNT; c->alt.d_counts = c->d_counts_base + 2 * C_COUNT;
-    CUDA_TRY(cudaMalloc(&c->d_misc, 64 * sizeof(int)));
+    CUDA_TRY(dev_alloc(c->d_misc, 64));
     CUDA_TRY(cudaMemset(c->d_misc, 0, 64 * sizeof(int)));
     c->d_err = c->d_misc + 0;
     {
         unsigned long long init[16]; for (auto& v : init) v = TICKET_INIT;
-        CUDA_TRY(cudaMalloc(&c->d_tick, sizeof(init)));
+        CUDA_TRY(dev_alloc(c->d_tick, 16));
         CUDA_TRY(cudaMemcpy(c->d_tick, init, sizeof(init), cudaMemcpyHostToDevice));
     }
     c->vg.mm_counter = c->d_misc + 1;
@@ -336,14 +349,13 @@ int liorf_create(const liorf_params* p, liorf_ctx** out) {
     c->grid.scan.ticket = c->d_tick + 2; c->grid.scan.err_flag = c->d_err;
     c->dk.scan.ticket = c->d_tick + 3; c->dk.scan.err_flag = c->d_err;
     c->combine_scan.ticket = c->d_tick + 4; c->combine_scan.err_flag = c->d_err;
-    int* lm_counter = c->d_misc + 7; (void)lm_counter;
-    CUDA_TRY(cudaMalloc(&c->vg.meta, sizeof(VoxMeta)));
+    CUDA_TRY(dev_alloc(c->vg.meta, 1));
     for (VoxelGridWork* vw : {&c->vg, &c->vg_map, &c->alt.vg}) {          // grid-barrier words of the one-kernel VoxelGrid
-        CUDA_TRY(cudaMalloc(&vw->fused_bar, 2 * sizeof(unsigned))); CUDA_TRY(cudaMemset(vw->fused_bar, 0, 2 * sizeof(unsigned))); vw->err_flag = c->d_err;
+        CUDA_TRY(dev_alloc(vw->fused_bar, 2)); CUDA_TRY(cudaMemset(vw->fused_bar, 0, 2 * sizeof(unsigned))); vw->err_flag = c->d_err;
     }
-    CUDA_TRY(cudaEventCreateWithFlags(&c->ev_main, cudaEventDisableTiming));
-    CUDA_TRY(cudaEventCreateWithFlags(&c->ev_map, cudaEventDisableTiming));
-    CUDA_TRY(cudaMalloc(&c->vg_map.meta, sizeof(VoxMeta)));
+    CUDA_TRY(event_create(c->ev_main, cudaEventDisableTiming));
+    CUDA_TRY(event_create(c->ev_map, cudaEventDisableTiming));
+    CUDA_TRY(dev_alloc(c->vg_map.meta, 1));
     c->vg_map.mm_counter = c->d_misc + 10;
     c->vg_map.sort.ticket = c->d_tick + 5; c->vg_map.sort.err_flag = c->d_err;
     c->vg_map.scan.ticket = c->d_tick + 6; c->vg_map.scan.err_flag = c->d_err;
@@ -351,27 +363,27 @@ int liorf_create(const liorf_params* p, liorf_ctx** out) {
     c->icpb.sort.ticket = c->d_tick + 11; c->icpb.sort.err_flag = c->d_err;
     c->icpb.scan.ticket = c->d_tick + 12; c->icpb.scan.err_flag = c->d_err;
     c->icpb.grid_scan.ticket = c->d_tick + 13; c->icpb.grid_scan.err_flag = c->d_err;
-    CUDA_TRY(cudaMalloc(&c->icpb.d_flags, 2 * sizeof(int)));
-    CUDA_TRY(cudaMalloc(&c->dk.start_inv, 12 * sizeof(float)));
+    CUDA_TRY(dev_alloc(c->icpb.d_flags, 2));
+    CUDA_TRY(dev_alloc(c->dk.start_inv, 12));
     c->dk.first_kept = c->d_counts + C_FIRST_KEPT;
     // the alternate front set: its own look-back tickets, VoxelGrid meta and deskew scalars
     c->alt.vg.mm_counter = c->d_misc + 20;
     c->alt.vg.sort.ticket = c->d_tick + 8; c->alt.vg.sort.err_flag = c->d_err;
     c->alt.vg.scan.ticket = c->d_tick + 9; c->alt.vg.scan.err_flag = c->d_err;
     c->alt.dk.scan.ticket = c->d_tick + 10; c->alt.dk.scan.err_flag = c->d_err;
-    CUDA_TRY(cudaMalloc(&c->alt.vg.meta, sizeof(VoxMeta)));
-    CUDA_TRY(cudaMalloc(&c->alt.dk.start_inv, 12 * sizeof(float)));
+    CUDA_TRY(dev_alloc(c->alt.vg.meta, 1));
+    CUDA_TRY(dev_alloc(c->alt.dk.start_inv, 12));
     c->alt.dk.first_kept = c->alt.d_counts + C_FIRST_KEPT;
-    CUDA_TRY(cudaEventCreateWithFlags(&c->ev_pre_done, cudaEventDisableTiming));
-    CUDA_TRY(cudaEventCreateWithFlags(&c->ev_frame_start, cudaEventDisableTiming));
-    CUDA_TRY(cudaHostAlloc(&c->h_mail, 65536 + 2 * 65536, cudaHostAllocDefault));
-    CUDA_TRY(cudaMalloc(&c->d_tf6, 6 * sizeof(float)));
+    CUDA_TRY(event_create(c->ev_pre_done, cudaEventDisableTiming));
+    CUDA_TRY(event_create(c->ev_frame_start, cudaEventDisableTiming));
+    { int rc = c->h_mail.reserve((65536 + 2 * 65536) / sizeof(int)); if (rc) return rc; }
+    CUDA_TRY(dev_alloc(c->d_tf6, 6));
     CUDA_TRY(cudaMemset(c->d_tf6, 0, 6 * sizeof(float)));
-    CUDA_TRY(cudaMalloc(&c->d_lm, sizeof(LMDeviceState)));
+    CUDA_TRY(dev_alloc(c->d_lm, 1));
     CUDA_TRY(cudaMemset(c->d_lm, 0, sizeof(LMDeviceState)));
-    CUDA_TRY(cudaMalloc(&c->d_trace, sizeof(S2MTrace)));
+    CUDA_TRY(dev_alloc(c->d_trace, 1));
     CUDA_TRY(cudaMemset(c->d_trace, 0, sizeof(S2MTrace)));
-    CUDA_TRY(cudaMalloc(&c->d_lm_out, 48 * sizeof(float)));
+    CUDA_TRY(dev_alloc(c->d_lm_out, 48));
     int occ = 0;
     CUDA_TRY(cudaFuncSetAttribute(k_scan2map_persistent, cudaFuncAttributeMaxDynamicSharedMemorySize, S2MP_SMEM));
     CUDA_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, k_scan2map_persistent, S2MP_BLOCK, S2MP_SMEM));
@@ -397,14 +409,14 @@ int liorf_create(const liorf_params* p, liorf_ctx** out) {
         if (const char* e = std::getenv("LIORF_MAP_VG_GRID")) c->map_vg_grid = std::atoi(e);
         if (c->map_vg_grid > c->num_sms) c->map_vg_grid = c->num_sms;
     }
-    CUDA_TRY(cudaMalloc(&c->d_partial, (size_t)2 * c->num_sms * NPROD * sizeof(double)));
-    CUDA_TRY(cudaMalloc(&c->d_mail, sizeof(S2MMail)));
+    CUDA_TRY(dev_alloc(c->d_partial, (size_t)2 * c->num_sms * NPROD));
+    CUDA_TRY(dev_alloc(c->d_mail, 1));
     // hand-off words of the solver (epoch-tagged: zero never matches an epoch, launch sequence numbers start at 1)
-    CUDA_TRY(cudaMalloc(&c->d_wpart, (size_t)c->num_sms * NPROD * sizeof(ulonglong2)));
+    CUDA_TRY(dev_alloc(c->d_wpart, (size_t)c->num_sms * NPROD));
     CUDA_TRY(cudaMemset(c->d_wpart, 0, (size_t)c->num_sms * NPROD * sizeof(ulonglong2)));
-    CUDA_TRY(cudaMalloc(&c->d_res, 8 * sizeof(unsigned long long)));
+    CUDA_TRY(dev_alloc(c->d_res, 8));
     CUDA_TRY(cudaMemset(c->d_res, 0, 8 * sizeof(unsigned long long)));
-    CUDA_TRY(cudaMalloc(&c->d_bins, SC_DESC * sizeof(unsigned)));
+    CUDA_TRY(dev_alloc(c->d_bins, SC_DESC));
     {   // arm the ScanContext bins with the NO_POINT code
         std::vector<unsigned> init(SC_DESC);
         float f = -1000.f; unsigned u; std::memcpy(&u, &f, 4); u = (u & 0x80000000u) ? ~u : (u | 0x80000000u);
@@ -412,7 +424,7 @@ int liorf_create(const liorf_params* p, liorf_ctx** out) {
         CUDA_TRY(cudaMemcpy(c->d_bins, init.data(), SC_DESC * sizeof(unsigned), cudaMemcpyHostToDevice));
     }
     CUDA_TRY(cudaStreamSynchronize(c->stream));
-    *out = c;
+    *out = c.release();
     return LIORF_OK;
 }
 
@@ -428,75 +440,6 @@ void liorf_destroy(liorf_ctx* c) {
                 1e3 * c->tl_ms[1] / c->host_frames, 1e3 * c->tl_ms[2] / c->host_frames, 1e3 * c->tl_ms[3] / c->host_frames, 1e3 * c->tl_ms[4] / c->host_frames,
                 1e3 * c->tl_ms[5] / c->host_frames);
     }
-    cudaSetDevice(c->P.device);
-    cudaStreamSynchronize(c->stream);
-    if (c->stream_pre) cudaStreamSynchronize(c->stream_pre);
-    {   // the alternate front set (the current one is released below)
-        liorf_ctx::FrontSet& a = c->alt;
-        a.scan.release(); a.scan_ds.release(); a.dk.raw.release(); a.dk.imu.release(); a.dk.kept.release(); a.dk.scan.status.release();
-        a.vg.partial.release(); a.vg.keys.release(); a.vg.seg_start.release(); a.vg.sort.keys_alt.release(); a.vg.sort.vals_a.release();
-        a.vg.sort.vals_b.release(); a.vg.sort.hist.release(); a.vg.sort.status.release(); a.vg.scan.status.release();
-        cudaFree(a.vg.meta); cudaFree(a.dk.start_inv);
-    }
-    if (c->stream_pre) cudaStreamDestroy(c->stream_pre);
-    if (c->ev_pre_done) cudaEventDestroy(c->ev_pre_done);
-    if (c->ev_frame_start) cudaEventDestroy(c->ev_frame_start);
-    DevBuf<float4>* f4[] = {&c->scan, &c->scan_ds, &c->map_raw, &c->map_ds, &c->kf_points, &c->h_coeff, &c->h_sel_pts, &c->h_ori_c, &c->h_coeff_c, &c->grid.sorted};
-    for (auto b : f4) b->release();
-    c->membership.release(); c->out_keys.release(); c->h_flag.release(); c->h_idx.release(); c->h_d2.release(); c->h_plane.release();
-    c->lm_partial.release(); c->d_sel.release();
-    if (c->stream_map) cudaStreamSynchronize(c->stream_map);
-    for (VoxelGridWork* w : {&c->vg_map}) { w->partial.release(); w->keys.release(); w->seg_start.release(); w->sort.keys_alt.release(); w->sort.vals_a.release();
-        w->sort.vals_b.release(); w->sort.hist.release(); w->sort.status.release(); w->scan.status.release(); cudaFree(w->meta); }
-    for (auto& kv : c->map_graphs) { if (kv.second.vg) cudaGraphExecDestroy(kv.second.vg); if (kv.second.grid) cudaGraphExecDestroy(kv.second.grid); }
-    cudaEventDestroy(c->ev_main); cudaEventDestroy(c->ev_map); if (c->stream_map) cudaStreamDestroy(c->stream_map);
-    c->vg.partial.release(); c->vg.keys.release(); c->vg.seg_start.release();
-    c->vg.sort.keys_alt.release(); c->vg.sort.vals_a.release(); c->vg.sort.vals_b.release(); c->vg.sort.hist.release(); c->vg.sort.status.release();
-    c->vg.scan.status.release(); c->grid.scan.status.release(); c->dk.scan.status.release(); c->combine_scan.status.release();
-    c->grid.counts.release(); c->grid.cell_start.release();
-    c->dk.raw.release(); c->dk.imu.release(); c->dk.kept.release();
-    if (!c->sc_borrowed) { c->sc_desc.release(); c->sc_sk.release(); c->sc_cn.release(); c->sc_keys.release(); }
-    c->sc_part_d.release(); c->sc_part_i.release();
-    c->sc_q_d.release(); c->sc_q_i.release(); c->sc_pair_d.release(); c->sc_pair_s.release();
-    c->sc_qdesc.release(); c->sc_qkeys.release(); c->sc_res_i.release(); c->sc_res_d.release();
-    c->scdb_io.release(); if (c->h_scdb) cudaFreeHost(c->h_scdb);
-    c->sct_aimg.release(); c->sct_cmin.release(); c->sct_cmin32.release(); c->sct_qnorm.release(); c->sct_part.release(); c->sct_cand.release(); c->sct_cnt.release();
-    for (liorf_ctx::KeySet* k : {&c->ks_local, &c->ks_all}) { k->bimg.release(); if (k->center) cudaFree(k->center); if (k->nmax) cudaFree(k->nmax); }
-    c->icp_raw.release(); c->icp_src.release(); c->icp_src0.release(); c->icp_tgt.release(); c->icp_partial.release(); c->icp_sel.release(); c->icp_nn_idx.release();
-    c->icp_nn_d2.release(); c->icp_grid.counts.release(); c->icp_grid.cell_start.release(); c->icp_grid.sorted.release(); c->icp_grid.scan.status.release();
-    if (c->icp_out) cudaFree(c->icp_out);
-    {
-        liorf_ctx::IcpBatch& B = c->icpb;
-        B.sel.release(); B.tiles.release(); B.seg_n.release(); B.seg_vox.release(); B.counters.release(); B.mm.release(); B.keys.release(); B.seg_start.release();
-        B.counts.release(); B.cell_start.release(); B.metas.release(); B.seg_base.release(); B.raw.release(); B.vox.release(); B.src_cur.release(); B.sorted.release();
-        B.pd.release(); B.act.release(); B.st.release(); B.partial.release(); B.fit.release();
-        B.sort.keys_alt.release(); B.sort.vals_a.release(); B.sort.vals_b.release(); B.sort.hist.release(); B.sort.status.release();
-        B.scan.status.release(); B.grid_scan.status.release();
-        if (B.d_flags) cudaFree(B.d_flags);
-        if (B.h_stage) cudaFreeHost(B.h_stage);
-    }
-    if (c->sct_over_cnt) cudaFree(c->sct_over_cnt);
-    for (VoxelGridWork* vw : {&c->vg, &c->vg_map, &c->alt.vg}) {
-        vw->pts_sorted.release(); vw->cta_hist.release(); vw->cta_heads.release();
-        if (vw->fused_bar) cudaFree(vw->fused_bar); vw->fused_bar = nullptr;
-        if (vw->dbg) cudaFree(vw->dbg); vw->dbg = nullptr;
-    }
-    cudaFree(c->d_counts_base); cudaFree(c->d_misc); cudaFree(c->d_tick); cudaFree(c->vg.meta); cudaFree(c->dk.start_inv); cudaFree(c->d_tf6); cudaFree(c->d_lm);
-    cudaFree(c->d_trace); cudaFree(c->d_lm_out); cudaFree(c->d_partial); cudaFree(c->d_bins); cudaFree(c->d_wpart); cudaFree(c->d_res); cudaFree(c->d_mail); if (c->icp_state) cudaFree(c->icp_state); c->qcache.release(); c->cand.release();
-    if (c->d_dbg) cudaFree(c->d_dbg);
-    {   // peer windows
-        liorf_ctx::ScShard& S = c->shard;
-        for (int g = 0; g < SCSH_MAX; ++g) if (S.ipc_opened[g]) cudaIpcCloseMemHandle(S.W.base[g]);
-        if (S.W.base[S.W.rank]) cudaFree(S.W.base[S.W.rank]);
-        if (S.d_counter) cudaFree(S.d_counter);
-        if (S.graph) cudaGraphExecDestroy(S.graph);
-        S.list.release();
-    }
-    if (c->d_dbg_gt) cudaFree(c->d_dbg_gt);
-    if (c->h_sel) cudaFreeHost(c->h_sel);
-    for (int a = 0; a < 2; ++a) for (int b = 0; b < 2; ++b) if (c->stage_ev[a][b]) cudaEventDestroy(c->stage_ev[a][b]);
-    cudaFreeHost(c->h_mail);
-    cudaStreamDestroy(c->stream);
     delete c;
 }
 
@@ -520,7 +463,7 @@ static int project_common(liorf_ctx* c, const RawPoint* d_raw, int n, double t0,
         if ((rc = c->dk.imu.reserve((size_t)4 * rows))) return rc;
         if ((size_t)4 * rows * sizeof(double) > 65536) return LIORF_ERR_ARG;        // queueLength = 2000 rows (src/imageProjection.cpp:62) = 64000 B
         const int slot = stage_slot(c, 1); if (slot < 0) return LIORF_ERR_CUDA;
-        double* stage = reinterpret_cast<double*>(c->h_mail + 16384 + slot * 16384);   // pinned staging (two 64 KB halves above the mailbox)
+        double* stage = reinterpret_cast<double*>(c->h_mail.p + 16384 + slot * 16384);   // pinned staging (two 64 KB halves above the mailbox)
         std::memcpy(stage, imu_time, rows * sizeof(double)); std::memcpy(stage + rows, rx, rows * sizeof(double));
         std::memcpy(stage + 2 * rows, ry, rows * sizeof(double)); std::memcpy(stage + 3 * rows, rz, rows * sizeof(double));
         CUDA_TRY(cudaMemcpyAsync(c->dk.imu.p, stage, (size_t)4 * rows * sizeof(double), cudaMemcpyHostToDevice, c->stream));
@@ -571,9 +514,9 @@ static int set_scan_common(liorf_ctx* c, const void* src, int n, cudaMemcpyKind 
     int rc;
     if ((rc = c->scan.reserve(n > 0 ? n : 1))) return rc;
     if (n > 0) CUDA_TRY(cudaMemcpyAsync(c->scan.p, src, (size_t)n * sizeof(float4), kind, c->stream));
-    c->h_mail[100] = n;
+    c->h_mail.p[100] = n;
     // count goes through a kernel-visible device int
-    CUDA_TRY(cudaMemcpyAsync(c->d_counts + C_N_SCAN, &c->h_mail[100], sizeof(int), cudaMemcpyHostToDevice, c->stream));
+    CUDA_TRY(cudaMemcpyAsync(c->d_counts + C_N_SCAN, &c->h_mail.p[100], sizeof(int), cudaMemcpyHostToDevice, c->stream));
     CUDA_TRY(cudaStreamSynchronize(c->stream));
     c->n_scan_bound = n; c->h_n_scan = n; c->h_n_ds = -1;
     return LIORF_OK;
@@ -614,8 +557,8 @@ int liorf_set_current_scan_strided(liorf_ctx* c, const void* data, int n, int po
     }
     if (n > 0) k_unpack_strided<<<(n + 255) / 256, 256, 0, c->stream>>>(d_raw, n, point_step, offset_xyz, offset_intensity, c->scan.p);
     CUDA_TRY(cudaGetLastError());
-    c->h_mail[100] = n;
-    CUDA_TRY(cudaMemcpyAsync(c->d_counts + C_N_SCAN, &c->h_mail[100], sizeof(int), cudaMemcpyHostToDevice, c->stream));
+    c->h_mail.p[100] = n;
+    CUDA_TRY(cudaMemcpyAsync(c->d_counts + C_N_SCAN, &c->h_mail.p[100], sizeof(int), cudaMemcpyHostToDevice, c->stream));
     CUDA_TRY(cudaStreamSynchronize(c->stream));
     c->n_scan_bound = n; c->h_n_scan = n; c->h_n_ds = -1; c->launches += 1;
     return LIORF_OK;
@@ -675,15 +618,14 @@ int liorf_voxel_grid(liorf_ctx* c, const liorf_point* in, int n, float leaf, lio
     if ((rc = c->out_keys.reserve(cap))) return rc;
     if (n > 0) CUDA_TRY(cudaMemcpyAsync(c->map_raw.p, in, (size_t)n * sizeof(float4), cudaMemcpyHostToDevice, c->stream));
     rc = voxel_grid_device(c->map_raw.p, Count::of_host(n), leaf, tmp_out.p, c->d_counts + C_NSEL, c->membership.p, c->out_keys.p, c->vg, c->stream, c->num_sms);
-    if (rc) { tmp_out.release(); return rc; }
-    CUDA_TRY(cudaMemcpyAsync(c->h_mail + 200, c->d_counts + C_NSEL, sizeof(int), cudaMemcpyDeviceToHost, c->stream));
+    if (rc) return rc;
+    CUDA_TRY(cudaMemcpyAsync(c->h_mail.p + 200, c->d_counts + C_NSEL, sizeof(int), cudaMemcpyDeviceToHost, c->stream));
     CUDA_TRY(cudaStreamSynchronize(c->stream));
-    int no = c->h_mail[200]; *n_out = no;
+    int no = c->h_mail.p[200]; *n_out = no;
     if (out && no > 0) CUDA_TRY(cudaMemcpyAsync(out, tmp_out.p, (size_t)no * sizeof(float4), cudaMemcpyDeviceToHost, c->stream));
     if (membership && n > 0) CUDA_TRY(cudaMemcpyAsync(membership, c->membership.p, (size_t)n * sizeof(int), cudaMemcpyDeviceToHost, c->stream));
     if (out_keys && no > 0) CUDA_TRY(cudaMemcpyAsync(out_keys, c->out_keys.p, (size_t)no * sizeof(int), cudaMemcpyDeviceToHost, c->stream));
     rc = check_err(c);
-    tmp_out.release();
     c->map_valid = false;                                 // map_raw scratch was reused
     return rc;
 }
@@ -741,16 +683,14 @@ int liorf_extract_surrounding_keyframes(liorf_ctx* c, const int* ids, int n_ids,
         return LIORF_OK;
     }
     const int ns = (int)sel.size();
-    if (ns + 1 > c->h_sel_cap) {
+    if ((size_t)ns + 1 > c->h_sel.cap / 2) {
         CUDA_TRY(cudaStreamSynchronize(c->stream));
         if (c->stream_map) CUDA_TRY(cudaStreamSynchronize(c->stream_map));
-        if (c->h_sel) cudaFreeHost(c->h_sel);
-        c->h_sel_cap = 2 * ns + 64;
-        CUDA_TRY(cudaHostAlloc(&c->h_sel, (size_t)2 * c->h_sel_cap * sizeof(KfSel), cudaHostAllocDefault));
+        if ((rc = c->h_sel.reserve((size_t)2 * (2 * ns + 64)))) return rc;
     }
     if ((rc = c->d_sel.reserve(ns + 1))) return rc;
     const int slot = stage_slot(c, 0); if (slot < 0) return LIORF_ERR_CUDA;
-    KfSel* hsel = c->h_sel + (size_t)slot * c->h_sel_cap;      // entry 0 = header {nsel, total}, selections from entry 1
+    KfSel* hsel = c->h_sel.p + (size_t)slot * (c->h_sel.cap / 2);      // entry 0 = header {nsel, total}, selections from entry 1
     long long total = 0;
     for (int i = 0; i < ns; ++i) {
         const Keyframe& k = c->kfs[sel[i]];
@@ -805,23 +745,24 @@ int liorf_extract_surrounding_keyframes(liorf_ctx* c, const int* ids, int n_ids,
         const void* sig[20] = {c->kf_points.p, c->d_sel.p, c->map_raw.p, c->map_ds.p, w.partial.p, w.keys.p, w.seg_start.p, w.sort.keys_alt.p, w.sort.vals_a.p,
                                w.sort.vals_b.p, w.sort.hist.p, w.sort.status.p, w.scan.status.p, gr.counts.p, gr.cell_start.p, gr.sorted.p, gr.scan.status.p,
                                w.meta, (const void*)(size_t)(w.force_large | (w.force_multi << 1) | (c->map_vg_grid << 2)), w.pts_sorted.p};
-        if (G.vg && std::memcmp(sig, G.sig, sizeof(sig)) != 0) { cudaGraphExecDestroy(G.vg); cudaGraphExecDestroy(G.grid); G.vg = G.grid = nullptr; }
+        if (G.vg && std::memcmp(sig, G.sig, sizeof(sig)) != 0) { G.vg.reset(); G.grid.reset(); }
         if (!G.vg) {
             const bool prof_on = c->prof.enabled; c->prof.enabled = false;          // no timing events inside a capture
-            cudaGraph_t g1 = nullptr, g2 = nullptr;
+            Graph g1, g2;
             CUDA_TRY(cudaStreamBeginCapture(ms, cudaStreamCaptureModeThreadLocal));
             rc = enqueue_vg();
-            cudaError_t e1 = cudaStreamEndCapture(ms, &g1);
+            cudaError_t e1 = end_capture(g1, ms);
             if (!rc && e1 == cudaSuccess) {
                 CUDA_TRY(cudaStreamBeginCapture(ms, cudaStreamCaptureModeThreadLocal));
                 rc = enqueue_grid();
-                e1 = cudaStreamEndCapture(ms, &g2);
+                e1 = end_capture(g2, ms);
             }
             c->prof.enabled = prof_on;
-            if (rc || e1 != cudaSuccess) { if (g1) cudaGraphDestroy(g1); if (g2) cudaGraphDestroy(g2); return rc ? rc : LIORF_ERR_CUDA; }
-            CUDA_TRY(cudaGraphInstantiate(&G.vg, g1, 0));
-            CUDA_TRY(cudaGraphInstantiate(&G.grid, g2, 0));
-            cudaGraphDestroy(g1); cudaGraphDestroy(g2);
+            if (rc || e1 != cudaSuccess) return rc ? rc : LIORF_ERR_CUDA;
+            GraphExec vg, grid;                     // the pair is kept only when both instantiate
+            CUDA_TRY(graph_instantiate(vg, g1));
+            CUDA_TRY(graph_instantiate(grid, g2));
+            G.vg = std::move(vg); G.grid = std::move(grid);
             std::memcpy(G.sig, sig, sizeof(sig));
         }
         { ProfScope ps(c, SEC_MAP_BUILD, ms); c->launches += 10; CUDA_TRY(cudaGraphLaunch(G.vg, ms)); }
@@ -919,8 +860,8 @@ int liorf_set_local_map(liorf_ctx* c, const liorf_point* map_ds, int m) {
     if ((rc = join_map(c))) return rc;
     if ((rc = c->map_ds.reserve(m > 0 ? m : 1))) return rc;
     if (m > 0) CUDA_TRY(cudaMemcpyAsync(c->map_ds.p, map_ds, (size_t)m * sizeof(float4), cudaMemcpyHostToDevice, c->stream));
-    c->h_mail[101] = m;
-    CUDA_TRY(cudaMemcpyAsync(c->d_shared + C_M_DS, &c->h_mail[101], sizeof(int), cudaMemcpyHostToDevice, c->stream));
+    c->h_mail.p[101] = m;
+    CUDA_TRY(cudaMemcpyAsync(c->d_shared + C_M_DS, &c->h_mail.p[101], sizeof(int), cudaMemcpyHostToDevice, c->stream));
     c->m_bound = m; c->h_m_ds = m; c->map_valid = false;
     if ((rc = build_map_grid(c->map_ds.p, Count::of_host(m), c->grid, c->stream))) return rc;
     return check_err(c);
@@ -1013,15 +954,15 @@ int liorf_get_pose(liorf_ctx* c, float pose6[6], liorf_lm_trace* trace) {
     if (!c || !pose6) return LIORF_ERR_ARG;
     CUDA_TRY(cudaSetDevice(c->P.device));
     { int rcj = join_map(c); if (rcj) return rcj; }
-    CUDA_TRY(cudaMemcpyAsync(c->h_mail + 320, c->d_tf6, 6 * sizeof(float), cudaMemcpyDeviceToHost, c->stream));
+    CUDA_TRY(cudaMemcpyAsync(c->h_mail.p + 320, c->d_tf6, 6 * sizeof(float), cudaMemcpyDeviceToHost, c->stream));
     CUDA_TRY(mail_counts(c));
-    if (trace) CUDA_TRY(cudaMemcpyAsync(c->h_mail + 1024, c->d_trace, sizeof(S2MTrace), cudaMemcpyDeviceToHost, c->stream));
-    else CUDA_TRY(cudaMemcpyAsync(c->h_mail + 1024 + 448, &c->d_trace->iters, 4 * sizeof(int), cudaMemcpyDeviceToHost, c->stream));
+    if (trace) CUDA_TRY(cudaMemcpyAsync(c->h_mail.p + 1024, c->d_trace, sizeof(S2MTrace), cudaMemcpyDeviceToHost, c->stream));
+    else CUDA_TRY(cudaMemcpyAsync(c->h_mail.p + 1024 + 448, &c->d_trace->iters, 4 * sizeof(int), cudaMemcpyDeviceToHost, c->stream));
     int rc = check_err(c); if (rc) return rc;
     take_counts(c);                                              // one round trip refreshes the counts too
     c->rep_counts[0] = c->h_n_scan; c->rep_counts[1] = c->h_n_ds; c->rep_counts[2] = c->h_m_ds;
-    std::memcpy(pose6, c->h_mail + 320, 6 * sizeof(float));
-    if (trace) std::memcpy(trace, c->h_mail + 1024, sizeof(S2MTrace));
+    std::memcpy(pose6, c->h_mail.p + 320, 6 * sizeof(float));
+    if (trace) std::memcpy(trace, c->h_mail.p + 1024, sizeof(S2MTrace));
     return LIORF_OK;
 }
 // liorf_process_frame's round trip: the solver left everything the host needs in ONE 64-byte record (pose, iteration count,
@@ -1029,11 +970,11 @@ int liorf_get_pose(liorf_ctx* c, float pose6[6], liorf_lm_trace* trace) {
 static int get_pose_mail(liorf_ctx* c, float pose6[6], int* iters, int* converged, int* degenerate, int* ran) {
     if (!c->mail_fresh) {
         int rc = liorf_get_pose(c, pose6, nullptr); if (rc) return rc;
-        *iters = c->h_mail[1024 + 448]; *converged = c->h_mail[1024 + 449]; *degenerate = c->h_mail[1024 + 450]; *ran = c->h_mail[1024 + 451];
+        *iters = c->h_mail.p[1024 + 448]; *converged = c->h_mail.p[1024 + 449]; *degenerate = c->h_mail.p[1024 + 450]; *ran = c->h_mail.p[1024 + 451];
         return LIORF_OK;
     }
     c->mail_fresh = false;
-    S2MMail* hm = reinterpret_cast<S2MMail*>(c->h_mail + 3200);
+    S2MMail* hm = reinterpret_cast<S2MMail*>(c->h_mail.p + 3200);
     CUDA_TRY(cudaMemcpyAsync(hm, c->d_mail, sizeof(S2MMail), cudaMemcpyDeviceToHost, c->stream));
     CUDA_TRY(cudaStreamSynchronize(c->stream));
     prof_flush(c);
@@ -1042,7 +983,7 @@ static int get_pose_mail(liorf_ctx* c, float pose6[6], int* iters, int* converge
     *iters = hm->iters; *converged = hm->converged; *degenerate = hm->degenerate; *ran = hm->ran;
     c->h_n_scan = hm->n_scan; c->h_n_ds = hm->n_ds; c->h_m_ds = hm->m_ds;
     c->rep_counts[0] = c->h_n_scan; c->rep_counts[1] = c->h_n_ds; c->rep_counts[2] = c->h_m_ds;
-    c->h_mail[1024 + 448] = hm->iters;                           // liorf_get_last_counts reads the iteration count here
+    c->h_mail.p[1024 + 448] = hm->iters;                           // liorf_get_last_counts reads the iteration count here
     return LIORF_OK;
 }
 
@@ -1090,9 +1031,9 @@ int liorf_combine_optimization_coeffs(liorf_ctx* c, liorf_point* ori, liorf_poin
     if ((rc = c->h_ori_c.reserve(cap)) || (rc = c->h_coeff_c.reserve(cap))) return rc;
     if ((rc = launch_scan(Count::of_host(n), FlagLoad{c->h_flag.p}, CombineStore{c->scan_ds.p, c->h_coeff.p, c->h_ori_c.p, c->h_coeff_c.p}, c->combine_scan,
                           (unsigned*)(c->d_counts + C_HOOK_NSEL), c->stream))) return rc;
-    CUDA_TRY(cudaMemcpyAsync(c->h_mail + 400, c->d_counts + C_HOOK_NSEL, sizeof(int), cudaMemcpyDeviceToHost, c->stream));
+    CUDA_TRY(cudaMemcpyAsync(c->h_mail.p + 400, c->d_counts + C_HOOK_NSEL, sizeof(int), cudaMemcpyDeviceToHost, c->stream));
     CUDA_TRY(cudaStreamSynchronize(c->stream));
-    const int ns = c->h_mail[400]; *n_sel = ns;
+    const int ns = c->h_mail.p[400]; *n_sel = ns;
     if (ori && ns > 0) CUDA_TRY(cudaMemcpyAsync(ori, c->h_ori_c.p, (size_t)ns * sizeof(float4), cudaMemcpyDeviceToHost, c->stream));
     if (coeff && ns > 0) CUDA_TRY(cudaMemcpyAsync(coeff, c->h_coeff_c.p, (size_t)ns * sizeof(float4), cudaMemcpyDeviceToHost, c->stream));
     return check_err(c);
@@ -1110,17 +1051,17 @@ int liorf_lm_optimization(liorf_ctx* c, int iter, float pose6[6], float AtA[36],
                                              c->lm_partial.p, c->d_misc + 7, c->d_lm_out, c->d_lm_out + 36, c->d_lm_out + 42, c->d_counts + C_NSEL,
                                              c->d_counts + C_CONV);
     CUDA_TRY(cudaGetLastError());
-    CUDA_TRY(cudaMemcpyAsync(c->h_mail + 320, c->d_tf6, 6 * sizeof(float), cudaMemcpyDeviceToHost, c->stream));
-    CUDA_TRY(cudaMemcpyAsync(c->h_mail + 500, c->d_lm_out, 48 * sizeof(float), cudaMemcpyDeviceToHost, c->stream));
-    CUDA_TRY(cudaMemcpyAsync(c->h_mail + 600, c->d_counts, C_COUNT * sizeof(int), cudaMemcpyDeviceToHost, c->stream));
+    CUDA_TRY(cudaMemcpyAsync(c->h_mail.p + 320, c->d_tf6, 6 * sizeof(float), cudaMemcpyDeviceToHost, c->stream));
+    CUDA_TRY(cudaMemcpyAsync(c->h_mail.p + 500, c->d_lm_out, 48 * sizeof(float), cudaMemcpyDeviceToHost, c->stream));
+    CUDA_TRY(cudaMemcpyAsync(c->h_mail.p + 600, c->d_counts, C_COUNT * sizeof(int), cudaMemcpyDeviceToHost, c->stream));
     if ((rc = check_err(c))) return rc;
-    std::memcpy(pose6, c->h_mail + 320, 6 * sizeof(float));
-    const float* o = reinterpret_cast<const float*>(c->h_mail + 500);
+    std::memcpy(pose6, c->h_mail.p + 320, 6 * sizeof(float));
+    const float* o = reinterpret_cast<const float*>(c->h_mail.p + 500);
     if (AtA) std::memcpy(AtA, o, 36 * sizeof(float));
     if (AtB) std::memcpy(AtB, o + 36, 6 * sizeof(float));
     if (X) std::memcpy(X, o + 42, 6 * sizeof(float));
-    if (n_sel) *n_sel = c->h_mail[600 + C_NSEL];
-    return c->h_mail[600 + C_CONV] ? 1 : 0;
+    if (n_sel) *n_sel = c->h_mail.p[600 + C_NSEL];
+    return c->h_mail.p[600 + C_CONV] ? 1 : 0;
 }
 int liorf_get_lm_state(liorf_ctx* c, int* deg, float matP[36]) {
     LIORF_NVTX;
@@ -1158,7 +1099,7 @@ int liorf_sc_make_and_save(liorf_ctx* c, const liorf_point* cloud, int n) {
     } else {
         d_pts = c->scan.p; cnt = c->h_n_scan >= 0 ? Count::of_host(c->h_n_scan) : Count::of_dev(c->d_counts + C_N_SCAN, c->n_scan_bound);
     }
-    if (c->sc_borrowed) return LIORF_ERR_STATE;
+    if (c->sc_borrowed()) return LIORF_ERR_STATE;
     if ((rc = sc_reserve(c, c->sc_n + 1))) return rc;
     ProfScope ps(c, SEC_SC_MAKE); c->launches += 2;
     if (cnt.bound > 0) {
@@ -1166,8 +1107,8 @@ int liorf_sc_make_and_save(liorf_ctx* c, const liorf_point* cloud, int n) {
         k_sc_bins<<<blocks, 256, 0, c->stream>>>(d_pts, cnt, c->d_bins);
     }
     const size_t e = (size_t)c->sc_n;
-    k_sc_finalize<<<1, 64, 0, c->stream>>>(c->d_bins, nullptr, c->sc_desc.p + e * SC_DESC, c->sc_keys.p + e * SC_RING, c->sc_sk.p + e * SC_SECTOR,
-                                           c->sc_cn.p + e * SC_SECTOR);
+    k_sc_finalize<<<1, 64, 0, c->stream>>>(c->d_bins, nullptr, c->sc_db->desc.p + e * SC_DESC, c->sc_db->keys.p + e * SC_RING, c->sc_db->sk.p + e * SC_SECTOR,
+                                           c->sc_db->cn.p + e * SC_SECTOR);
     CUDA_TRY(cudaGetLastError());
     ++c->sc_n;
     if (cloud) CUDA_TRY(cudaStreamSynchronize(c->stream));
@@ -1180,12 +1121,12 @@ int liorf_sc_add_descriptors(liorf_ctx* c, const double* descs, int count) {
     CUDA_TRY(cudaSetDevice(c->P.device));
     int rc;
     if (count == 0) return LIORF_OK;
-    if (c->sc_borrowed) return LIORF_ERR_STATE;
+    if (c->sc_borrowed()) return LIORF_ERR_STATE;
     if ((rc = sc_reserve(c, c->sc_n + count))) return rc;
     const size_t e = (size_t)c->sc_n;
-    CUDA_TRY(cudaMemcpyAsync(c->sc_desc.p + e * SC_DESC, descs, (size_t)count * SC_DESC * sizeof(double), cudaMemcpyHostToDevice, c->stream));
-    k_sc_keys_batch<<<count, 64, 0, c->stream>>>(c->sc_desc.p + e * SC_DESC, count, c->sc_keys.p + e * SC_RING, c->sc_sk.p + e * SC_SECTOR,
-                                                 c->sc_cn.p + e * SC_SECTOR);
+    CUDA_TRY(cudaMemcpyAsync(c->sc_db->desc.p + e * SC_DESC, descs, (size_t)count * SC_DESC * sizeof(double), cudaMemcpyHostToDevice, c->stream));
+    k_sc_keys_batch<<<count, 64, 0, c->stream>>>(c->sc_db->desc.p + e * SC_DESC, count, c->sc_db->keys.p + e * SC_RING, c->sc_db->sk.p + e * SC_SECTOR,
+                                                 c->sc_db->cn.p + e * SC_SECTOR);
     CUDA_TRY(cudaGetLastError());
     c->sc_n += count;
     CUDA_TRY(cudaStreamSynchronize(c->stream));
@@ -1197,13 +1138,12 @@ int liorf_sc_add_descriptors(liorf_ctx* c, const double* descs, int count) {
 int liorf_sc_borrow_database(liorf_ctx* dst, liorf_ctx* src) {
     LIORF_NVTX;
     if (!dst || !src || dst == src || dst->P.device != src->P.device) return LIORF_ERR_ARG;
-    if (!dst->sc_borrowed && (dst->sc_n != 0 || dst->sc_desc.p)) return LIORF_ERR_STATE;
+    if (!dst->sc_borrowed() && (dst->sc_n != 0 || dst->sc_own.desc.p)) return LIORF_ERR_STATE;
     CUDA_TRY(cudaSetDevice(src->P.device));
     CUDA_TRY(cudaStreamSynchronize(src->stream));
-    dst->sc_desc = src->sc_desc; dst->sc_sk = src->sc_sk; dst->sc_cn = src->sc_cn; dst->sc_keys = src->sc_keys; dst->sc_n = src->sc_n;
+    dst->sc_db = src->sc_db; dst->sc_n = src->sc_n;            // borrowing from a borrower reads the owner's database
     // a sharded owner's replicated index (liorf_sc_shard_sync_keys) is shared too; the borrower builds its own operand image from it
     dst->ks_all.keys = src->ks_all.keys; dst->ks_all.n = src->ks_all.n; dst->ks_all.gen = src->ks_all.gen;
-    dst->sc_borrowed = true;
     return LIORF_OK;
 }
 int liorf_sc_size(liorf_ctx* c) { return c ? c->sc_n : LIORF_ERR_ARG; }
@@ -1212,9 +1152,9 @@ int liorf_sc_get(liorf_ctx* c, int i, double desc[1200], float ringkey[20], doub
     if (!c || i < 0 || i >= c->sc_n) return LIORF_ERR_ARG;
     CUDA_TRY(cudaSetDevice(c->P.device));
     CUDA_TRY(cudaStreamSynchronize(c->stream));
-    if (desc) CUDA_TRY(cudaMemcpy(desc, c->sc_desc.p + (size_t)i * SC_DESC, SC_DESC * sizeof(double), cudaMemcpyDeviceToHost));
-    if (ringkey) CUDA_TRY(cudaMemcpy(ringkey, c->sc_keys.p + (size_t)i * SC_RING, SC_RING * sizeof(float), cudaMemcpyDeviceToHost));
-    if (sectorkey) CUDA_TRY(cudaMemcpy(sectorkey, c->sc_sk.p + (size_t)i * SC_SECTOR, SC_SECTOR * sizeof(double), cudaMemcpyDeviceToHost));
+    if (desc) CUDA_TRY(cudaMemcpy(desc, c->sc_db->desc.p + (size_t)i * SC_DESC, SC_DESC * sizeof(double), cudaMemcpyDeviceToHost));
+    if (ringkey) CUDA_TRY(cudaMemcpy(ringkey, c->sc_db->keys.p + (size_t)i * SC_RING, SC_RING * sizeof(float), cudaMemcpyDeviceToHost));
+    if (sectorkey) CUDA_TRY(cudaMemcpy(sectorkey, c->sc_db->sk.p + (size_t)i * SC_SECTOR, SC_SECTOR * sizeof(double), cudaMemcpyDeviceToHost));
     return LIORF_OK;
 }
 
@@ -1243,11 +1183,9 @@ static int sc_knn_brute(liorf_ctx* c, const float* d_keys, int n_keys, const flo
 static int sct_prepare(liorf_ctx* c, liorf_ctx::KeySet& ks, int n_keys, const float* d_qkeys, int Q, SctArgs& a, int& grid) {
     int rc;
     const int nkt = (n_keys + SCT_KT - 1) / SCT_KT, n_sqt = (Q + SCT_QT - 1) / SCT_QT;
-    if (!ks.center) {
-        CUDA_TRY(cudaMalloc(&ks.center, SC_RING * sizeof(float)));
-        CUDA_TRY(cudaMalloc(&ks.nmax, sizeof(unsigned)));
-    }
-    if (!c->sct_over_cnt) { CUDA_TRY(cudaMalloc(&c->sct_over_cnt, sizeof(int))); CUDA_TRY(cudaMemsetAsync(c->sct_over_cnt, 0, sizeof(int), c->stream)); }
+    if (!ks.center) CUDA_TRY(dev_alloc(ks.center, SC_RING));
+    if (!ks.nmax) CUDA_TRY(dev_alloc(ks.nmax, 1));
+    if (!c->sct_over_cnt) { CUDA_TRY(dev_alloc(c->sct_over_cnt, 1)); CUDA_TRY(cudaMemsetAsync(c->sct_over_cnt, 0, sizeof(int), c->stream)); }
     if (!c->sct_attr_set) {
         CUDA_TRY(cudaFuncSetAttribute(k_sc_tensor<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, SCT_SMEM));
         CUDA_TRY(cudaFuncSetAttribute(k_sc_tensor<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, SCT_SMEM));
@@ -1312,7 +1250,7 @@ static int sc_knn(liorf_ctx* c, liorf_ctx::KeySet& ks, int n_keys, const float* 
     if (sc_want_tensor(c, Q, n_keys)) return sc_knn_tensor(c, ks, n_keys, d_qkeys, Q, idx_offset, d_dist, d_idx);
     return sc_knn_brute(c, ks.keys, n_keys, d_qkeys, Q, idx_offset, d_dist, d_idx);
 }
-static liorf_ctx::KeySet& local_keys(liorf_ctx* c) { c->ks_local.keys = c->sc_keys.p; c->ks_local.n = c->sc_n; return c->ks_local; }
+static liorf_ctx::KeySet& local_keys(liorf_ctx* c) { c->ks_local.keys = c->sc_db->keys.p; c->ks_local.n = c->sc_n; return c->ks_local; }
 
 // shared-memory limit and occupancy of both instantiations of the stage-2 kernel, once per context
 static int scdb_setup(liorf_ctx* c) {
@@ -1347,9 +1285,9 @@ static int sc_distance_launch(liorf_ctx* c, const double* qd, const int* cand, i
     if (blocks < 1) blocks = 1;                                   // a rank that owns no pair still raises its phase-D flag
     ShardPush P; std::memset(&P, 0, sizeof(P));
     if (push) P = *push;
-    if (q16) k_sc_distance_bulk<true><<<blocks, SCDB_THREADS, SCDB_SMEM, c->stream>>>(qd, cand, pairs, SC_NUM_CAND, c->sc_desc.p, c->sc_sk.p, c->sc_cn.p, global_offset,
+    if (q16) k_sc_distance_bulk<true><<<blocks, SCDB_THREADS, SCDB_SMEM, c->stream>>>(qd, cand, pairs, SC_NUM_CAND, c->sc_db->desc.p, c->sc_db->sk.p, c->sc_db->cn.p, global_offset,
                                                                                     c->sc_n, pd, ps, c->d_err, pair_list, n_list, P);
-    else k_sc_distance_bulk<false><<<blocks, SCDB_THREADS, SCDB_SMEM, c->stream>>>(qd, cand, pairs, SC_NUM_CAND, c->sc_desc.p, c->sc_sk.p, c->sc_cn.p, global_offset,
+    else k_sc_distance_bulk<false><<<blocks, SCDB_THREADS, SCDB_SMEM, c->stream>>>(qd, cand, pairs, SC_NUM_CAND, c->sc_db->desc.p, c->sc_db->sk.p, c->sc_db->cn.p, global_offset,
                                                                                  c->sc_n, pd, ps, c->d_err, pair_list, n_list, P);
     CUDA_TRY(cudaGetLastError());
     c->launches += 1;
@@ -1417,9 +1355,7 @@ int liorf_debug_qr_solve6(liorf_ctx* c, const float* A, const float* b, int n, f
     k_debug_qr6<<<(n + 1) / 2, 64, 0, c->stream>>>(dA, db, n, dx, c->d_err);
     CUDA_TRY(cudaGetLastError());
     CUDA_TRY(cudaMemcpyAsync(x, dx, (size_t)6 * n * sizeof(float), cudaMemcpyDeviceToHost, c->stream));
-    rc = check_err(c);
-    d.release();
-    return rc;
+    return check_err(c);
 }
 /* tests: 1 = run the multi-kernel (large-cloud) VoxelGrid path on small clouds too; 0 = automatic */
 int liorf_debug_force_large_voxelgrid(liorf_ctx* c, int on) {
@@ -1435,9 +1371,9 @@ int liorf_debug_voxelgrid_stamps(liorf_ctx* c, int enable, unsigned long long* o
     if (!c) return LIORF_ERR_ARG;
     CUDA_TRY(cudaSetDevice(c->P.device));
     CUDA_TRY(cudaStreamSynchronize(c->stream));
-    if (enable && !c->vg.dbg) { CUDA_TRY(cudaMalloc(&c->vg.dbg, 32 * sizeof(unsigned long long))); CUDA_TRY(cudaMemset(c->vg.dbg, 0, 32 * sizeof(unsigned long long))); }
+    if (enable && !c->vg.dbg) { CUDA_TRY(dev_alloc(c->vg.dbg, 32)); CUDA_TRY(cudaMemset(c->vg.dbg, 0, 32 * sizeof(unsigned long long))); }
     if (out && c->vg.dbg) CUDA_TRY(cudaMemcpy(out, c->vg.dbg, 32 * sizeof(unsigned long long), cudaMemcpyDeviceToHost));
-    if (!enable && c->vg.dbg) { cudaFree(c->vg.dbg); c->vg.dbg = nullptr; }
+    if (!enable) c->vg.dbg.reset();
     return LIORF_OK;
 }
 /* tests: 1 = run the one-kernel cooperative VoxelGrid path on small clouds too; 0 = automatic */
@@ -1493,9 +1429,7 @@ int liorf_sc_tensor_dump(liorf_ctx* c, const float* qkeys, int Q, float* out, lo
     CUDA_TRY(cudaGetLastError());
     CUDA_TRY(cudaMemcpyAsync(out, dump.p, (size_t)Q * cols * sizeof(float), cudaMemcpyDeviceToHost, c->stream));
     if (center) CUDA_TRY(cudaMemcpyAsync(center, ks.center, SC_RING * sizeof(float), cudaMemcpyDeviceToHost, c->stream));
-    rc = check_err(c);
-    dump.release();
-    return rc;
+    return check_err(c);
 }
 
 static int sc_reserve_query(liorf_ctx* c, int Q) {
@@ -1555,10 +1489,10 @@ int liorf_sc_shard_init(liorf_ctx* c, int rank, int world, int q_max, int k_tota
     S.W.off_d = S.W.off_c + scsh_round((size_t)q_max * 24);
     S.off_keys = S.W.off_d + scsh_round((size_t)q_max * 36);
     S.win_bytes = S.off_keys + scsh_round((size_t)k_total_max * SC_RING * sizeof(float));
-    unsigned char* win = nullptr;
-    CUDA_TRY(cudaMalloc(&win, S.win_bytes));
+    CUDA_TRY(dev_alloc(S.win, S.win_bytes));
+    unsigned char* win = S.win;
     CUDA_TRY(cudaMemset(win, 0, S.win_bytes));
-    CUDA_TRY(cudaMalloc(&S.d_counter, 4 * sizeof(unsigned) + SCSH_NPHASE * sizeof(unsigned long long)));
+    CUDA_TRY(dev_alloc(S.d_counter, 4 + SCSH_NPHASE * sizeof(unsigned long long) / sizeof(unsigned)));
     CUDA_TRY(cudaMemset(S.d_counter, 0, 4 * sizeof(unsigned) + SCSH_NPHASE * sizeof(unsigned long long)));
     S.d_nlist = reinterpret_cast<int*>(S.d_counter + 2);
     S.d_batch = S.d_counter + 1;
@@ -1598,9 +1532,8 @@ int liorf_sc_shard_connect(liorf_ctx* c, const void* ipc_handles /*world x 64 B,
             if (window_ptrs) S.W.base[g] = (unsigned char*)window_ptrs[g];               // same process: the peer context's pointer is directly usable
             else {
                 cudaIpcMemHandle_t h; std::memcpy(&h, (const unsigned char*)ipc_handles + (size_t)64 * g, 64);
-                void* p = nullptr;
-                CUDA_TRY(cudaIpcOpenMemHandle(&p, h, cudaIpcMemLazyEnablePeerAccess));
-                S.W.base[g] = (unsigned char*)p; S.ipc_opened[g] = true;
+                CUDA_TRY(ipc_open(S.ipc[g], h));
+                S.W.base[g] = S.ipc[g];
             }
             if (!S.W.base[g]) return LIORF_ERR_ARG;
         }
@@ -1623,7 +1556,7 @@ int liorf_sc_shard_sync_keys_phases(liorf_ctx* c, int phases) {
         ++S.keys_gen; S.keys_pushed = true;
         const size_t words = (size_t)c->sc_n * SC_RING;
         const int blocks = (int)std::max<size_t>(1, std::min<size_t>(4 * c->num_sms, (words + 1023) / 1024));
-        k_scsh_push_keys<<<blocks, 256, 0, c->stream>>>(S.W, c->sc_keys.p, c->sc_n, S.keys_gen, S.d_counter);
+        k_scsh_push_keys<<<blocks, 256, 0, c->stream>>>(S.W, c->sc_db->keys.p, c->sc_n, S.keys_gen, S.d_counter);
         CUDA_TRY(cudaGetLastError());
         c->launches += 1;
     }
@@ -1659,7 +1592,7 @@ int liorf_sc_shard_debug_nowait(liorf_ctx* c, int on) {
     LIORF_NVTX;
     if (!c) return LIORF_ERR_ARG;
     c->shard.W.nowait = on != 0;
-    if (c->shard.graph) { cudaGraphExecDestroy(c->shard.graph); c->shard.graph = nullptr; }
+    c->shard.graph.reset();
     return LIORF_OK;
 }
 
@@ -1732,7 +1665,7 @@ int liorf_sc_shard_query_dev(liorf_ctx* c, const void* d_qdescs, int Q, int glob
         const void* v[40] = {d_qdescs, (const void*)(size_t)Q, (const void*)(size_t)global_offset, d_loop_id, d_shift, d_dist, d_cand, (const void*)(size_t)c->sc_n,
                              (const void*)(size_t)ks.n, (const void*)(size_t)ks.gen, (const void*)(size_t)ks.img_n, (const void*)(size_t)ks.img_gen, ks.keys, ks.bimg.p, ks.center,
                              (const void*)(size_t)c->sc_path, (const void*)(size_t)S.W.nowait,
-                             c->sc_desc.p, c->sc_sk.p, c->sc_cn.p, c->sc_keys.p, c->sc_qkeys.p, c->sc_q_d.p, c->sc_q_i.p, c->sc_pair_d.p, c->sc_pair_s.p, c->sc_part_d.p, c->sc_part_i.p,
+                             c->sc_db->desc.p, c->sc_db->sk.p, c->sc_db->cn.p, c->sc_db->keys.p, c->sc_qkeys.p, c->sc_q_d.p, c->sc_q_i.p, c->sc_pair_d.p, c->sc_pair_s.p, c->sc_part_d.p, c->sc_part_i.p,
                              S.list.p, c->sct_aimg.p, c->sct_qnorm.p, c->sct_cmin.p, c->sct_cmin32.p, c->sct_part.p, c->sct_cand.p, c->sct_cnt.p, c->sct_over_cnt, nullptr, nullptr, nullptr};
         std::memcpy(sig, v, sizeof(v));
     };
@@ -1746,21 +1679,20 @@ int liorf_sc_shard_query_dev(liorf_ctx* c, const void* d_qdescs, int Q, int glob
     }
     if (std::memcmp(sig, S.last_sig, sizeof(sig)) == 0) {        // second identical request: every buffer is sized and the operand image is current → capture
         CUDA_TRY(cudaSetDevice(c->P.device));
-        if (S.graph) { cudaGraphExecDestroy(S.graph); S.graph = nullptr; }
-        cudaGraph_t g = nullptr;
+        S.graph.reset();
+        Graph g;
         const long long launches0 = c->launches;
         CUDA_TRY(cudaStreamBeginCapture(c->stream, cudaStreamCaptureModeThreadLocal));
         const int rc = liorf_sc_shard_query_phases_dev(c, d_qdescs, Q, global_offset, d_loop_id, d_shift, d_dist, d_cand, 7);
-        const cudaError_t e = cudaStreamEndCapture(c->stream, &g);
+        const cudaError_t e = end_capture(g, c->stream);
         c->launches = launches0;
-        if (rc || e != cudaSuccess) { if (g) cudaGraphDestroy(g); (void)cudaGetLastError(); return rc ? rc : LIORF_ERR_CUDA; }
+        if (rc || e != cudaSuccess) { (void)cudaGetLastError(); return rc ? rc : LIORF_ERR_CUDA; }
         make_sig(sig);
         if (std::memcmp(sig, S.last_sig, sizeof(sig)) != 0) {     // something was (re)allocated or rebuilt during the capture after all: do not keep it
-            cudaGraphDestroy(g); std::memset(S.last_sig, 0, sizeof(S.last_sig));
+            std::memset(S.last_sig, 0, sizeof(S.last_sig));
             return liorf_sc_shard_query_phases_dev(c, d_qdescs, Q, global_offset, d_loop_id, d_shift, d_dist, d_cand, 7);
         }
-        CUDA_TRY(cudaGraphInstantiate(&S.graph, g, 0));
-        cudaGraphDestroy(g);
+        CUDA_TRY(graph_instantiate(S.graph, g));
         std::memcpy(S.gsig, sig, sizeof(sig));
         CUDA_TRY(cudaGraphLaunch(S.graph, c->stream));
         c->launches += 11;
@@ -1803,22 +1735,22 @@ int liorf_sc_detect_loop_closure_id(liorf_ctx* c, int* loop_id, float* yaw_diff_
     int rc;
     if ((rc = sc_reserve_query(c, 1))) return rc;
     const size_t qe = (size_t)c->sc_n - 1;                                       // query = last entry (:257-258)
-    if ((rc = sc_knn(c, local_keys(c), c->sc_tree_n, c->sc_keys.p + qe * SC_RING, 1, 0, c->sc_q_d.p, c->sc_q_i.p))) return rc;
+    if ((rc = sc_knn(c, local_keys(c), c->sc_tree_n, c->sc_db->keys.p + qe * SC_RING, 1, 0, c->sc_q_d.p, c->sc_q_i.p))) return rc;
     // result slots are zero-initialised in the reference (:289-290): an unfilled slot means candidate 0
-    CUDA_TRY(cudaMemcpyAsync(c->h_mail + 700, c->sc_q_i.p, 3 * sizeof(int), cudaMemcpyDeviceToHost, c->stream));
+    CUDA_TRY(cudaMemcpyAsync(c->h_mail.p + 700, c->sc_q_i.p, 3 * sizeof(int), cudaMemcpyDeviceToHost, c->stream));
     CUDA_TRY(cudaStreamSynchronize(c->stream));
-    int cand[3]; for (int j = 0; j < 3; ++j) { cand[j] = c->h_mail[700 + j]; if (cand[j] == 0x7fffffff) cand[j] = 0; c->h_mail[704 + j] = cand[j]; }
-    CUDA_TRY(cudaMemcpyAsync(c->sc_q_i.p, c->h_mail + 704, 3 * sizeof(int), cudaMemcpyHostToDevice, c->stream));
-    k_sc_distance<<<1, SCD_WARPS * 32, 0, c->stream>>>(c->sc_desc.p + qe * SC_DESC, c->sc_sk.p + qe * SC_SECTOR, c->sc_cn.p + qe * SC_SECTOR, c->sc_q_i.p, 3, 3,
-                                                       c->sc_desc.p, c->sc_sk.p, c->sc_cn.p, 0, c->sc_n, c->sc_pair_d.p, c->sc_pair_s.p);
+    int cand[3]; for (int j = 0; j < 3; ++j) { cand[j] = c->h_mail.p[700 + j]; if (cand[j] == 0x7fffffff) cand[j] = 0; c->h_mail.p[704 + j] = cand[j]; }
+    CUDA_TRY(cudaMemcpyAsync(c->sc_q_i.p, c->h_mail.p + 704, 3 * sizeof(int), cudaMemcpyHostToDevice, c->stream));
+    k_sc_distance<<<1, SCD_WARPS * 32, 0, c->stream>>>(c->sc_db->desc.p + qe * SC_DESC, c->sc_db->sk.p + qe * SC_SECTOR, c->sc_db->cn.p + qe * SC_SECTOR, c->sc_q_i.p, 3, 3,
+                                                       c->sc_db->desc.p, c->sc_db->sk.p, c->sc_db->cn.p, 0, c->sc_n, c->sc_pair_d.p, c->sc_pair_s.p);
     k_sc_decide<<<1, 128, 0, c->stream>>>(c->sc_pair_d.p, c->sc_pair_s.p, c->sc_q_i.p, 1, c->sc_res_i.p, c->sc_res_i.p + 1, c->sc_res_d.p);
     CUDA_TRY(cudaGetLastError());
-    CUDA_TRY(cudaMemcpyAsync(c->h_mail + 710, c->sc_res_i.p, 2 * sizeof(int), cudaMemcpyDeviceToHost, c->stream));
-    CUDA_TRY(cudaMemcpyAsync(c->h_mail + 720, c->sc_res_d.p, sizeof(double), cudaMemcpyDeviceToHost, c->stream));
+    CUDA_TRY(cudaMemcpyAsync(c->h_mail.p + 710, c->sc_res_i.p, 2 * sizeof(int), cudaMemcpyDeviceToHost, c->stream));
+    CUDA_TRY(cudaMemcpyAsync(c->h_mail.p + 720, c->sc_res_d.p, sizeof(double), cudaMemcpyDeviceToHost, c->stream));
     if ((rc = check_err(c))) return rc;
-    *loop_id = c->h_mail[710];
-    const int nn_align = c->h_mail[711];
-    double md; std::memcpy(&md, c->h_mail + 720, sizeof(double));
+    *loop_id = c->h_mail.p[710];
+    const int nn_align = c->h_mail.p[711];
+    double md; std::memcpy(&md, c->h_mail.p + 720, sizeof(double));
     if (min_dist) *min_dist = md;
     if (cand3) { cand3[0] = cand[0]; cand3[1] = cand[1]; cand3[2] = cand[2]; }
     *yaw_diff_rad = sc_yaw_rad(nn_align);
@@ -1844,28 +1776,26 @@ int liorf_sc_detect_loop_closure_id_batch(liorf_ctx* c, const int* n_db, const i
     int rc;
     if (Qd > 0) {
         const size_t io_ints = (size_t)9 * Qd;
-        if (io_ints > c->h_scdb_cap) {
-            if (c->h_scdb) { CUDA_TRY(cudaStreamSynchronize(c->stream)); CUDA_TRY(cudaFreeHost(c->h_scdb)); c->h_scdb = nullptr; c->h_scdb_cap = 0; }
-            const size_t cap = std::max<size_t>(io_ints, 1 << 16);
-            CUDA_TRY(cudaHostAlloc(&c->h_scdb, cap * sizeof(int), cudaHostAllocDefault));
-            c->h_scdb_cap = cap;
+        if (io_ints > c->h_scdb.cap) {
+            if (c->h_scdb.p) CUDA_TRY(cudaStreamSynchronize(c->stream));
+            if ((rc = c->h_scdb.reserve(std::max<size_t>(io_ints, 1 << 16)))) return rc;
         }
         if ((rc = c->scdb_io.reserve(io_ints)) || (rc = c->sc_qdesc.reserve((size_t)Qd * SC_DESC)) || (rc = c->sc_qkeys.reserve((size_t)Qd * SC_RING)) ||
             (rc = sc_reserve_query(c, Qd))) return rc;
-        int* H = c->h_scdb;
+        int* H = c->h_scdb.p;
         for (int q = 0, k = 0; q < Q; ++q)
             if (n_db[q] >= SC_EXCLUDE_RECENT + 1) { H[7 * Qd + k] = n_db[q]; H[8 * Qd + k] = n_tree[q]; ++k; }
         int* D = c->scdb_io.p;
         double* d_dist = reinterpret_cast<double*>(D);
         int *d_loop = D + 2 * Qd, *d_shift = D + 3 * Qd, *d_cand = D + 4 * Qd, *d_rows = D + 7 * Qd, *d_lim = D + 8 * Qd;
         CUDA_TRY(cudaMemcpyAsync(d_rows, H + 7 * Qd, (size_t)2 * Qd * sizeof(int), cudaMemcpyHostToDevice, c->stream));
-        k_sc_gather_queries<<<Qd, 128, 0, c->stream>>>(c->sc_desc.p, c->sc_keys.p, d_rows, Qd, c->sc_qdesc.p, c->sc_qkeys.p);
+        k_sc_gather_queries<<<Qd, 128, 0, c->stream>>>(c->sc_db->desc.p, c->sc_db->keys.p, d_rows, Qd, c->sc_qdesc.p, c->sc_qkeys.p);
         CUDA_TRY(cudaGetLastError());
         c->launches += 1;
         // stage 1 on the path the batch search would take for Qd queries against this database; the CUDA-core kernel needs to look no
         // further than the largest limit, the tensor-core filter keeps the database's operand image
         if (sc_want_tensor(c, Qd, c->sc_n)) rc = sc_knn_tensor(c, local_keys(c), c->sc_n, c->sc_qkeys.p, Qd, 0, c->sc_q_d.p, d_cand, nullptr, d_lim);
-        else rc = sc_knn_brute(c, c->sc_keys.p, max_tree, c->sc_qkeys.p, Qd, 0, c->sc_q_d.p, d_cand, d_lim);
+        else rc = sc_knn_brute(c, c->sc_db->keys.p, max_tree, c->sc_qkeys.p, Qd, 0, c->sc_q_d.p, d_cand, d_lim);
         if (rc) return rc;
         if (min_tree < SC_NUM_CAND) {
             k_sc_cand_unfilled_to_zero<<<(3 * Qd + 127) / 128, 128, 0, c->stream>>>(d_cand, 3 * Qd);
@@ -1877,7 +1807,7 @@ int liorf_sc_detect_loop_closure_id_batch(liorf_ctx* c, const int* n_db, const i
         CUDA_TRY(cudaMemcpyAsync(H, D, (size_t)7 * Qd * sizeof(int), cudaMemcpyDeviceToHost, c->stream));
         if ((rc = check_err(c))) return rc;
     }
-    const int* H = c->h_scdb;
+    const int* H = c->h_scdb.p;
     for (int q = 0, k = 0; q < Q; ++q) {
         loop_id[q] = -1; yaw_diff_rad[q] = 0.f;
         if (n_db[q] < SC_EXCLUDE_RECENT + 1) continue;
@@ -1925,9 +1855,9 @@ static int icp_build_cloud(liorf_ctx* c, int key, int search_num, int loop_index
     CUDA_TRY(cudaStreamSynchronize(c->stream));                      // `sel` is pageable host memory going out of scope
     k_transform_concat<<<(tot + 255) / 256, 256, 0, c->stream>>>(c->kf_points.p, c->icp_sel.p, ns, tot, c->icp_raw.p);
     if ((rc = voxel_grid_device(c->icp_raw.p, Count::of_host(tot), leaf, out.p, c->d_counts + C_HOOK_NSEL, nullptr, nullptr, c->vg, c->stream))) return rc;
-    CUDA_TRY(cudaMemcpyAsync(c->h_mail + 900, c->d_counts + C_HOOK_NSEL, sizeof(int), cudaMemcpyDeviceToHost, c->stream));
+    CUDA_TRY(cudaMemcpyAsync(c->h_mail.p + 900, c->d_counts + C_HOOK_NSEL, sizeof(int), cudaMemcpyDeviceToHost, c->stream));
     CUDA_TRY(cudaStreamSynchronize(c->stream));
-    *n_out = c->h_mail[900];
+    *n_out = c->h_mail.p[900];
     c->launches += 10;
     return LIORF_OK;
 }
@@ -1967,7 +1897,7 @@ int liorf_loop_closure_icp(liorf_ctx* c, int loop_key_cur, int loop_key_pre, int
     out->n_source = n_src; out->n_target = n_tgt;
     if (n_src < 300 || n_tgt < 1000) return check_err(c);           // :655-656
     out->ran = 1;
-    if (!c->icp_out) { CUDA_TRY(cudaMalloc(&c->icp_out, ICP_NSUM * sizeof(double))); c->icp_counter = c->d_misc + 14; }
+    if (!c->icp_out) { CUDA_TRY(dev_alloc(c->icp_out, ICP_NSUM)); c->icp_counter = c->d_misc + 14; }
     int blocks = (n_src + ICP_BLOCK - 1) / ICP_BLOCK; if (blocks > 4 * c->num_sms) blocks = 4 * c->num_sms;
     if ((rc = c->icp_partial.reserve((size_t)blocks * ICP_NSUM)) || (rc = c->icp_src.reserve(n_src))) return rc;
     if ((rc = build_map_grid(c->icp_tgt.p, Count::of_host(n_tgt), c->icp_grid, c->stream))) return rc;
@@ -1975,7 +1905,7 @@ int liorf_loop_closure_icp(liorf_ctx* c, int loop_key_cur, int loop_key_pre, int
     const int r_max = (int)std::ceil(max_corr_dist) + 1;
     const float max_d2 = max_corr_dist * max_corr_dist;
     // the loop runs on the device (csrc/icp.cuh): iterations are enqueued in chunks and the state is read back once per chunk
-    if (!c->icp_state) CUDA_TRY(cudaMalloc(&c->icp_state, sizeof(IcpState)));
+    if (!c->icp_state) CUDA_TRY(dev_alloc(c->icp_state, 1));
     IcpState hs = icp_initial_state(max_iters);
     CUDA_TRY(cudaMemcpyAsync(c->icp_state, &hs, sizeof(hs), cudaMemcpyHostToDevice, c->stream));
     CUDA_TRY(cudaStreamSynchronize(c->stream));                       // hs is pageable: the copy must have left it before it is reused below
@@ -1989,7 +1919,7 @@ int liorf_loop_closure_icp(liorf_ctx* c, int loop_key_cur, int loop_key_pre, int
         CUDA_TRY(cudaMemcpyAsync(&hs, c->icp_state, sizeof(hs), cudaMemcpyDeviceToHost, c->stream));
         CUDA_TRY(cudaStreamSynchronize(c->stream));
     }
-    double* h_sums = reinterpret_cast<double*>(c->h_mail + 3000);   // 8-byte aligned slot of the pinned mailbox
+    double* h_sums = reinterpret_cast<double*>(c->h_mail.p + 3000);   // 8-byte aligned slot of the pinned mailbox
     // getFitnessScore(): the original source under the final transformation, no range limit
     {
         IcpT Tf; std::memcpy(Tf.t, hs.final_T, 12 * sizeof(float));
@@ -2026,13 +1956,10 @@ constexpr int ICPB_MAX_PAIRS = 256;                  // 512 clouds per wave; 2^2
 struct IcpbPair { int cur, pre, li; long long raw_src, raw_tgt; };
 
 static int icpb_stage(liorf_ctx* c, size_t bytes) {   // pinned staging (grows between waves, when the stream is idle)
-    liorf_ctx::IcpBatch& B = c->icpb;
-    if (bytes <= B.h_cap) return LIORF_OK;
-    if (B.h_stage) { CUDA_TRY(cudaStreamSynchronize(c->stream)); CUDA_TRY(cudaFreeHost(B.h_stage)); B.h_stage = nullptr; B.h_cap = 0; }
-    const size_t cap = std::max<size_t>(bytes, 1 << 20);
-    CUDA_TRY(cudaHostAlloc(&B.h_stage, cap, cudaHostAllocDefault));
-    B.h_cap = cap;
-    return LIORF_OK;
+    HostBuf<unsigned char>& h = c->icpb.h_stage;
+    if (bytes <= h.cap) return LIORF_OK;
+    if (h.p) CUDA_TRY(cudaStreamSynchronize(c->stream));
+    return h.reserve(std::max<size_t>(bytes, 1 << 20));
 }
 
 // one wave: pairs P[0 .. W).  *split = 1 (nothing written to out) when the wave's VoxelGrid keys need more than 32 bits: the caller halves it.
@@ -2063,7 +1990,7 @@ static int icpb_wave(liorf_ctx* c, const IcpbPair* P, int W, liorf_icp_result* c
     const size_t o_pd = take((size_t)W * sizeof(IcpPairDesc)), o_act = take((size_t)2 * W * sizeof(int2)), o_st = take((size_t)W * sizeof(IcpState));
     const size_t o_vox = take((size_t)2 * S * sizeof(int) + 2 * sizeof(int)), o_stb = take((size_t)W * sizeof(IcpState)), o_fit = take((size_t)2 * W * sizeof(double));
     if ((rc = icpb_stage(c, off))) return rc;
-    unsigned char* H = B.h_stage;
+    unsigned char* H = B.h_stage.p;
     int* h_vox = reinterpret_cast<int*>(H + o_vox);           // [2 S] (first voxel, count) per cloud, then the two flags
     if (tot > 0) {
         std::memcpy(H + o_sel, sel.data(), (size_t)ns * sizeof(KfSel));
@@ -2085,9 +2012,9 @@ static int icpb_wave(liorf_ctx* c, const IcpbPair* P, int W, liorf_icp_result* c
         unsigned* sorted_idx = nullptr;
         const Count cnt = Count::of_host(tot);
         if ((rc = radix_sort_pairs_iota(B.keys.p, cnt, B.sort, &sorted_idx, s))) return rc;
-        if ((rc = launch_scan(cnt, VgHeadLoad{B.keys.p}, VgHeadStore{B.seg_start.p, cnt}, B.scan, (unsigned*)B.d_flags, s))) return rc;
-        k_vg_centroid<<<(tot + 127) / 128, 128, 0, s>>>(B.raw.p, sorted_idx, B.seg_start.p, (const unsigned*)B.d_flags, B.vox.p, nullptr, B.keys.p, nullptr);
-        k_vgseg_out<<<(S + 255) / 256, 256, 0, s>>>(B.keys.p, B.seg_start.p, (const unsigned*)B.d_flags, B.seg_base.p, S, B.seg_vox.p);
+        if ((rc = launch_scan(cnt, VgHeadLoad{B.keys.p}, VgHeadStore{B.seg_start.p, cnt}, B.scan, (unsigned*)B.d_flags.get(), s))) return rc;
+        k_vg_centroid<<<(tot + 127) / 128, 128, 0, s>>>(B.raw.p, sorted_idx, B.seg_start.p, (const unsigned*)B.d_flags.get(), B.vox.p, nullptr, B.keys.p, nullptr);
+        k_vgseg_out<<<(S + 255) / 256, 256, 0, s>>>(B.keys.p, B.seg_start.p, (const unsigned*)B.d_flags.get(), B.seg_base.p, S, B.seg_vox.p);
         CUDA_TRY(cudaGetLastError());
         c->launches += 16;
         CUDA_TRY(cudaMemcpyAsync(h_vox, B.seg_vox.p, (size_t)2 * S * sizeof(int), cudaMemcpyDeviceToHost, s));
@@ -2259,9 +2186,9 @@ int liorf_build_global_map(liorf_ctx* c, float search_radius, float pose_density
     const float4* result = c->icp_raw.p; int n = tot;
     if (leaf > 0.f) {
         if ((rc = voxel_grid_device(c->icp_raw.p, Count::of_host(tot), leaf, c->icp_tgt.p, c->d_counts + C_HOOK_NSEL, nullptr, nullptr, c->vg, c->stream))) return rc;
-        CUDA_TRY(cudaMemcpyAsync(c->h_mail + 900, c->d_counts + C_HOOK_NSEL, sizeof(int), cudaMemcpyDeviceToHost, c->stream));
+        CUDA_TRY(cudaMemcpyAsync(c->h_mail.p + 900, c->d_counts + C_HOOK_NSEL, sizeof(int), cudaMemcpyDeviceToHost, c->stream));
         CUDA_TRY(cudaStreamSynchronize(c->stream));
-        n = c->h_mail[900]; result = c->icp_tgt.p;
+        n = c->h_mail.p[900]; result = c->icp_tgt.p;
     }
     c->launches += 10;
     *n_out = n;
@@ -2278,10 +2205,10 @@ static int front_prefetch(liorf_ctx* c, const liorf_frame_in* nx) {
     c->pre_valid = false;
     front_swap(c);                                   // the enqueue helpers below work on "the current set" and "the context's stream"
     { int rcs = need_stream_pre(c); if (rcs) return rcs; }
-    cudaStream_t main_stream = c->stream; c->stream = c->stream_pre;
+    std::swap(c->stream, c->stream_pre);            // until the swap back below, c->stream is the look-ahead stream
     int rc = LIORF_OK;
     // the set being overwritten was last read by work enqueued on the main stream before this frame began (keyframe copy, ScanContext)
-    if (c->frame_start_recorded && cudaStreamWaitEvent(c->stream_pre, c->ev_frame_start, 0) != cudaSuccess) rc = LIORF_ERR_CUDA;
+    if (c->frame_start_recorded && cudaStreamWaitEvent(c->stream, c->ev_frame_start, 0) != cudaSuccess) rc = LIORF_ERR_CUDA;
     if (!rc) {
         if (nx->pts_on_device) rc = liorf_project_point_cloud_dev(c, nx->pts, nx->n, nx->time_scan_cur, nx->imu_time, nx->imu_rot_x, nx->imu_rot_y, nx->imu_rot_z,
                                                                   nx->imu_pointer_cur, nx->deskew_enabled);
@@ -2289,8 +2216,8 @@ static int front_prefetch(liorf_ctx* c, const liorf_frame_in* nx) {
                                             nx->imu_rot_z, nx->imu_pointer_cur, nx->deskew_enabled, nullptr, nullptr, nullptr);
     }
     if (!rc) rc = downsample_async(c, nullptr, c->num_sms - c->s2m_grid >= 4 ? c->num_sms - c->s2m_grid : 0);      // beside the solver: its spare SMs
-    if (!rc && cudaEventRecord(c->ev_pre_done, c->stream_pre) != cudaSuccess) rc = LIORF_ERR_CUDA;
-    c->stream = main_stream;
+    if (!rc && cudaEventRecord(c->ev_pre_done, c->stream) != cudaSuccess) rc = LIORF_ERR_CUDA;
+    std::swap(c->stream, c->stream_pre);
     front_swap(c);
     if (rc) return rc;
     c->pre_valid = true; c->pre_index = nx->frame_index; c->pre_n = nx->n; c->pre_pts = nx->pts;
@@ -2313,7 +2240,7 @@ int liorf_process_frame(liorf_ctx* c, const liorf_frame_in* in, liorf_frame_out*
     std::memset(out, 0, sizeof(*out)); out->keyframe_id = -1; out->loop_id = -1;
     using clk = std::chrono::steady_clock;
     auto T0 = clk::now();
-    auto stamp = [&](int k, cudaStream_t st) { if (c->host_timing) { if (!c->tl_ev[k]) cudaEventCreate(&c->tl_ev[k]); cudaEventRecord(c->tl_ev[k], st); } };
+    auto stamp = [&](int k, cudaStream_t st) { if (c->host_timing) { if (!c->tl_ev[k]) (void)event_create(c->tl_ev[k], cudaEventDefault); cudaEventRecord(c->tl_ev[k], st); } };
     stamp(0, c->stream);
     auto lap = [&](int k) { if (c->host_timing) { auto t = clk::now(); c->host_us[k] += std::chrono::duration<double, std::micro>(t - T0).count(); T0 = t; } };
     // everything the earlier frames left on the main stream precedes this point: the front set they lived in may be refilled after it
@@ -2435,11 +2362,7 @@ int liorf_reserve(liorf_ctx* c, int n_scan_max, int m_raw_max, int n_keyframe_po
         (rc = reserve_zeroed(c->vg_map.scan.status, (m + SCAN_TILE - 1) / SCAN_TILE, c->stream))) return rc;
     if (n_keyframe_points_max > 0 && (rc = c->kf_points.reserve((size_t)n_keyframe_points_max, c->stream, true))) return rc;
     if (sc_entries_max > 0 && (rc = sc_reserve(c, sc_entries_max))) return rc;
-    if (c->h_sel_cap < 4096) {
-        if (c->h_sel) cudaFreeHost(c->h_sel);
-        c->h_sel_cap = 4096;
-        CUDA_TRY(cudaHostAlloc(&c->h_sel, (size_t)2 * c->h_sel_cap * sizeof(KfSel), cudaHostAllocDefault));
-    }
+    if ((rc = c->h_sel.reserve((size_t)2 * 4096))) return rc;
     CUDA_TRY(cudaStreamSynchronize(c->stream));
     return LIORF_OK;
 }
@@ -2504,9 +2427,9 @@ int liorf_debug_s2m_arrivals(liorf_ctx* c, int enable, unsigned long long* out /
     CUDA_TRY(cudaSetDevice(c->P.device));
     CUDA_TRY(cudaStreamSynchronize(c->stream));
     const size_t bytes = (size_t)S2M_MAX_ITERS * S2M_GT_STRIDE * sizeof(unsigned long long);
-    if (enable && !c->d_dbg_gt) { CUDA_TRY(cudaMalloc(&c->d_dbg_gt, bytes)); CUDA_TRY(cudaMemset(c->d_dbg_gt, 0, bytes)); }
+    if (enable && !c->d_dbg_gt) { CUDA_TRY(dev_alloc(c->d_dbg_gt, (size_t)S2M_MAX_ITERS * S2M_GT_STRIDE)); CUDA_TRY(cudaMemset(c->d_dbg_gt, 0, bytes)); }
     if (out && c->d_dbg_gt) CUDA_TRY(cudaMemcpy(out, c->d_dbg_gt, bytes, cudaMemcpyDeviceToHost));
-    if (!enable && c->d_dbg_gt) { cudaFree(c->d_dbg_gt); c->d_dbg_gt = nullptr; }
+    if (!enable) c->d_dbg_gt.reset();
     return LIORF_OK;
 }
 int liorf_debug_s2m_clocks(liorf_ctx* c, int enable, long long* out /*64*8 or null*/) {
@@ -2514,16 +2437,16 @@ int liorf_debug_s2m_clocks(liorf_ctx* c, int enable, long long* out /*64*8 or nu
     if (!c) return LIORF_ERR_ARG;
     CUDA_TRY(cudaSetDevice(c->P.device));
     CUDA_TRY(cudaStreamSynchronize(c->stream));
-    if (enable && !c->d_dbg) { CUDA_TRY(cudaMalloc(&c->d_dbg, S2M_MAX_ITERS * 8 * sizeof(long long))); CUDA_TRY(cudaMemset(c->d_dbg, 0, S2M_MAX_ITERS * 8 * sizeof(long long))); }
+    if (enable && !c->d_dbg) { CUDA_TRY(dev_alloc(c->d_dbg, S2M_MAX_ITERS * 8)); CUDA_TRY(cudaMemset(c->d_dbg, 0, S2M_MAX_ITERS * 8 * sizeof(long long))); }
     if (out && c->d_dbg) CUDA_TRY(cudaMemcpy(out, c->d_dbg, S2M_MAX_ITERS * 8 * sizeof(long long), cudaMemcpyDeviceToHost));
-    if (!enable && c->d_dbg) { cudaFree(c->d_dbg); c->d_dbg = nullptr; }
+    if (!enable) c->d_dbg.reset();
     return LIORF_OK;
 }
 int liorf_get_last_counts(liorf_ctx* c, int* n_scan, int* n_ds, int* m_ds, int* iters) {
     LIORF_NVTX;
     if (!c) return LIORF_ERR_ARG;
     if (n_scan) *n_scan = c->rep_counts[0]; if (n_ds) *n_ds = c->rep_counts[1]; if (m_ds) *m_ds = c->rep_counts[2];
-    if (iters) *iters = c->h_mail[1024 + 448];       // S2MTrace.iters as of the last liorf_get_pose
+    if (iters) *iters = c->h_mail.p[1024 + 448];       // S2MTrace.iters as of the last liorf_get_pose
     return LIORF_OK;
 }
 int liorf_get_keyframe(liorf_ctx* c, int id, liorf_point* out, int capacity, int* n, float pose6[6], double* time) {

@@ -140,8 +140,8 @@ struct DeskewWork {
     DevBuf<RawPoint> raw;           // staging for host input
     DevBuf<double> imu;             // 4 x rows (time, rx, ry, rz)
     DevBuf<int> kept;               // ordered raw indices of the kept points
-    float* start_inv = nullptr;     // 12 floats (device)
-    int* first_kept = nullptr;
+    DevMem<float> start_inv;       // 12 floats
+    int* first_kept = nullptr;     // view: a word of the front set's counts
     ScanWork scan;
 };
 

@@ -138,9 +138,9 @@ __device__ __forceinline__ int draw_ticket(unsigned long long* ticket, unsigned&
 }
 
 struct ScanWork {            // per-scan scratch: ticket word + status array
-    unsigned long long* ticket = nullptr;       // device, initialised to TICKET_INIT once
+    unsigned long long* ticket = nullptr;       // view: a word of the context's tickets, initialised to TICKET_INIT once
     DevBuf<unsigned long long> status;
-    int* err_flag = nullptr;
+    int* err_flag = nullptr;                    // view: the context's error flag
 };
 
 __device__ __forceinline__ unsigned warp_incl_scan(unsigned v) {
@@ -294,8 +294,8 @@ __global__ void __launch_bounds__(SORT_BLOCK) k_radix_pass(const unsigned* __res
 struct SortWork {
     DevBuf<unsigned> keys_alt, vals_a, vals_b, hist;
     DevBuf<unsigned long long> status;
-    unsigned long long* ticket = nullptr;       // device, initialised to TICKET_INIT once (see draw_ticket)
-    int* err_flag = nullptr;
+    unsigned long long* ticket = nullptr;       // view: a word of the context's tickets, initialised to TICKET_INIT once (see draw_ticket)
+    int* err_flag = nullptr;                    // view: the context's error flag
 };
 
 // Sorts keys (in place semantic: result ends in keys / vals_out) stably; values start as iota.

@@ -28,18 +28,18 @@ struct VoxelGridWork {
     DevBuf<float> partial;          // per-block min/max (6 floats each)
     DevBuf<unsigned> keys;
     DevBuf<unsigned> seg_start;     // start of each voxel segment in the sorted order (+ sentinel)
-    VoxMeta* meta = nullptr;        // device
-    int* mm_counter = nullptr;      // device, zero-initialised
+    DevMem<VoxMeta> meta;
+    int* mm_counter = nullptr;      // view: a zero-initialised word of the context's counters
     SortWork sort;
     ScanWork scan;
     bool small_attr_set = false;
     bool force_large = false;       // tests: run the multi-kernel path on small clouds too
     // one-kernel path (k_vg_fused)
     DevBuf<float4> pts_sorted; DevBuf<unsigned> cta_hist; DevBuf<unsigned> cta_heads;
-    unsigned* fused_bar = nullptr;  // device [2], zero-initialised once
-    int* err_flag = nullptr;
+    DevMem<unsigned> fused_bar;     // [2], zero-initialised once
+    int* err_flag = nullptr;        // view: the context's error flag
     bool force_multi = false;       // tests: never take the one-kernel path
-    unsigned long long* dbg = nullptr;   // debug: phase stamps of the one-kernel path
+    DevMem<unsigned long long> dbg;      // debug: phase stamps of the one-kernel path
     int last_launches = 0;          // kernels (and memsets) the last voxel_grid_device call enqueued
 };
 
