@@ -365,6 +365,7 @@ int liorf_debug_qr_solve6(liorf_ctx* ctx, const float* A, const float* b, int n,
 int liorf_debug_force_large_voxelgrid(liorf_ctx* ctx, int on);   /* tests: multi-kernel VoxelGrid path on every cloud */
 int liorf_debug_voxelgrid_stamps(liorf_ctx* ctx, int enable, unsigned long long* out /* 32, nullable */);   /* debug: phase stamps of the one-kernel VoxelGrid */
 int liorf_debug_force_fused_voxelgrid(liorf_ctx* ctx, int on);   /* tests: one-kernel cooperative VoxelGrid path on small clouds too */
+int liorf_debug_voxelgrid_grid(liorf_ctx* ctx, int ctas);       /* tests: CTAs of liorf_voxel_grid's one-kernel VoxelGrid, 1..co-resident limit (0 = all SMs) */
 int liorf_debug_s2m_global_state(liorf_ctx* ctx, int on);          /* tests: solver keeps per-query state in global memory (the multi-round layout) */
 int liorf_debug_s2m_disable_cache(liorf_ctx* ctx, int on);        /* tests: full 27-cell search + plane refit every iteration */
 int liorf_debug_s2m_grid(liorf_ctx* ctx, int ctas);               /* tests: solver CTAs of every launch, 2..SMs (0 = defaults) */

@@ -403,6 +403,10 @@ class Context:
     def forceLargeVoxelGrid(self, on=True):
         _chk(self.lib.liorf_debug_force_large_voxelgrid(self.h, C.c_int(int(on))), "liorf_debug_force_large_voxelgrid")
 
+    def debugVoxelGridGrid(self, ctas=0):
+        """run voxelGrid's one-kernel cooperative path on `ctas` CTAs (0 = all SMs); widths the device cannot hold co-resident raise"""
+        _chk(self.lib.liorf_debug_voxelgrid_grid(self.h, C.c_int(int(ctas))), "liorf_debug_voxelgrid_grid")
+
     # ---- measurement helpers ----
     def enableTiming(self, on=True, sections=None):
         """sections: iterable of section names to time (None = all)"""

@@ -94,6 +94,7 @@ struct liorf_ctx {
     DevMem<IcpState> icp_state; DevBuf<QueryCache> qcache; DevBuf<float4> cand; unsigned s2m_launch_seq = 0; DevMem<S2MMail> d_mail; bool mail_fresh = false; bool s2m_global_state = false;
     int s2m_grid = 0; bool s2m_no_cache = false; int map_vg_grid = 0;
     int s2m_ctas = 0;                // tests: solver CTAs of every launch (0 = num_sms per function call, s2m_grid in liorf_process_frame)
+    int vg_ctas = 0;                 // tests: CTAs of liorf_voxel_grid's one-kernel VoxelGrid (0 = num_sms)
     DevBuf<float4> h_coeff, h_sel_pts, h_ori_c, h_coeff_c; DevBuf<unsigned char> h_flag; DevBuf<int> h_idx; DevBuf<float> h_d2, h_plane;
     DevBuf<double> lm_partial; ScanWork combine_scan; int hook_n = 0;
     DevMem<float> d_lm_out;         // AtA[36] AtB[6] X[6]
@@ -617,7 +618,7 @@ int liorf_voxel_grid(liorf_ctx* c, const liorf_point* in, int n, float leaf, lio
     if ((rc = c->membership.reserve(cap))) return rc;
     if ((rc = c->out_keys.reserve(cap))) return rc;
     if (n > 0) CUDA_TRY(cudaMemcpyAsync(c->map_raw.p, in, (size_t)n * sizeof(float4), cudaMemcpyHostToDevice, c->stream));
-    rc = voxel_grid_device(c->map_raw.p, Count::of_host(n), leaf, tmp_out.p, c->d_counts + C_NSEL, c->membership.p, c->out_keys.p, c->vg, c->stream, c->num_sms);
+    rc = voxel_grid_device(c->map_raw.p, Count::of_host(n), leaf, tmp_out.p, c->d_counts + C_NSEL, c->membership.p, c->out_keys.p, c->vg, c->stream, c->vg_ctas ? c->vg_ctas : c->num_sms);
     if (rc) return rc;
     CUDA_TRY(cudaMemcpyAsync(c->h_mail.p + 200, c->d_counts + C_NSEL, sizeof(int), cudaMemcpyDeviceToHost, c->stream));
     CUDA_TRY(cudaStreamSynchronize(c->stream));
@@ -1384,6 +1385,19 @@ int liorf_debug_force_fused_voxelgrid(liorf_ctx* c, int on) {
     c->vg.force_multi = c->vg_map.force_multi = c->alt.vg.force_multi = false;
     return LIORF_OK;
 }
+/* tests: liorf_voxel_grid runs the one-kernel cooperative VoxelGrid on `ctas` CTAs (0 = all SMs), so that every chunk length and grid width
+ * it can run with is reachable from small clouds.  Its grid barrier needs every CTA resident at once: widths beyond what the device holds
+ * co-resident are refused. */
+int liorf_debug_voxelgrid_grid(liorf_ctx* c, int ctas) {
+    LIORF_NVTX;
+    if (!c || ctas < 0) return LIORF_ERR_ARG;
+    CUDA_TRY(cudaSetDevice(c->P.device));
+    int occ = 0;
+    CUDA_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, k_vg_fused, VGF_THREADS, 0));
+    if (ctas > occ * c->num_sms) return LIORF_ERR_ARG;
+    c->vg_ctas = ctas;
+    return LIORF_OK;
+}
 /* selects the ring-key search implementation: 0 auto, 1 CUDA-core brute force, 2 tensor-core filter + exact re-rank */
 int liorf_sc_set_search_path(liorf_ctx* c, int mode) {
     LIORF_NVTX;
@@ -2021,6 +2035,20 @@ static int icpb_wave(liorf_ctx* c, const IcpbPair* P, int W, liorf_icp_result* c
         CUDA_TRY(cudaMemcpyAsync(h_vox + 2 * S, B.d_flags, 2 * sizeof(int), cudaMemcpyDeviceToHost, s));
         CUDA_TRY(cudaStreamSynchronize(s));                                    // sync 1: voxel counts of every cloud
         if (h_vox[2 * S + 1] && W > 1) { *split = 1; return LIORF_OK; }
+        if (h_vox[2 * S + 1]) {
+            // one pair whose key ranges sum past 2^32 (a cloud near PCL's guard has a range up to ~2^32 by itself): the segmented keys
+            // wrapped, so its two clouds are filtered one at a time from the same transformed points, as the single-pair call filters them
+            int at = 0;
+            for (int sg = 0; sg < S; ++sg) {
+                if ((rc = voxel_grid_device(B.raw.p + seg_first[sg], Count::of_host(seg_n[sg]), leaf, B.vox.p + at, c->d_counts + C_HOOK_NSEL, nullptr, nullptr,
+                                            c->vg, s))) return rc;
+                CUDA_TRY(cudaMemcpyAsync(h_vox + 2 * sg + 1, c->d_counts + C_HOOK_NSEL, sizeof(int), cudaMemcpyDeviceToHost, s));
+                CUDA_TRY(cudaStreamSynchronize(s));
+                h_vox[2 * sg] = at; at += h_vox[2 * sg + 1];
+                c->launches += c->vg.last_launches;
+            }
+            h_vox[2 * S] = at;
+        }
     } else {
         std::memset(h_vox, 0, (size_t)(2 * S + 2) * sizeof(int));
     }

@@ -288,7 +288,8 @@ __global__ void __launch_bounds__(VGS_THREADS, 1) k_vg_small(const float4* __res
     {
         const float inv = s_meta.inv; const int b0 = s_meta.min_b[0], b1 = s_meta.min_b[1], b2 = s_meta.min_b[2], m1 = s_meta.mul1, m2 = s_meta.mul2;
         const bool ovf = s_meta.overflow != 0;
-        const unsigned max_key = ovf ? (unsigned)(n - 1) : (unsigned)((long long)s_meta.div_b[0] * s_meta.div_b[1] * s_meta.div_b[2] - 1);
+        // the div_b product can pass 2^32 under PCL's guard (which bounds the d product): its keys wrap and span all 32 bits
+        const unsigned max_key = ovf ? (unsigned)(n - 1) : (unsigned)min((long long)s_meta.div_b[0] * s_meta.div_b[1] * s_meta.div_b[2] - 1, 0xffffffffLL);
         bits = 32 - __clz(max_key | 1u);
         for (int i = tid; i < P; i += VGS_THREADS) {
             unsigned key = 0xffffffffu;
@@ -494,7 +495,8 @@ __global__ void __launch_bounds__(VGF_THREADS, 2) k_vg_fused(VgFusedArgs a) {
         vgf_finish(a.bar);
         return;
     }
-    const unsigned max_key = (unsigned)((long long)s_meta.div_b[0] * s_meta.div_b[1] * s_meta.div_b[2] - 1);
+    // the div_b product can pass 2^32 under PCL's guard (which bounds the d product): its keys wrap and span all 32 bits
+    const unsigned max_key = (unsigned)min((long long)s_meta.div_b[0] * s_meta.div_b[1] * s_meta.div_b[2] - 1, 0xffffffffLL);
     const int bits = 32 - __clz(max_key | 1u);
     const int npass = (bits + RADIX_BITS - 1) / RADIX_BITS;
     // the CTA's chunk of the input order: whole tiles, contiguous

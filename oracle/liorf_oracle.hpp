@@ -70,7 +70,8 @@ inline P4 apply_affine(const float t[12], const P4& p) {
 // call sites src/mapOptmization.cpp:1037-1038 (local map), 1064-1065 (current scan).
 // Returns number of output points, or -1 when PCL's int32 index overflow guard fires (PCL then
 // copies the input through unfiltered).  membership[i] = output slot of input point i.
-// Canonical rule for the unspecified (unstable-sort) intra-voxel order: ascending input index.
+// Voxel order: PCL's, ascending unsigned index (wrapped mod 2^32).  Canonical rule for the unspecified (unstable-sort)
+// intra-voxel order: ascending input index.
 // ------------------------------------------------------------------------------------------------
 struct VoxelMeta { float minp[3], maxp[3]; int min_b[3], div_b[3]; float inv_leaf; };
 
@@ -97,15 +98,17 @@ inline int voxel_grid(const P4* in, int n, float leaf, std::vector<P4>& out, std
     }
     if (meta) { for (int a = 0; a < 3; ++a) { meta->minp[a] = mn[a]; meta->maxp[a] = mx[a]; meta->min_b[a] = min_b[a]; meta->div_b[a] = div_b[a]; } meta->inv_leaf = inv; }
     if (dx * dy * dz > (int64_t)std::numeric_limits<int32_t>::max()) return -1;   // "Leaf size is too small"
-    const int mul1 = div_b[0], mul2 = div_b[0] * div_b[1];
-    std::vector<std::pair<int, int>> iv(n);     // (voxel idx, point index)
+    // The guard bounds dx·dy·dz, but the index uses div_b, which can be one larger per axis: indices can pass 2^31 and even 2^32.
+    // PCL computes the index in int (wrapping) and stores it as unsigned int; cloud_point_index_idx::operator< compares unsigned.
+    const int64_t mul1 = div_b[0], mul2 = (int64_t)div_b[0] * div_b[1];
+    std::vector<std::pair<uint32_t, int>> iv(n);     // (voxel idx mod 2^32, point index)
     for (int k = 0; k < n; ++k) {
         int i0 = (int)(std::floor(in[k].x * inv) - (float)min_b[0]);
         int i1 = (int)(std::floor(in[k].y * inv) - (float)min_b[1]);
         int i2 = (int)(std::floor(in[k].z * inv) - (float)min_b[2]);
-        iv[k] = {i0 + i1 * mul1 + i2 * mul2, k};
+        iv[k] = {(uint32_t)(i0 + i1 * mul1 + i2 * mul2), k};
     }
-    std::sort(iv.begin(), iv.end());            // (idx, point index) lexicographic == stable by idx
+    std::sort(iv.begin(), iv.end());            // (unsigned idx, point index) lexicographic == stable by idx
     int k = 0;
     while (k < n) {
         int j = k;
@@ -118,7 +121,7 @@ inline int voxel_grid(const P4* in, int n, float leaf, std::vector<P4>& out, std
         }
         float cnt = (float)(j - k);
         out.push_back(P4{sx / cnt, sy / cnt, sz / cnt, si / cnt});
-        if (out_keys) out_keys->push_back(iv[k].first);
+        if (out_keys) out_keys->push_back((int)iv[k].first);     // the int32 bit pattern of the unsigned index
         k = j;
     }
     return (int)out.size();
